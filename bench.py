@@ -149,6 +149,41 @@ def measured_peaks():
         return {}
 
 
+DUMP_LIMIT_BYTES = 60 << 20       # --dump-outputs: below 64 MB in all, .npy headers included
+
+
+def last_chain_row(h, world=1, rank=0):
+    """The last stored row of the chains as sample() returns it, [P][d + 2] with one row per particle id of the whole job.
+    A sharded handle has no chains of its own: every rank sends its last row by position to rank 0, which merges the
+    rows by particle id as distributed.sample() does (None on the other ranks)."""
+    if world == 1:
+        return h.chains(h.stored_iterations - 1, 1)[:, :, 0]
+    import torch.distributed as dist
+
+    from demcmc_b200 import distributed
+    parts = distributed._gather_arrays(dist, h.history_by_slot(h.stored_iterations - 1, 1), rank, world, h.cfg.device)
+    if rank != 0:
+        return None
+    th, w, ids, acc = (p if isinstance(p, np.ndarray) else p.cpu().numpy() for p in parts)
+    samples, lp, accept, final_ids = distributed._merge_by_id(th, w, ids, acc, 1, h.P_total, h.d)
+    return np.column_stack([samples[:, :, 0], accept[final_ids, 0], lp[final_ids, 0]])
+
+
+def dump_outputs(out_dir, row):
+    """Writes what the timed run left for a caller, so that two builds can be compared output for output: `row`, the
+    last_chain_row() of the run, split into the parameters, the acceptance flags and the log posteriors, float64.  When
+    it exceeds DUMP_LIMIT_BYTES, a fixed, seeded sample of the particle ids is written; particle_id.npy names the ids
+    either way."""
+    ids = np.arange(row.shape[0])
+    if row.nbytes + ids.size * 8 > DUMP_LIMIT_BYTES:
+        ids = np.sort(np.random.default_rng(0).choice(ids.size, DUMP_LIMIT_BYTES // ((row.shape[1] + 1) * 8), replace=False))
+        row = row[ids]
+    os.makedirs(out_dir, exist_ok=True)
+    d = row.shape[1] - 2
+    for name, a in (("samples", row[:, :d]), ("acceptance", row[:, d]), ("lp", row[:, d + 1]), ("particle_id", ids)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------
 # CPU arm: the C restatement of the reference's algorithm (oracle/), one thread per group as the
 # reference's ThreadsX.map over groups (src/main.jl:135-148)
@@ -267,6 +302,10 @@ def run_b200(args):
     barrier()
     t1 = time.time()
     c1 = h.counters()
+    if args.dump_outputs:
+        row = last_chain_row(h, world, rank)                         # every rank takes part in the gather
+        if rank == 0:
+            dump_outputs(args.dump_outputs, row)
     windows = [(t0, t1, "timed")]
     wall_timed = t1 - t0
     # second pass of the same length with every likelihood launch bracketed by CUDA events on the
@@ -509,6 +548,8 @@ def run_single_process(args):
     h.run(args.steps)
     wall = time.perf_counter() - t0
     c1 = h.counters()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_chain_row(h))
     h.set_timing(0, False)
     h.run(args.steps)
     c2 = h.counters()
@@ -552,7 +593,11 @@ def main():
     ap.add_argument("--dim", type=int, default=None, help="dimensions of the multivariate normal (default 50)")
     ap.add_argument("--particles", type=int, default=None, help="particles per group (default 256)")
     ap.add_argument("--groups-per-gpu", type=int, default=None, help="groups per GPU (default 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the chains' last row (parameters, acceptance, lp) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 arm computed; the reference arm runs fewer particles")
     global N_DIM, NP, GROUPS_PER_GPU
     shape_given = args.dim or args.particles or args.groups_per_gpu
     N_DIM, NP, GROUPS_PER_GPU = args.dim or N_DIM, args.particles or NP, args.groups_per_gpu or GROUPS_PER_GPU

@@ -26,3 +26,15 @@ def cuda():
     import common
     common.use_cuda()
     yield
+
+
+@pytest.fixture(autouse=True)
+def _bind_requested_library(request):
+    """emu and cuda are set up once per session, but one session may run CPU and GPU tests in turn: every test
+    that asks for one of them gets its library bound again, not the one the test before it left bound."""
+    import common
+    if "cuda" in request.fixturenames:
+        common.use_cuda()
+    elif "emu" in request.fixturenames:
+        common.D._ffi.use_library(common.EMU_LIB)
+    yield
