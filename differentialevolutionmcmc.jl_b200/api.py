@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from .handle import Handle
+from .handle import Handle, compile_loglike
 
 
 # ---- registered priors (replace prior_loglike closures) -----------------------------------------
@@ -92,11 +92,15 @@ class GPULoglike:
     GPULoglike("lba", choice=c, rt=t)            sum(logpdf.(LBA(;ν,A,k,τ), c, t))
     GPULoglike("hier_normal", Y)                 Y is n_subj × n_per (Examples/Hierarchical_Example.jl)
     GPULoglike("mvnormal_full", X, cov=Σ)        sum(logpdf(MvNormal(μ, σ²Σ), X')) with a known covariance Σ
+    GPULoglike("custom", X, source=src)          sum_i demcmc_obs(par, X[i]) + demcmc_particle(θ): a likelihood written as
+                                                 CUDA C++ (include/demcmc_b200.h: DEMCMC_CUSTOM), compiled here for
+                                                 sm_100a; X is a vector, an n_obs × n_cols matrix, or None (no data)
     (Examples/Guassian_Example_Vector.jl is the "gaussian" kernel: its loglike(data, θ...) destructures μ, σ)
     """
-    KINDS = ("gaussian", "mvnormal", "binomial", "lnr", "lba", "hier_normal", "rastrigin", "mvnormal_full")
+    KINDS = ("gaussian", "mvnormal", "binomial", "lnr", "lba", "hier_normal", "rastrigin", "mvnormal_full", "custom")
 
-    def __init__(self, kind, x=None, *, choice=None, rt=None, N=None, k=None, sigma=None, lba_floor=1e-10, cov=None):
+    def __init__(self, kind, x=None, *, choice=None, rt=None, N=None, k=None, sigma=None, lba_floor=1e-10, cov=None,
+                 source=None):
         kind = str(kind).lstrip(":")
         if kind not in self.KINDS:
             raise ValueError(f"no registered kernel for {kind!r}; registered: {self.KINDS}")
@@ -105,7 +109,16 @@ class GPULoglike:
         self.sigma = sigma
         self.lba_floor = lba_floor
         self.cov = None if cov is None else np.ascontiguousarray(cov, dtype=np.float64)   # mvnormal_full: the known covariance
-        if kind == "rastrigin":              # the objective of test/optimization_tests.jl:15-23: no data
+        self.source = None
+        if kind == "custom":
+            if not isinstance(source, (str, bytes)) or not source:
+                raise ValueError("custom needs source=: CUDA C++ text that defines demcmc_obs (include/demcmc_b200.h)")
+            self.x = None if x is None else np.ascontiguousarray(x, dtype=np.float64)
+            if self.x is not None and (self.x.ndim not in (1, 2) or (self.x.ndim == 2 and self.x.shape[1] == 0)):
+                raise ValueError("custom data must be a vector or an n_obs x n_cols matrix with n_cols >= 1")
+            compile_loglike(source)          # a source that does not compile fails here, with the compiler log
+            self.source = source
+        elif kind == "rastrigin":              # the objective of test/optimization_tests.jl:15-23: no data
             self.x = np.zeros(0)
         elif kind == "binomial":
             if N is None or k is None:
@@ -434,7 +447,8 @@ def build_handle(model: DEModel, de: DE, device=0, trace=False, group_begin=0, g
     if not isinstance(ll, GPULoglike):
         raise TypeError(
             "loglike must be a GPULoglike bound to a registered kernel "
-            f"{GPULoglike.KINDS}; an arbitrary closure cannot run on the device and there is no CPU fallback")
+            f"{GPULoglike.KINDS}; an arbitrary closure cannot run on the device and there is no CPU fallback "
+            "(write the likelihood as CUDA source instead: GPULoglike(\"custom\", X, source=...))")
     theta0 = model.sample_prior()
     shapes = _shapes(theta0)
     d = len(_flatten(theta0))
@@ -456,7 +470,7 @@ def build_handle(model: DEModel, de: DE, device=0, trace=False, group_begin=0, g
     table = _prior_table(model, shapes, needed=de.evaluate_fitness is not evaluate_fun)
 
     def bind():
-        h.set_model(ll.kind, table, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov)
+        h.set_model(ll.kind, table, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov, source=ll.source)
     if background_model:
         return h, shapes, d, _Background(bind)
     bind()

@@ -69,6 +69,17 @@ int launch_propose(const ConfigDev &cfg, const ModelDev &m, const Level &lv);
 // has cleared it and set ll_q); the other models write ll_part
 int launch_loglik(const ConfigDev &cfg, const ModelDev &m, const double *theta, const Level &lv, double *ll_part, long long *ll_acc);
 int launch_accept(const ConfigDev &cfg, const ModelDev &m, const Level &lv);
+// user-written likelihoods (M_CUSTOM): custom_compile builds a DEMCMC_CUSTOM source into an sm_100a cubin with NVRTC and
+// keeps it in a per-process cache keyed by the source text (no device needed).  0; -1 = the source does not compile (the
+// compiler log is last_error()); -2 = unsupported (no NVRTC, DEMCMC_NPAR above CUSTOM_MAX_PAR, no CUDA backend).
+// custom_load loads the source's cubin (compiled first if needed; the same codes, -3 = the CUDA load failed) on the current
+// device; launch_loglik
+// then runs it for ModelDev.custom = *module.  custom_unload frees a module no launch is still using.
+// Declared weak: a backend without a run-time compiler (the host-only test double) does not define them, they resolve to
+// null there, and the engine refuses custom models with DEMCMC_EUNSUPPORTED.
+int custom_compile(const char *source) __attribute__((weak));
+int custom_load(const char *source, void **module, int *has_obs /* the source defines demcmc_obs */) __attribute__((weak));
+void custom_unload(void *module) __attribute__((weak));
 // small pointwise problems: propose + likelihood + accept of a level in one launch, one warp per
 // particle; returns 1 when the model / size does not qualify (launch the three kernels instead)
 int launch_level_fused(const ConfigDev &cfg, const ModelDev &m, const Level &lv);

@@ -14,7 +14,9 @@ constexpr int SSD_KS = 4 * SSD_NJ; // max dimensions per dimension split
 constexpr int PW_TP = 8;          // particles per tile of the pointwise kernels
 constexpr int PW_THREADS = 256;
 
-enum ModelKind { M_GAUSSIAN = 0, M_MVNORMAL = 1, M_BINOMIAL = 2, M_LNR = 3, M_LBA = 4, M_HIER = 5, M_RASTRIGIN = 6, M_MVN_FULL = 7 };
+enum ModelKind { M_GAUSSIAN = 0, M_MVNORMAL = 1, M_BINOMIAL = 2, M_LNR = 3, M_LBA = 4, M_HIER = 5, M_RASTRIGIN = 6, M_MVN_FULL = 7,
+                 M_CUSTOM = 8 /* user-written per-observation density compiled at run time (kernels.cu: k_ll_custom) */ };
+constexpr int CUSTOM_MAX_PAR = 256;   // d and DEMCMC_NPAR of a custom model (the per-particle values staged in shared memory)
 // the likelihoods that are a sum of squared deviations from per-dimension means (the streamed DMMA kernels k_xdot / k_chunk_persist)
 DE_HD bool is_ssd(int kind) { return kind == M_MVNORMAL || kind == M_HIER || kind == M_MVN_FULL; }
 enum { UPDATE_MH = 0, UPDATE_MAXIMIZE = 1, UPDATE_MINIMIZE = 2 };
@@ -59,6 +61,8 @@ struct ModelDev {
     // how many slices one CTA happens to process
     int32_t n_osplit, n_ksplit, split_len, ksplit_len;
     uint32_t ksplit_magic;    // ceil(2^32 / ksplit_len): k / ksplit_len = umulhi(k, magic) for every dimension index k < 2^32 / ksplit_len
+    int32_t n_cols;           // M_CUSTOM: values per observation, x[n_obs][n_cols]
+    void *custom;             // M_CUSTOM: the module loaded on this device (be::custom_load), host-side handle
 };
 
 // Packed layout of the centred data for k_xdot: element (observation i, dimension k) lives in the

@@ -65,6 +65,7 @@ struct demcmc_handle {
     ModelDev dmodel;
     bool has_model = false, has_state = false;
     std::vector<void *> model_allocs;
+    void *custom_mod = nullptr;                         // DEMCMC_CUSTOM: the likelihood module loaded on this device
     // state rows
     int64_t hist_cap = 0, iters_done = 0;
     int64_t iter_offset = 0;                            // iterations the chain ran before this handle (demcmc_set_iteration)
@@ -600,6 +601,7 @@ int demcmc_destroy(demcmc_handle *h)
     be::dfree(h->ghist_theta); be::dfree(h->ghist_pos); be::dfree(h->gid_tmp);
     if (h->comm) be::comm_destroy(h->comm);
     for (void *p : h->model_allocs) be::dfree(p);
+    if (h->custom_mod) be::custom_unload(h->custom_mod);
     void *ptrs[] = { h->hist_theta, h->hist_w, h->hist_id, h->hist_acc, h->hist_pos, h->scr_theta, h->scr_w, h->scr_id, h->scr_acc,
                      h->prop_theta, h->prop_prior, h->prop_adj, h->prop_msq, h->prop_inb, h->ll_acc, h->ll_q, h->base_th, h->base_cw, h->base_tot, h->ll_part, h->d_lo, h->d_hi, h->d_blocks,
                      h->plan_recs, h->d_picks, h->d_stage, h->d_stage_recv, h->d_mig_log, h->tr_theta, h->tr_w, h->tr_adj, h->tr_xdot, h->tr_acc, h->flush_buf };
@@ -609,6 +611,9 @@ int demcmc_destroy(demcmc_handle *h)
     delete h;
     return 0;
 }
+
+static_assert(CUSTOM_MAX_PAR == DEMCMC_CUSTOM_MAX_PAR, "k_ll_custom stages DEMCMC_CUSTOM_MAX_PAR values per particle");
+static const char NO_CUSTOM[] = "custom likelihoods need the CUDA backend (this backend has no run-time compiler)";
 
 int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
 {
@@ -622,6 +627,11 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
     BE(be::set_device(h->cfg.device));
     for (void *p : h->model_allocs) be::dfree(p);
     h->model_allocs.clear();
+    if (h->custom_mod) {                                     // rebinding: no launch may still use the old module
+        BE(be::sync());
+        be::custom_unload(h->custom_mod);
+        h->custom_mod = nullptr;
+    }
     be::dfree(h->ll_part); h->ll_part = nullptr;
     ModelDev &D = h->dmodel;
     memset(&D, 0, sizeof D);
@@ -644,10 +654,17 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
     case DEMCMC_HIER_NORMAL: want_d = m->n_dim + 3; break;
     case DEMCMC_RASTRIGIN: want_d = m->d; break;
     case DEMCMC_MVNORMAL_FULL: want_d = m->n_dim + 1; break;
+    case DEMCMC_CUSTOM:
+        if (!be::custom_load) return fail(DEMCMC_EUNSUPPORTED, "%s", NO_CUSTOM);
+        if (m->d < 1 || m->d > DEMCMC_CUSTOM_MAX_PAR) return fail(DEMCMC_EUNSUPPORTED, "a custom likelihood takes 1..%d parameters, got d = %d", DEMCMC_CUSTOM_MAX_PAR, m->d);
+        if (!m->source) return fail(DEMCMC_EINVAL, "a custom likelihood needs model.source");
+        if (m->n_obs > 0 && m->n_cols < 1) return fail(DEMCMC_EINVAL, "a custom likelihood with observations needs n_cols >= 1, got %d", m->n_cols);
+        want_d = m->d;
+        break;
     default: return fail(DEMCMC_EUNSUPPORTED, "no registered kernel for model kind %d: arbitrary closures are not supported and there is no CPU fallback", m->kind);
     }
     if (m->d != want_d) return fail(DEMCMC_EINVAL, "model kind %d expects d = %d, got %d", m->kind, want_d, m->d);
-    if (!m->x && m->kind != DEMCMC_RASTRIGIN) return fail(DEMCMC_EINVAL, "model data missing");
+    if (!m->x && m->kind != DEMCMC_RASTRIGIN && !(m->kind == DEMCMC_CUSTOM && m->n_obs == 0)) return fail(DEMCMC_EINVAL, "model data missing");
     if ((m->kind == DEMCMC_LNR || m->kind == DEMCMC_LBA) && (!m->choice || m->n_dim < 2 || m->n_dim > MAX_ACC))
         return fail(DEMCMC_EINVAL, "LNR/LBA need choices and 2..%d accumulators", MAX_ACC);
     if (m->n_obs < 0) return fail(DEMCMC_EINVAL, "negative n_obs");
@@ -744,8 +761,24 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         } else
         BE(be::launch_pack_ssd(m->x, dev, m->center, &D));       // centres and packs the data, fills D.ssd_xx / D.ssd_rowmax
     } else {
-        D.x = (const double *)upload(m->x, sizeof(double) * m->n_obs, dev);
+        // the pointwise kinds, and DEMCMC_CUSTOM: x[n_obs][n_cols], through the same observation splits (k_ll_custom).
+        // A custom model never qualifies for the fused / small-chunk / persistent kernels (their densities are the
+        // registered ones): every level runs propose -> k_ll_custom -> accept
+        const int64_t n_val = m->n_obs * (m->kind == DEMCMC_CUSTOM ? (int64_t)m->n_cols : 1);
+        D.x = (const double *)upload(m->x, sizeof(double) * n_val, dev);
         if (!D.x) return fail(DEMCMC_ENOMEM, "data upload failed");
+        if (m->kind == DEMCMC_CUSTOM) {
+            D.n_cols = m->n_cols;
+            int has_obs = 0;
+            if (int rc = be::custom_load(m->source, &h->custom_mod, &has_obs)) {
+                g_err = be::last_error();                    // the whole compiler log (fail() would cut it)
+                return rc == -1 ? DEMCMC_EINVAL : rc == -2 ? DEMCMC_EUNSUPPORTED : DEMCMC_ECUDA;
+            }
+            if (m->n_obs > 0 && !has_obs)
+                return fail(DEMCMC_EINVAL, "the model has %lld observations but its source defines no "
+                            "__device__ double demcmc_obs(const double *par, const double *x)", (long long)m->n_obs);
+            D.custom = h->custom_mod;
+        }
         if (m->choice) { D.choice = (const int32_t *)upload(m->choice, sizeof(int32_t) * m->n_obs, dev); if (!D.choice) return fail(DEMCMC_ENOMEM, "data upload failed"); }
         if (m->sigma) { D.has_sigma = 1; for (int r = 0; r < m->n_dim && r < MAX_ACC; ++r) D.sigma_acc[r] = m->sigma[r]; }
         const int64_t chunk = PW_THREADS;
@@ -760,6 +793,18 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
     BE(be::sync());
     h->has_model = true;
     return 0;
+}
+
+int demcmc_compile_loglike(const char *source, char *log, int64_t log_cap)
+{
+    if (log && log_cap > 0) log[0] = 0;
+    if (!source) return fail(DEMCMC_EINVAL, "null source");
+    if (!be::custom_compile) return fail(DEMCMC_EUNSUPPORTED, "%s", NO_CUSTOM);
+    const int rc = be::custom_compile(source);
+    if (rc == 0) return 0;
+    g_err = be::last_error();                                // the whole compiler log (fail() would cut it)
+    if (log && log_cap > 0) { const size_t n = std::min(g_err.size(), (size_t)log_cap - 1); memcpy(log, g_err.data(), n); log[n] = 0; }
+    return rc == -2 ? DEMCMC_EUNSUPPORTED : DEMCMC_EINVAL;
 }
 
 int demcmc_set_history(demcmc_handle *h, const double *rows)

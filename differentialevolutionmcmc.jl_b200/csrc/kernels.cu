@@ -7,16 +7,19 @@
 //                  (DMMA m8n8k4): the likelihood of the isotropic MVN and the hierarchical
 //                  normal models                                           (fp64-pipe-bound)
 //   k_ll_pointwise per-observation log densities (Gaussian, LNR, LBA) for a tile of particles
+//   k_ll_custom    the same for a density the caller writes (DEMCMC_CUSTOM), compiled at run time with NVRTC
 //   k_accept       one warp per particle: fixed-order reduction of the partial sums, Metropolis
 //                  accept, state-row write (replaces store_samples!)       (HBM-bound)
 //   k_mig_*        migration picks and the cyclic shift
 //   k_history      by-slot rows -> the reference's samples[n_rows, d, P] layout
 #include <cuda_runtime.h>
 #include <dlfcn.h>
+#include <nvrtc.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <map>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -2088,6 +2091,214 @@ int launch_chunk_persist(const ConfigDev &cfg, const ModelDev &m, const int32_t 
     return 0;
 }
 
+// ------------------------------------------------------------------------------------------------
+// user-written likelihoods (M_CUSTOM): the caller's per-observation density (include/demcmc_b200.h: DEMCMC_CUSTOM) is
+// compiled at run time with NVRTC into k_ll_custom, the structure of k_ll_pointwise<M_GAUSSIAN> specialised to that
+// density: PW_TP particles x one observation split per CTA, the same split partition, the same summation order
+// (thread-strided, warp shuffle, CTA in warp order), and the same ll_part slots, which accept_particle / k_eval_finish
+// reduce as for the registered pointwise kinds.  libnvrtc is loaded with dlopen, so the library still loads (and every
+// registered kind still runs) where it is missing.  The kernel is plain-launched (no programmatic dependent launch):
+// k_propose triggers its dependents early and k_ll_custom has no griddepcontrol.wait before it reads the proposals.
+// ------------------------------------------------------------------------------------------------
+static_assert(PW_TP == 8 && PW_THREADS == 256 && LV_POS_MASK == 0xFFFFFFu, "k_ll_custom's source spells these out");
+
+// ahead of the user's text: calls of demcmc_obs / demcmc_particle that the source does not define resolve to these
+// stand-ins (a definition in the source matches `const double *` exactly, these need a user-defined conversion); they
+// add 0, and their return type tells the kernel source which of the two the user wrote
+static const char CUSTOM_PRELUDE[] = R"CU(
+#define DEMCMC_INF __longlong_as_double(0x7ff0000000000000LL)
+#define DEMCMC_NAN __longlong_as_double(0x7ff8000000000000LL)
+struct demcmc_zero_ { __device__ operator double() const { return 0.0; } };
+struct demcmc_any_ptr_ { __device__ demcmc_any_ptr_(const double *) {} };
+__device__ inline demcmc_zero_ demcmc_obs(demcmc_any_ptr_, demcmc_any_ptr_) { return demcmc_zero_(); }
+__device__ inline demcmc_zero_ demcmc_particle(demcmc_any_ptr_) { return demcmc_zero_(); }
+#line 1 "user.cu"
+)CU";
+
+// after it: the likelihood kernel (k_ll_pointwise's Gaussian form with the density inlined)
+static const char CUSTOM_KERNEL[] = R"CU(
+#line 1 "demcmc_custom_kernel.cu"
+template <class T> struct demcmc_is_double_ { enum { value = 0 }; };
+template <> struct demcmc_is_double_<double> { enum { value = 1 }; };
+constexpr int demcmc_has_obs_ = demcmc_is_double_<decltype(demcmc_obs((const double *)0, (const double *)0))>::value;
+constexpr int demcmc_has_particle_ = demcmc_is_double_<decltype(demcmc_particle((const double *)0))>::value;
+static_assert(demcmc_has_obs_ || demcmc_has_particle_, "the source must define  __device__ double demcmc_obs(const double *par, "
+              "const double *x)  (or, for a likelihood without observations, __device__ double demcmc_particle(const double *theta))");
+// read by the host when the module is loaded: a model with observations needs demcmc_obs
+extern "C" __device__ int demcmc_custom_has_obs = demcmc_has_obs_;
+#ifdef DEMCMC_NPAR
+static_assert(DEMCMC_NPAR >= 1, "DEMCMC_NPAR must be at least 1");
+static_assert(DEMCMC_NPAR <= 256, "DEMCMC_NPAR is above DEMCMC_CUSTOM_MAX_PAR (256)");
+#define DEMCMC_PAR_LEN_ (DEMCMC_NPAR)
+#else
+#define DEMCMC_PAR_LEN_ 256
+#endif
+
+extern "C" __global__ void __launch_bounds__(256) k_ll_custom(const double *theta, int d, const int *order, int n, const double *x,
+                                                              int n_cols, long long n_obs, int split_len, int n_split, double *part)
+{
+    __shared__ double par[8][DEMCMC_PAR_LEN_];
+    __shared__ double red[8][8];
+    const int tile = blockIdx.x, split = blockIdx.y, tid = threadIdx.x;
+    const int nt = min(8, n - tile * 8);
+#ifdef DEMCMC_NPAR
+    if (tid < nt) {
+        const int p = order ? (int)((unsigned)order[tile * 8 + tid] & 0xFFFFFFu) : tile * 8 + tid;
+        demcmc_prepare(theta + (size_t)p * d, par[tid]);
+    }
+#else
+    for (int e = tid; e < nt * d; e += 256) {
+        const int t = e / d, k = e - t * d;
+        const int p = order ? (int)((unsigned)order[tile * 8 + t] & 0xFFFFFFu) : tile * 8 + t;
+        par[t][k] = theta[(size_t)p * d + k];
+    }
+#endif
+    __syncthreads();
+    double acc[8];
+#pragma unroll
+    for (int t = 0; t < 8; ++t) acc[t] = 0.0;
+    const long long i0 = (long long)split * split_len;
+    const long long i1 = min(n_obs, i0 + (long long)split_len);
+    for (long long i = i0 + tid; i < i1; i += 256) {
+        const double *xi = x + (size_t)i * n_cols;
+#pragma unroll
+        for (int t = 0; t < 8; ++t)
+            if (t < nt) acc[t] += (double)demcmc_obs(par[t], xi);
+    }
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+        double v = acc[t];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if ((tid & 31) == 0) red[tid >> 5][t] = v;
+    }
+    __syncthreads();
+    if (tid < nt) {
+        double v = 0.0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) v += red[w][tid];
+        const int p = order ? (int)((unsigned)order[tile * 8 + tid] & 0xFFFFFFu) : tile * 8 + tid;
+        if (demcmc_has_particle_ && split == 0) v += (double)demcmc_particle(theta + (size_t)p * d);
+        part[(size_t)p * n_split + split] = v;
+    }
+}
+)CU";
+
+struct NvrtcApi {
+    void *lib = nullptr;
+    decltype(&nvrtcCreateProgram) CreateProgram = nullptr;
+    decltype(&nvrtcCompileProgram) CompileProgram = nullptr;
+    decltype(&nvrtcGetProgramLogSize) GetProgramLogSize = nullptr;
+    decltype(&nvrtcGetProgramLog) GetProgramLog = nullptr;
+    decltype(&nvrtcGetCUBINSize) GetCUBINSize = nullptr;
+    decltype(&nvrtcGetCUBIN) GetCUBIN = nullptr;
+    decltype(&nvrtcDestroyProgram) DestroyProgram = nullptr;
+    decltype(&nvrtcGetErrorString) GetErrorString = nullptr;
+};
+static NvrtcApi g_nvrtc;
+static std::mutex g_custom_mu;                                   // the NVRTC table and the cubin cache
+static std::map<std::string, std::string> g_custom_cubin;        // source text -> sm_100a cubin
+
+static int nvrtc_load()                                          // under g_custom_mu
+{
+    if (g_nvrtc.lib) return 0;
+    void *lib = dlopen("libnvrtc.so.12", RTLD_NOW | RTLD_LOCAL);
+    if (!lib) { g_be_err = std::string("custom likelihoods need NVRTC: cannot load libnvrtc.so.12: ") + dlerror(); return -2; }
+#define SYM(field, sym) do { *(void **)(&g_nvrtc.field) = dlsym(lib, sym); if (!g_nvrtc.field) { g_be_err = std::string("libnvrtc misses ") + sym; dlclose(lib); return -2; } } while (0)
+    SYM(CreateProgram, "nvrtcCreateProgram"); SYM(CompileProgram, "nvrtcCompileProgram");
+    SYM(GetProgramLogSize, "nvrtcGetProgramLogSize"); SYM(GetProgramLog, "nvrtcGetProgramLog");
+    SYM(GetCUBINSize, "nvrtcGetCUBINSize"); SYM(GetCUBIN, "nvrtcGetCUBIN");
+    SYM(DestroyProgram, "nvrtcDestroyProgram"); SYM(GetErrorString, "nvrtcGetErrorString");
+#undef SYM
+    g_nvrtc.lib = lib;
+    return 0;
+}
+
+// the cubin of `source`, compiled on the first request (under g_custom_mu)
+static int custom_cubin(const char *source, const std::string **cubin)
+{
+    auto it = g_custom_cubin.find(source);
+    if (it != g_custom_cubin.end()) { *cubin = &it->second; return 0; }
+    if (int rc = nvrtc_load()) return rc;
+    const std::string text = std::string(CUSTOM_PRELUDE) + source + "\n" + CUSTOM_KERNEL;
+    nvrtcProgram prog = nullptr;
+    nvrtcResult r = g_nvrtc.CreateProgram(&prog, text.c_str(), "demcmc_custom.cu", 0, nullptr, nullptr);
+    if (r != NVRTC_SUCCESS) { g_be_err = std::string("nvrtcCreateProgram: ") + g_nvrtc.GetErrorString(r); return -1; }
+    // --fmad=false: the library's own arithmetic (csrc/Makefile) and the reference's, without contraction
+    const char *opts[] = { "-arch=sm_100a", "-std=c++17", "--fmad=false" };
+    r = g_nvrtc.CompileProgram(prog, 3, opts);
+    if (r != NVRTC_SUCCESS) {
+        size_t n = 0;
+        std::string log;
+        if (g_nvrtc.GetProgramLogSize(prog, &n) == NVRTC_SUCCESS && n > 1) { log.resize(n); g_nvrtc.GetProgramLog(prog, &log[0]); log.resize(n - 1); }
+        g_nvrtc.DestroyProgram(&prog);
+        g_be_err = "custom likelihood does not compile (" + std::string(g_nvrtc.GetErrorString(r)) + "):\n" + log;
+        return log.find("DEMCMC_NPAR is above") != std::string::npos ? -2 : -1;
+    }
+    size_t n = 0;
+    std::string bin;
+    r = g_nvrtc.GetCUBINSize(prog, &n);
+    if (r == NVRTC_SUCCESS) { bin.resize(n); r = g_nvrtc.GetCUBIN(prog, &bin[0]); }
+    g_nvrtc.DestroyProgram(&prog);
+    if (r != NVRTC_SUCCESS) { g_be_err = std::string("nvrtcGetCUBIN: ") + g_nvrtc.GetErrorString(r); return -1; }
+    *cubin = &(g_custom_cubin[source] = std::move(bin));
+    return 0;
+}
+
+int custom_compile(const char *source)
+{
+    std::lock_guard<std::mutex> lk(g_custom_mu);
+    const std::string *cubin = nullptr;
+    return custom_cubin(source, &cubin);
+}
+
+struct CustomModule { cudaLibrary_t lib; cudaKernel_t kernel; };
+
+int custom_load(const char *source, void **module, int *has_obs)
+{
+    *module = nullptr;
+    std::string cubin;
+    {
+        std::lock_guard<std::mutex> lk(g_custom_mu);
+        const std::string *c = nullptr;
+        if (int rc = custom_cubin(source, &c)) return rc;
+        cubin = *c;
+    }
+    CustomModule *mod = new CustomModule();
+    cudaError_t e = cudaLibraryLoadData(&mod->lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+    if (e != cudaSuccess) { delete mod; cu_fail(e, "cudaLibraryLoadData (custom likelihood)"); return -3; }
+    e = cudaLibraryGetKernel(&mod->kernel, mod->lib, "k_ll_custom");
+    void *flag = nullptr;
+    size_t bytes = 0;
+    if (e == cudaSuccess) e = cudaLibraryGetGlobal(&flag, &bytes, mod->lib, "demcmc_custom_has_obs");
+    if (e == cudaSuccess) e = cudaMemcpy(has_obs, flag, sizeof(int), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) { cudaLibraryUnload(mod->lib); delete mod; cu_fail(e, "loading k_ll_custom"); return -3; }
+    *module = mod;
+    return 0;
+}
+
+void custom_unload(void *module)
+{
+    if (!module) return;
+    CustomModule *mod = (CustomModule *)module;
+    cudaLibraryUnload(mod->lib);
+    delete mod;
+}
+
+static int launch_ll_custom(const ModelDev &m, const double *theta, const Level &lv, double *ll_part)
+{
+    if (!m.custom) { g_be_err = "custom likelihood not loaded"; return -1; }
+    const CustomModule *mod = (const CustomModule *)m.custom;
+    int d = m.d, n = lv.n, n_cols = m.n_cols, split_len = m.split_len, n_split = m.n_osplit * m.n_ksplit;
+    long long n_obs = m.n_obs;
+    const int *order = lv.order;
+    const double *x = m.x;
+    void *args[] = { &theta, &d, &order, &n, &x, &n_cols, &n_obs, &split_len, &n_split, &ll_part };
+    CU(cudaLaunchKernel((const void *)mod->kernel, dim3((lv.n + PW_TP - 1) / PW_TP, n_split), dim3(PW_THREADS), args, 0, stream()));
+    LAUNCHED("k_ll_custom");
+    return 0;
+}
+
 int launch_loglik(const ConfigDev &cfg, const ModelDev &m, const double *theta, const Level &lv, double *ll_part, long long *ll_acc)
 {
     (void)cfg;
@@ -2098,6 +2309,7 @@ int launch_loglik(const ConfigDev &cfg, const ModelDev &m, const double *theta, 
         if (!xs.bfrag || !xs.magic) { g_be_err = "mean staging buffer missing"; return -1; }
         return launch_xdot(m, xs, lv, ll_acc);
     }
+    if (m.kind == M_CUSTOM) return launch_ll_custom(m, theta, lv, ll_part);
     dim3 grid((lv.n + PW_TP - 1) / PW_TP, m.n_osplit);
     if (m.kind == M_GAUSSIAN) k_ll_pointwise<M_GAUSSIAN><<<grid, PW_THREADS, 0, stream()>>>(m, theta, lv, ll_part);
     else if (m.kind == M_LNR) k_ll_pointwise<M_LNR><<<grid, PW_THREADS, 0, stream()>>>(m, theta, lv, ll_part);

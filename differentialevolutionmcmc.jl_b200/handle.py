@@ -10,7 +10,8 @@ import numpy as np
 from . import _ffi
 from ._ffi import _bp, _dp, _ip, check, f8, ptr
 
-KINDS = {"gaussian": 0, "mvnormal": 1, "binomial": 2, "lnr": 3, "lba": 4, "hier_normal": 5, "rastrigin": 6, "mvnormal_full": 7}
+KINDS = {"gaussian": 0, "mvnormal": 1, "binomial": 2, "lnr": 3, "lba": 4, "hier_normal": 5, "rastrigin": 6, "mvnormal_full": 7,
+         "custom": 8}
 UPDATES = {"mh": 0, "maximize": 1, "minimize": 2}
 FITNESS = {"posterior": 0, "fun": 1}
 PRIORS = {"flat": 0, "normal": 1, "halfcauchy": 2, "uniform": 3, "beta": 4, "normal_ref": 5}
@@ -88,9 +89,12 @@ class Handle:
 
     # ---- model ---------------------------------------------------------------------------------
     def set_model(self, kind, prior, x=None, choice=None, sigma=None, lba_floor=1e-10, device_ptrs=None, n_obs=None,
-                  n_dim=0, n_per=0, center=None, cov=None):
+                  n_dim=0, n_per=0, center=None, cov=None, source=None, n_cols=None):
         """Bind a registered likelihood kernel.  `prior` is a list of (name, a, b, ref) per
         flattened parameter.  `device_ptrs=(x_ptr, choice_ptr)` passes data already in HBM.
+        kind="custom": `source` is the CUDA C++ text of the likelihood (include/demcmc_b200.h: DEMCMC_CUSTOM) and x an
+        n_obs-vector (n_cols = 1), an n_obs x n_cols matrix, or None (no observations); with device pointers pass
+        n_obs and n_cols.
         `center` (mvnormal / hier_normal, test hook): centre the data on this vector instead of on their
         column means, which makes the streamed cross term non-zero (demcmc_model.center)."""
         d = self.d
@@ -122,6 +126,15 @@ class Handle:
                 n_obs = 1
             elif kind == "rastrigin":
                 n_obs = 0
+            elif kind == "custom":
+                if x is None:
+                    n_obs, n_cols = 0, 0
+                elif xs.ndim == 1:
+                    n_obs, n_cols = xs.shape[0], 1
+                elif xs.ndim == 2:
+                    n_obs, n_cols = xs.shape
+                else:
+                    raise ValueError("custom data must be a vector or an n_obs x n_cols matrix")
             else:
                 n_obs = xs.shape[0]
                 if kind in ("lnr", "lba") and not n_dim:
@@ -133,8 +146,10 @@ class Handle:
         cv = None if cov is None else f8(cov)
         if kind == "mvnormal_full" and (cv is None or cv.shape != (int(n_dim), int(n_dim))):
             raise ValueError("mvnormal_full needs cov of shape (n_dim, n_dim)")
-        m = _ffi.Model(kind_id, d, int(n_obs), int(n_dim), int(n_per), xp, cp, ptr(sg, _dp), float(lba_floor), pr, on_dev, 0, ptr(cv, _dp), ptr(cen, _dp))
-        self._keep = [xs, cs, sg, pr, cen, cv]
+        src = None if source is None else source.encode() if isinstance(source, str) else bytes(source)
+        m = _ffi.Model(kind_id, d, int(n_obs), int(n_dim), int(n_per), xp, cp, ptr(sg, _dp), float(lba_floor), pr, on_dev,
+                       int(n_cols or 0), ptr(cv, _dp), ptr(cen, _dp), src)
+        self._keep = [xs, cs, sg, pr, cen, cv, src]
         check(_ffi.lib().demcmc_set_model(self._h, C.byref(m)))
 
     # ---- state ---------------------------------------------------------------------------------
@@ -313,6 +328,16 @@ class Handle:
     def comm_init(self, uid: bytes, rank: int, n_ranks: int):
         buf = np.frombuffer(uid, dtype=np.uint8).copy()
         check(_ffi.lib().demcmc_comm_init(self._h, ptr(buf, _bp), rank, n_ranks))
+
+
+def compile_loglike(source):
+    """Compiles a custom likelihood source for sm_100a (demcmc_compile_loglike; no device needed).  Raises DemcmcError
+    with the compiler log when it does not compile; the result is cached for later set_model calls."""
+    src = source.encode() if isinstance(source, str) else bytes(source)
+    log = C.create_string_buffer(1 << 16)
+    rc = _ffi.lib().demcmc_compile_loglike(src, log, len(log))
+    if rc != 0:
+        raise _ffi.DemcmcError(rc, log.value.decode(errors="replace") or _ffi.lib().demcmc_last_error().decode(errors="replace"))
 
 
 def comm_unique_id() -> bytes:

@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define DEMCMC_ABI_VERSION 4
+#define DEMCMC_ABI_VERSION 5
 
 enum { DEMCMC_OK = 0, DEMCMC_EINVAL = -1, DEMCMC_ENODEVICE = -2, DEMCMC_ECUDA = -3, DEMCMC_ENOMEM = -4,
        DEMCMC_ESTATE = -5, DEMCMC_EUNSUPPORTED = -6, DEMCMC_ECOMM = -7 };
@@ -37,7 +37,24 @@ enum { DEMCMC_GAUSSIAN = 0, DEMCMC_MVNORMAL = 1, DEMCMC_BINOMIAL = 2, DEMCMC_LNR
        DEMCMC_MVNORMAL_FULL = 7 /* sum(logpdf(MvNormal(mu, sigma^2 * Sigma), data)) with a KNOWN full covariance Sigma
                                    (demcmc_model.cov); parameters mu[n_dim], sigma: d = n_dim + 1 (SURVEY 8f-4).  The data are
                                    whitened once through the Cholesky factor (y = L^-1 x), every proposal's mean is whitened
-                                   when it is staged (nu = L^-1 mu), and the isotropic kernels stream y against nu */ };
+                                   when it is staged (nu = L^-1 mu), and the isotropic kernels stream y against nu */,
+       DEMCMC_CUSTOM = 8        /* a likelihood the caller writes in CUDA C++ (demcmc_model.source), compiled at run time for
+                                   sm_100a; see the source contract below */ };
+/* DEMCMC_CUSTOM source contract.  demcmc_model.source is CUDA C++ text (no #include) that defines
+ *   demcmc_obs       required (unless n_obs == 0): __device__ double, arguments (const double *par, const double *x): the
+ *                    log density of ONE observation; x = that observation's n_cols values (row i of demcmc_model.x)
+ *   demcmc_particle  optional: __device__ double, argument (const double *theta): a term added once per particle (constant
+ *                    terms, or the whole objective when n_obs == 0)
+ *   DEMCMC_NPAR      optional, with demcmc_prepare: __device__ void, arguments (const double *theta, double *par): a
+ *                    per-particle precompute hoisted out of the observation loop (e.g. log(sigma)) that fills
+ *                    par[DEMCMC_NPAR]; without it par = theta
+ * and the log-likelihood of theta[d] is demcmc_obs of (par, x_i) summed over the observations i, plus demcmc_particle of
+ * theta.  theta is the flattened parameter vector in `names` order; d and DEMCMC_NPAR are at most DEMCMC_CUSTOM_MAX_PAR.
+ * The observations are summed in a fixed order (per thread, then warp, then block, then split), so a value is the same from run to run and on any
+ * number of GPUs.  The CUDA math library (exp, log, lgamma, erfc, normcdf, ...) is available; DEMCMC_INF and
+ * DEMCMC_NAN are defined.  A custom model takes the level-by-level path only: the fused and persistent kernels are
+ * specialised to the registered kinds. */
+#define DEMCMC_CUSTOM_MAX_PAR 256
 /* (Examples/Guassian_Example_Vector.jl is the Gaussian model with `loglike(data, theta...)` destructuring its arguments:
  * DEMCMC_GAUSSIAN is its kernel, d = 2 whether the two parameters are named separately or as one 2-vector.) */
 /* de.update_particle! (src/utilities.jl:201-226): mh_update!, or the greedy maximize! / minimize! of
@@ -78,7 +95,8 @@ typedef struct {
     double lba_floor;       /* LBA density floor (1e-10 in SequentialSamplingModels), 0 disables */
     const demcmc_prior *prior; /* [d], host memory */
     int32_t data_on_device; /* 1: x / choice are device pointers on the handle's device */
-    int32_t reserved;
+    int32_t n_cols;         /* CUSTOM: values per observation, x[n_obs][n_cols] (= Julia n_cols x n_obs column-major);
+                               >= 1 when n_obs > 0.  Unused by the registered kinds */
     const double *cov;      /* MVNORMAL_FULL: covariance [n_dim][n_dim] (host memory), symmetric positive definite */
     const double *center;   /* MVNORMAL / HIER_NORMAL: NULL (the default) = the kernel centres the data on their column
                                means, x' = x - mean: the sum of squares is then  sum x'^2 - 2 B + n sum m'^2  with the
@@ -87,6 +105,7 @@ typedef struct {
                                stream was computed correctly.  center[n_dim] (host memory) centres on THAT vector
                                instead: B is then n (mean - center).m', not zero, and demcmc_get_trace_xdot /
                                demcmc_eval_xdot expose it, which is how the parity tests pin the DMMA kernels. */
+    const char *source;     /* CUSTOM: NUL-terminated CUDA C++ source (host memory), see DEMCMC_CUSTOM; else NULL */
 } demcmc_model;
 
 /* Mirrors the DE sampler struct field by field (src/structs.jl:57-131). */
@@ -176,6 +195,12 @@ int demcmc_create(const demcmc_config *cfg, demcmc_handle **out);
 int demcmc_destroy(demcmc_handle *h);
 /* DEModel(; loglike = GPULoglike(...), prior_loglike = ..., data) (src/structs.jl:176-189) */
 int demcmc_set_model(demcmc_handle *h, const demcmc_model *model);
+/* Compiles a DEMCMC_CUSTOM source for sm_100a with NVRTC (no device needed) and keeps the result in a per-process cache
+ * keyed by the source text, so a later demcmc_set_model with the same text does not compile again.  Returns 0, or
+ * DEMCMC_EINVAL with the compiler's log (user lines are reported as user.cu(<line>)) copied into log[log_cap] (may be
+ * NULL) and into demcmc_last_error(); DEMCMC_EUNSUPPORTED when libnvrtc.so.12 cannot be loaded or DEMCMC_NPAR is above
+ * DEMCMC_CUSTOM_MAX_PAR. */
+int demcmc_compile_loglike(const char *source, char *log, int64_t log_cap);
 /* initialize_samples (src/utilities.jl:29-41) when n_initial > 0: rows[n_initial][P][d], row i = the
  * i-th sample_prior() draw of every particle id; they become rows 1..n_initial of de.samples.  A sharded
  * job passes the rows of its own particles, [n_initial][P_local][d] -- unless sample = resample: then (after

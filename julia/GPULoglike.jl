@@ -23,9 +23,9 @@
 # GPU path with a closure throws an ArgumentError -- there is no silent CPU fallback.
 
 const LIBDEMCMC = get(ENV, "LIBDEMCMC_B200", "libdemcmc_b200.so")
-const DEMCMC_ABI_VERSION = Int32(4)
+const DEMCMC_ABI_VERSION = Int32(5)
 
-const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7)
+const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7, custom = 8)
 const GPU_PRIORS = (flat = 0, normal = 1, halfcauchy = 2, uniform = 3, beta = 4, normal_ref = 5)
 
 """
@@ -35,6 +35,12 @@ const GPU_PRIORS = (flat = 0, normal = 1, halfcauchy = 2, uniform = 3, beta = 4,
 `kind ∈ (:gaussian, :mvnormal, :binomial, :lnr, :lba, :hier_normal)`.  `x` is the data vector
 (`:gaussian`), the `n_dim × n_obs` matrix handed to `MvNormal` (`:mvnormal`) or the vector of
 per-subject vectors / `n_per × n_subj` matrix (`:hier_normal`).
+
+    GPULoglike(:custom, X; source)
+
+A likelihood written as CUDA C++ (`source`, the DEMCMC_CUSTOM contract of include/demcmc_b200.h: `demcmc_obs`, and
+optionally `demcmc_particle` / `DEMCMC_NPAR` + `demcmc_prepare`), compiled by the library for sm_100a.  `X` is a vector
+(one value per observation), an `n_cols × n_obs` matrix (one column per observation), or `nothing` (no data).
 """
 struct GPULoglike{D}
     kind::Symbol
@@ -42,6 +48,7 @@ struct GPULoglike{D}
     sigma::Union{Nothing, Vector{Float64}}
     lba_floor::Float64
     cov::Matrix{Float64}   # :mvnormal_full: the known covariance Σ of MvNormal(μ, σ²Σ); empty otherwise
+    source::String         # :custom: the CUDA C++ source of the likelihood; empty otherwise
 end
 
 function GPULoglike(kind::Symbol; x = nothing, choice = nothing, rt = nothing, N = nothing, k = nothing,
@@ -57,7 +64,17 @@ function GPULoglike(kind::Symbol; x = nothing, choice = nothing, rt = nothing, N
         (x = Array{Float64}(x), choice = nothing)
     end
     kind == :mvnormal_full && size(cov) != (size(data.x, 1), size(data.x, 1)) && throw(ArgumentError(":mvnormal_full needs cov, n_dim × n_dim"))
-    return GPULoglike(kind, data, sigma === nothing ? nothing : Vector{Float64}(sigma), Float64(lba_floor), Matrix{Float64}(cov))
+    return GPULoglike(kind, data, sigma === nothing ? nothing : Vector{Float64}(sigma), Float64(lba_floor), Matrix{Float64}(cov), "")
+end
+
+# the source is compiled when the model is bound (demcmc_set_model caches the cubin per source text); a source that
+# does not compile raises there, with the compiler log as the library's error message
+function GPULoglike(kind::Symbol, X; source::AbstractString)
+    kind == :custom || throw(ArgumentError("GPULoglike(kind, X; source) is the :custom form"))
+    isempty(source) && throw(ArgumentError(":custom needs the CUDA source of demcmc_obs"))
+    x = X === nothing ? zeros(0, 0) : X isa AbstractVector ? Matrix{Float64}(reshape(X, 1, :)) : Matrix{Float64}(X)
+    (X !== nothing && size(x, 1) == 0) && throw(ArgumentError(":custom data need at least one value per observation"))
+    return GPULoglike(kind, (x = x, choice = nothing), nothing, 1e-10, zeros(0, 0), String(source))
 end
 
 # the device evaluates it; calling it on the host is an error, never a fallback
@@ -126,9 +143,10 @@ struct CModel
     lba_floor::Float64
     prior::Ptr{CPrior}
     data_on_device::Int32
-    reserved::Int32
+    n_cols::Int32          # :custom: values per observation (rows of the n_cols × n_obs data matrix)
     cov::Ptr{Float64}      # :mvnormal_full: the known covariance, n_dim × n_dim
     center::Ptr{Float64}   # C_NULL: centre the data on their column means (the product default)
+    source::Ptr{UInt8}     # :custom: NUL-terminated CUDA source (a Julia String's pointer), else C_NULL
 end
 
 struct CConfig
@@ -259,9 +277,12 @@ function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_e
     priors = prior_table(model, Θ1)
     x = ll.data.x
     choice = ll.data.choice
-    n_dim, n_per, n_obs = 0, 0, length(x)
+    n_dim, n_per, n_obs, n_cols = 0, 0, length(x), 0
     covm = ll.cov
-    if ll.kind == :mvnormal || ll.kind == :mvnormal_full
+    src = ll.source
+    if ll.kind == :custom
+        n_cols, n_obs = size(x)
+    elseif ll.kind == :mvnormal || ll.kind == :mvnormal_full
         n_dim, n_obs = size(x)
     elseif ll.kind == :hier_normal
         n_per, n_dim = size(x); n_obs = n_dim * n_per
@@ -285,14 +306,15 @@ function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_e
     init_rows = de.n_initial > 0 ?
         Float64[flatten_theta(de.samples[i, :, p])[k] for k = 1:d, p = 1:P, i = 1:(de.n_initial)] : Float64[]
     sig = ll.sigma === nothing ? Float64[] : ll.sigma
-    GC.@preserve theta0 lo hi blocks priors x choice sig covm samples accept lp final_ids final_theta final_weight init_rows devs begin
+    GC.@preserve theta0 lo hi blocks priors x choice sig covm src samples accept lp final_ids final_theta final_weight init_rows devs begin
         cfg = CConfig(DEMCMC_ABI_VERSION, de.n_groups, de.Np, d, de.burnin, de.n_initial, de.α, de.β, de.ϵ, de.σ, de.κ,
             de.θsnooker, proposal_id(de), n_blocks, isempty(blocks) ? C_NULL : pointer(blocks), pointer(lo), pointer(hi),
             seed, device, 0, 0, donors, 0, 1, update, fitness, length(devs), isempty(devs) ? C_NULL : pointer(devs))
         demcmc_check(ccall((:demcmc_create, LIBDEMCMC), Cint, (Ref{CConfig}, Ref{Ptr{Cvoid}}), cfg, h))
         try
             m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), choice === nothing ? C_NULL : pointer(choice),
-                isempty(sig) ? C_NULL : pointer(sig), ll.lba_floor, pointer(priors), 0, 0, isempty(covm) ? C_NULL : pointer(covm), C_NULL)
+                isempty(sig) ? C_NULL : pointer(sig), ll.lba_floor, pointer(priors), 0, n_cols, isempty(covm) ? C_NULL : pointer(covm), C_NULL,
+                isempty(src) ? C_NULL : pointer(src))
             demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
             if n_blocks > 0 && !all(!iszero, block_on)         # block updating in some iterations only
                 GC.@preserve block_on demcmc_check(ccall((:demcmc_set_blocking_schedule, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Int64), h[], block_on, length(block_on)))
@@ -358,7 +380,7 @@ function _sample_gpu_thinned(model, de, n_iter; device, devices, store_every, se
             pointer(lo), pointer(hi), seed, device, 0, 0, 0, 0, store_every, 0, 0, length(devs), isempty(devs) ? C_NULL : pointer(devs))
         demcmc_check(ccall((:demcmc_create, LIBDEMCMC), Cint, (Ref{CConfig}, Ref{Ptr{Cvoid}}), cfg, h))
         try
-            m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), C_NULL, C_NULL, ll.lba_floor, pointer(priors), 0, 0, C_NULL, C_NULL)
+            m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), C_NULL, C_NULL, ll.lba_floor, pointer(priors), 0, 0, C_NULL, C_NULL, C_NULL)
             demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
             demcmc_check(ccall((:demcmc_set_state, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}), h[], theta0, C_NULL))
             demcmc_check(ccall((:demcmc_run, LIBDEMCMC), Cint, (Ptr{Cvoid}, Int64), h[], n_iter))
