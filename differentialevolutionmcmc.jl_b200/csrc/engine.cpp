@@ -13,6 +13,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <array>
 #include <vector>
 
@@ -887,90 +888,103 @@ int demcmc_set_state(demcmc_handle *h, const double *theta, const int32_t *ids)
     return 0;
 }
 
-static int run_impl(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter)
-{
-    if (!h || n_iter < 0) return fail(DEMCMC_EINVAL, "bad argument");
-    if (!h->has_model || !h->has_state) return fail(DEMCMC_ESTATE, "set_model and set_state must come before run");
-    BE(be::set_device(h->cfg.device));
-    const demcmc_config &cfg = h->cfg;
-    const int Np = cfg.Np, Gt = cfg.n_groups, G = h->G_local, P = h->P, d = h->d, B = h->B;
-    const int64_t Pt = (int64_t)Gt * Np, S = n_iter * B;
-    const int64_t pbeg = (int64_t)cfg.group_begin * Np;
-    if (h->n0 > 0 && !h->has_history) return fail(DEMCMC_ESTATE, "n_initial > 0: demcmc_set_history must come before run");
-    if (cfg.donors && G != Gt && h->n_ranks <= 1) return fail(DEMCMC_ESTATE, "sample = resample on a sharded job reads the history of every particle id: demcmc_comm_init must come first");
-    const bool ghist = cfg.donors && h->n_ranks > 1;              // donors come from the replicated history
-    h->dcfg.P_hist = ghist ? (int32_t)Pt : (int32_t)P;
-    if (cfg.donors && h->iter_offset > 0) return fail(DEMCMC_EUNSUPPORTED, "sample = resample draws donors from the rows of earlier iterations: a resumed handle does not hold them");
-    if (int rc = grow_history(h, stored_rows(h, h->iters_done + n_iter))) return rc;
-
-    // ---- replay: upload the local shard of the tape ------------------------------------------------
+namespace {
+// The local shard of a replay tape: the device arrays the sweep contexts point into and the host copies the planner
+// reads.  It owns its device buffers, so every return out of a run frees them.
+struct TapeShard {
     uint8_t *t_kind = nullptr, *t_keep = nullptr;
     int32_t *t_idx = nullptr, *t_idx_row = nullptr;
     double *t_g1 = nullptr, *t_g2 = nullptr, *t_uacc = nullptr, *t_noise = nullptr;
-    std::vector<uint8_t> hk;          // host copy of local kinds / idx for the planner
-    std::vector<int32_t> hi;
-    std::vector<void *> tmp;
-    auto cleanup = [&]() { for (void *p : tmp) be::dfree(p); tmp.clear(); };
-    if (tape) {
-        if (!tape->kind || !tape->idx || !tape->gamma1 || !tape->gamma2 || !tape->u_acc || !tape->noise)
-            return fail(DEMCMC_EINVAL, "tape misses a required array");
-        if (cfg.kappa != 1.0 && !tape->keep) return fail(DEMCMC_EINVAL, "kappa != 1 needs tape.keep");
-        if (Gt > 1 && (!tape->mig_n || !tape->mig_groups || !tape->mig_pick_u)) return fail(DEMCMC_EINVAL, "tape misses the migration arrays");
-        if (cfg.donors && !tape->idx_row) return fail(DEMCMC_EINVAL, "sample = resample needs tape.idx_row");
-        auto shard = [&](const void *src, size_t elem, size_t per_particle) -> void * {
-            // [S][Pt][per] -> [S][P][per]
-            const size_t rowb = elem * per_particle;
-            std::vector<uint8_t> buf((size_t)S * P * rowb);
-            for (int64_t s = 0; s < S; ++s)
-                memcpy(buf.data() + (size_t)s * P * rowb, (const uint8_t *)src + ((size_t)s * Pt + pbeg) * rowb, (size_t)P * rowb);
-            void *p = be::dmalloc(std::max<size_t>(8, buf.size()));
-            if (!p) return nullptr;
-            tmp.push_back(p);
-            if (!buf.empty() && (be::h2d(p, buf.data(), buf.size()) || be::sync())) return nullptr;
-            return p;
-        };
-        t_kind = (uint8_t *)shard(tape->kind, 1, 1);
-        t_idx = (int32_t *)shard(tape->idx, 4, 3);
-        if (cfg.donors) t_idx_row = (int32_t *)shard(tape->idx_row, 4, 3);
-        t_g1 = (double *)shard(tape->gamma1, 8, 1);
-        t_g2 = (double *)shard(tape->gamma2, 8, 1);
-        t_uacc = (double *)shard(tape->u_acc, 8, 1);
-        t_noise = (double *)shard(tape->noise, 8, d);
-        if (cfg.kappa != 1.0) t_keep = (uint8_t *)shard(tape->keep, 1, d);
-        if (!t_kind || !t_idx || (cfg.donors && !t_idx_row) || !t_g1 || !t_g2 || !t_uacc || !t_noise || (cfg.kappa != 1.0 && !t_keep)) { cleanup(); return fail(DEMCMC_ENOMEM, "tape upload failed: %s", be::last_error()); }
-        hk.resize((size_t)S * P); hi.resize((size_t)S * P * 3);
-        for (int64_t s = 0; s < S; ++s) {
-            memcpy(hk.data() + (size_t)s * P, tape->kind + (size_t)s * Pt + pbeg, P);
-            memcpy(hi.data() + (size_t)s * P * 3, tape->idx + ((size_t)s * Pt + pbeg) * 3, sizeof(int32_t) * P * 3);
-        }
-        for (size_t i = 0; i < hk.size(); ++i) if (hk[i] > KIND_MUTATION) { cleanup(); return fail(DEMCMC_EINVAL, "tape.kind[%zu] = %d", i, hk[i]); }
-        for (size_t i = 0; i < hi.size(); ++i) {
-            const uint8_t k = hk[i / 3];
-            if (k == KIND_MUTATION) continue;
-            const bool base = k == KIND_DE && i % 3 == 0;          // slot of the base particle in the group, or -1
-            if (base && hi[i] < 0) continue;
-            const int64_t lim = (cfg.donors && !base) ? Pt : Np;   // resample donors are particle ids
-            if (hi[i] < 0 || hi[i] >= lim) { cleanup(); return fail(DEMCMC_EINVAL, "tape.idx[%zu] = %d out of range", i, hi[i]); }
-            if (cfg.donors && !base) {
-                const int64_t sw = (int64_t)(i / 3) / P, pl = (int64_t)(i / 3) % P;
-                const int64_t ub = stored_rows(h, h->iters_done + sw / B);                   // rows 1:de.iter-1
-                const int32_t r = tape->idx_row[((size_t)sw * Pt + pbeg + pl) * 3 + i % 3];
-                if (r < 0 || r >= ub) { cleanup(); return fail(DEMCMC_EINVAL, "tape.idx_row of sweep %lld particle %lld = %d outside the %lld stored rows", (long long)sw, (long long)pl, r, (long long)ub); }
-            }
+    std::vector<uint8_t> hk; std::vector<int32_t> hi;             // host copies of the local kinds and idx, for the planner
+    TapeShard() = default; TapeShard(const TapeShard &) = delete; TapeShard &operator=(const TapeShard &) = delete;
+    ~TapeShard() { for (void *p : { (void *)t_kind, (void *)t_idx, (void *)t_idx_row, (void *)t_g1, (void *)t_g2, (void *)t_uacc, (void *)t_noise, (void *)t_keep }) be::dfree(p); }
+};
+
+// what the steps of one run_impl call share
+struct RunCall {
+    const demcmc_tape *tape = nullptr;                            // replay, else nullptr
+    TapeShard shard;
+    int64_t n_iter = 0, S = 0;
+    bool ghist = false;                                           // donors come from the replicated history
+    bool skip_stream = false;                                     // the likelihood needs no O(N d) stream (demcmc_set_sufficient_stat)
+    int persist_lanes = 0, n_lanes = 1;                           // lanes of the persistent chunk kernel (0: not used), lanes launched
+    std::vector<std::pair<int64_t, int>> mig_events;              // iterations that migrated, and how many groups
+    // timing events: one pair per chunk when the L2 flush is on; the likelihood launches get their own pairs after those
+    size_t tev_ll0 = 0, tev_ll = 0, tev_chunks = 0;
+    int64_t n_levels = 0, sweeps_run = 0, chunks_this_call = 0;
+    double host_plan_s = 0.0, host_chunk_s = 0.0;
+    ChunkPlan plans[be::MAX_LANES];
+};
+
+// one chunk: `n_sw` consecutive sweeps starting at local iteration it0 (block b0), staged in ring slot u; lane_off[ln]:
+// the first entry of lane ln in u.d_order
+struct Chunk { int64_t it0; int b0, n_sw; bool blocked; Upload &u; bool basedep[MAX_CHUNK]; int32_t lane_off[be::MAX_LANES + 1]; };
+
+// DEMCMC_HOST_PROFILE=1: host seconds spent planning and launching, printed per call (stderr)
+bool host_profile() { static const bool on = [] { const char *e = getenv("DEMCMC_HOST_PROFILE"); return e && e[0] == '1'; }(); return on; }
+double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+struct HostTimer { double &acc; const double t0 = host_profile() ? now_s() : 0.0; ~HostTimer() { if (host_profile()) acc += now_s() - t0; } };
+} // namespace
+
+// validates a replay tape and uploads this handle's shard of it
+static int load_tape(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter, TapeShard &ts)
+{
+    const demcmc_config &cfg = h->cfg;
+    const int Np = cfg.Np, Gt = cfg.n_groups, P = h->P, d = h->d, B = h->B;
+    const int64_t Pt = (int64_t)Gt * Np, S = n_iter * B, pbeg = (int64_t)cfg.group_begin * Np;
+    if (!tape->kind || !tape->idx || !tape->gamma1 || !tape->gamma2 || !tape->u_acc || !tape->noise)
+        return fail(DEMCMC_EINVAL, "tape misses a required array");
+    if (cfg.kappa != 1.0 && !tape->keep) return fail(DEMCMC_EINVAL, "kappa != 1 needs tape.keep");
+    if (Gt > 1 && (!tape->mig_n || !tape->mig_groups || !tape->mig_pick_u)) return fail(DEMCMC_EINVAL, "tape misses the migration arrays");
+    if (cfg.donors && !tape->idx_row) return fail(DEMCMC_EINVAL, "sample = resample needs tape.idx_row");
+    auto slice = [&](const auto *src, size_t per) {           // [S][Pt][per] -> [S][P][per]
+        std::vector<std::remove_const_t<std::remove_reference_t<decltype(*src)>>> v((size_t)S * P * per);
+        for (int64_t s = 0; s < S; ++s) std::copy_n(src + ((size_t)s * Pt + pbeg) * per, (size_t)P * per, v.data() + (size_t)s * P * per);
+        return v;
+    };
+    auto upload = [](auto *&dst, const auto &v) {
+        const size_t bytes = sizeof v[0] * v.size();
+        dst = (std::remove_reference_t<decltype(dst)>)be::dmalloc(std::max<size_t>(8, bytes));
+        return dst && (!bytes || !(be::h2d(dst, v.data(), bytes) || be::sync()));
+    };
+    ts.hk = slice(tape->kind, 1); ts.hi = slice(tape->idx, 3);
+    if (!upload(ts.t_kind, ts.hk) || !upload(ts.t_idx, ts.hi) || (cfg.donors && !upload(ts.t_idx_row, slice(tape->idx_row, 3))) ||
+        !upload(ts.t_g1, slice(tape->gamma1, 1)) || !upload(ts.t_g2, slice(tape->gamma2, 1)) || !upload(ts.t_uacc, slice(tape->u_acc, 1)) ||
+        !upload(ts.t_noise, slice(tape->noise, d)) || (cfg.kappa != 1.0 && !upload(ts.t_keep, slice(tape->keep, d))))
+        return fail(DEMCMC_ENOMEM, "tape upload failed: %s", be::last_error());
+    const std::vector<uint8_t> &hk = ts.hk; const std::vector<int32_t> &hi = ts.hi;
+    for (size_t i = 0; i < hk.size(); ++i) if (hk[i] > KIND_MUTATION) return fail(DEMCMC_EINVAL, "tape.kind[%zu] = %d", i, hk[i]);
+    for (size_t i = 0; i < hi.size(); ++i) {
+        const uint8_t k = hk[i / 3];
+        if (k == KIND_MUTATION) continue;
+        const bool base = k == KIND_DE && i % 3 == 0;          // slot of the base particle in the group, or -1
+        if (base && hi[i] < 0) continue;
+        const int64_t lim = (cfg.donors && !base) ? Pt : Np;   // resample donors are particle ids
+        if (hi[i] < 0 || hi[i] >= lim) return fail(DEMCMC_EINVAL, "tape.idx[%zu] = %d out of range", i, hi[i]);
+        if (cfg.donors && !base) {
+            const int64_t sw = (int64_t)(i / 3) / P, pl = (int64_t)(i / 3) % P;
+            const int64_t ub = stored_rows(h, h->iters_done + sw / B);                   // rows 1:de.iter-1
+            const int32_t r = tape->idx_row[((size_t)sw * Pt + pbeg + pl) * 3 + i % 3];
+            if (r < 0 || r >= ub) return fail(DEMCMC_EINVAL, "tape.idx_row of sweep %lld particle %lld = %d outside the %lld stored rows", (long long)sw, (long long)pl, r, (long long)ub);
         }
     }
+    return 0;
+}
 
-    // ---- trace and migration log of this call ------------------------------------------------------
+// the trace and the migration log of this call
+static int reset_call_buffers(demcmc_handle *h, const RunCall &call)
+{
+    const int64_t S = call.S, n_iter = call.n_iter; const size_t P = h->P, d = h->d;
     be::dfree(h->tr_theta); be::dfree(h->tr_w); be::dfree(h->tr_adj); be::dfree(h->tr_acc); be::dfree(h->tr_xdot);
     h->tr_theta = h->tr_w = h->tr_adj = h->tr_xdot = nullptr; h->tr_acc = nullptr; h->tr_sweeps = 0;
     const bool ssd_model = is_ssd(h->dmodel.kind);
-    if (cfg.trace && S > 0) {
+    if (h->cfg.trace && S > 0) {
         h->tr_theta = (double *)be::dmalloc(sizeof(double) * S * P * d);
         h->tr_w = (double *)be::dmalloc(sizeof(double) * S * P);
         h->tr_adj = (double *)be::dmalloc(sizeof(double) * S * P);
         h->tr_acc = (uint8_t *)be::dmalloc((size_t)S * P);
         if (ssd_model) h->tr_xdot = (double *)be::dmalloc(sizeof(double) * S * P);
-        if (!h->tr_theta || !h->tr_w || !h->tr_adj || !h->tr_acc || (ssd_model && !h->tr_xdot)) { cleanup(); return fail(DEMCMC_ENOMEM, "trace buffers do not fit"); }
+        if (!h->tr_theta || !h->tr_w || !h->tr_adj || !h->tr_acc || (ssd_model && !h->tr_xdot)) return fail(DEMCMC_ENOMEM, "trace buffers do not fit");
         if (h->tr_xdot) BE(be::dzero(h->tr_xdot, sizeof(double) * S * P));
         if (!h->block_on.empty()) {                              // sweep slots of unblocked iterations stay unused: read as zero
             BE(be::dzero(h->tr_theta, sizeof(double) * S * P * d)); BE(be::dzero(h->tr_w, sizeof(double) * S * P));
@@ -979,388 +993,375 @@ static int run_impl(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter)
         h->tr_sweeps = S;
     }
     be::dfree(h->d_mig_log); h->d_mig_log = nullptr; h->mig_log_iters = n_iter;
-    h->last_mig_slots.assign((size_t)std::max<int64_t>(1, n_iter) * Gt, -1);
-    std::vector<std::pair<int64_t, MigSchedule>> mig_events;      // iterations that migrated
+    h->last_mig_slots.assign((size_t)std::max<int64_t>(1, n_iter) * h->cfg.n_groups, -1);
     if (n_iter > 0) {
         h->d_mig_log = (int32_t *)be::dmalloc(sizeof(int32_t) * n_iter * MAX_MIG);
-        if (!h->d_mig_log) { cleanup(); return fail(DEMCMC_ENOMEM, "migration log"); }
+        if (!h->d_mig_log) return fail(DEMCMC_ENOMEM, "migration log");
         BE(be::dfill(h->d_mig_log, 0xFF, sizeof(int32_t) * n_iter * MAX_MIG));   // -1: a cycle this rank took no part in
     }
+    return 0;
+}
 
-    const int64_t launches0 = be::launch_count();
-    int64_t n_levels = 0;
-    // timing events: one pair per chunk when the L2 flush is on; the likelihood launches get their
-    // own pairs after those
-    size_t tev_need = (h->flush_bytes ? 2 * (size_t)n_iter : 0), tev_ll0 = tev_need, tev_ll = 0, tev_chunks = 0;
-    if (h->time_loglik) tev_need += 2 * (size_t)S * 64;
-    while (h->tev.size() < tev_need) { void *e = be::tevent_create(); if (!e) { cleanup(); return fail(DEMCMC_ECUDA, "event pool: %s", be::last_error()); } h->tev.push_back(e); }
-    BE(be::timer_start());
-    ChunkPlan plans[be::MAX_LANES];
-    MigSchedule ms;
+static void get_mig(const demcmc_handle *h, const RunCall &call, int64_t it, MigSchedule &out)
+{
+    const int Gt = h->cfg.n_groups;
+    const demcmc_tape *tape = call.tape;
+    out.migrate = false; out.n = 0; out.groups.clear(); out.u_pick.clear();
+    if (Gt < 2) return;
+    if (!tape) return plan_migration(h->cfg.seed, (uint32_t)(h->iter_offset + h->iters_done + it), Gt, h->cfg.alpha, out);
+    out.n = tape->mig_n[it]; out.migrate = out.n > 0;
+    for (int i = 0; i < out.n; ++i) { out.groups.push_back(tape->mig_groups[it * Gt + i]); out.u_pick.push_back(tape->mig_pick_u[it * Gt + i]); }
+}
+static bool in_burnin_at(const demcmc_handle *h, int64_t it) { return h->iter_offset + h->iters_done + it + 1 + h->cfg.n_initial <= h->cfg.burnin; }   // de.iter <= burnin
+// native select_base reads the sweep-start weights: such a sweep starts from a complete state
+static bool needs_snapshot(const demcmc_handle *h, const RunCall &call, int64_t it) { return !call.tape && h->cfg.proposal == DEMCMC_RANDOM_GAMMA && in_burnin_at(h, it); }
+// blocking_on(de) (main.jl:137,162) of local iteration `it`
+static bool blocking_at(const demcmc_handle *h, int64_t it)
+{
+    const int64_t a = h->iter_offset + h->iters_done + it;
+    return h->B > 1 && (a >= (int64_t)h->block_on.size() || h->block_on[(size_t)a] != 0);
+}
 
-    auto get_mig = [&](int64_t it, MigSchedule &out) {
-        out.migrate = false; out.n = 0; out.groups.clear(); out.u_pick.clear();
-        if (Gt < 2) return;
-        if (tape) {
-            out.n = tape->mig_n[it]; out.migrate = out.n > 0;
-            for (int i = 0; i < out.n; ++i) { out.groups.push_back(tape->mig_groups[it * Gt + i]); out.u_pick.push_back(tape->mig_pick_u[it * Gt + i]); }
-        } else {
-            plan_migration(cfg.seed, (uint32_t)(h->iter_offset + h->iters_done + it), Gt, cfg.alpha, out);
+// the sweep contexts of a chunk, and the rows its sweeps write: the current state moves to the chunk's last row
+static void fill_sweep_contexts(demcmc_handle *h, const RunCall &call, Chunk &ck)
+{
+    const int G = h->G_local, P = h->P, d = h->d, B = h->B;
+    const TapeShard &ts = call.shard; const bool blocked = ck.blocked, ghist = call.ghist;
+    const int64_t itg0 = h->iters_done + ck.it0;
+    Row cur = cur_row(h);
+    for (int s = 0; s < ck.n_sw; ++s) {
+        // a chunk of blocked sweeps walks the blocks of consecutive iterations: sweep s is block (b0 + s) % B of
+        // iteration it0 + (b0 + s) / B; an unblocked chunk holds one sweep per iteration
+        const int b = blocked ? (ck.b0 + s) % B : 0;
+        const int64_t it = ck.it0 + (blocked ? (ck.b0 + s) / B : s), itg = itg0 + (blocked ? (ck.b0 + s) / B : s);
+        const bool last = !blocked || b == B - 1;             // this sweep completes its iteration
+        const int64_t s_local = it * B + b;
+        const bool inb = in_burnin_at(h, it);
+        ck.basedep[s] = call.tape && h->cfg.proposal == DEMCMC_RANDOM_GAMMA && inb;
+        // destination row: the history row of the iteration on its last block, else scratch
+        // (thinning: only every k_store-th iteration has a history row; the others live in the scratch ring,
+        // whose MAX_CHUNK + 2 rows keep every row of a chunk write-once)
+        const bool stored = last && (itg + 1) % h->k_store == 0;
+        const int64_t hist_row = h->n0 + (itg + 1) / h->k_store - 1;
+        Row next;
+        int next_scratch = -1;
+        if (stored) next = row_of(h, true, hist_row);
+        else {
+            // never the row of an earlier sweep of this chunk: overlapped sweeps read each other's rows out of
+            // order (a late update of sweep t still reads row t-1 while sweep t+3 is being written)
+            next_scratch = h->scr_cursor = (h->scr_cursor + 1) % h->n_scratch;
+            if (h->cur_hist < 0 && next_scratch == h->cur_scratch) next_scratch = h->scr_cursor = (h->scr_cursor + 1) % h->n_scratch;
+            next = row_of(h, false, next_scratch);
         }
-    };
-    auto in_burnin_at = [&](int64_t it) { return h->iter_offset + h->iters_done + it + 1 + cfg.n_initial <= cfg.burnin; };   // de.iter <= burnin
-    // native select_base reads the sweep-start weights: such a sweep starts from a complete state
-    auto needs_snapshot = [&](int64_t it) { return !tape && cfg.proposal == DEMCMC_RANDOM_GAMMA && in_burnin_at(it); };
+        SweepCtx &ctx = ck.u.h_ctx[s];
+        memset(&ctx, 0, sizeof ctx);
+        ctx.sweep = (uint32_t)((h->iter_offset + itg) * B + b); ctx.block = blocked ? b : -1; ctx.in_burnin = inb; ctx.replay = call.tape != nullptr;
+        ctx.exact_base = call.tape != nullptr;
+        ctx.cur_theta = cur.theta; ctx.cur_w = cur.w; ctx.cur_id = cur.id;
+        ctx.next_theta = next.theta; ctx.next_w = next.w; ctx.next_id = next.id; ctx.next_acc = next.acc;
+        ctx.mutate = ck.u.d_mut + (size_t)s * G;
+        ctx.plan = (call.tape || !h->plan_recs) ? nullptr : h->plan_recs + (size_t)s * P;
+        if (call.tape) {
+            ctx.t_kind = ts.t_kind + (size_t)s_local * P; ctx.t_idx = ts.t_idx + (size_t)s_local * P * 3;
+            ctx.t_g1 = ts.t_g1 + (size_t)s_local * P; ctx.t_g2 = ts.t_g2 + (size_t)s_local * P; ctx.t_uacc = ts.t_uacc + (size_t)s_local * P;
+            ctx.t_noise = ts.t_noise + (size_t)s_local * P * d; ctx.t_keep = ts.t_keep ? ts.t_keep + (size_t)s_local * P * d : nullptr;
+            ctx.t_idx_row = ts.t_idx_row ? ts.t_idx_row + (size_t)s_local * P * 3 : nullptr;
+        }
+        ctx.prop_theta = h->prop_theta; ctx.prop_prior = h->prop_prior; ctx.prop_adj = h->prop_adj; ctx.prop_inb = h->prop_inb; ctx.prop_msq = h->prop_msq;
+        ctx.ll_part = h->ll_part; ctx.ll_acc = h->ll_acc; ctx.ll_q = h->ll_q;
+        ctx.base_cw = h->base_cw; ctx.base_tot = h->base_tot;
+        // resample: donors are (row, id) cells of the rows stored before this iteration (crossover.jl:115)
+        ctx.hist_theta = ghist ? h->ghist_theta : h->hist_theta; ctx.hist_pos = ghist ? h->ghist_pos : h->hist_pos; ctx.donor_rows = stored_rows(h, itg);
+        ctx.next_pos = (stored && h->hist_pos && !ghist) ? h->hist_pos + (size_t)hist_row * P : nullptr;
+        if (h->tr_sweeps) {
+            ctx.tr_theta = h->tr_theta + (size_t)s_local * P * d; ctx.tr_w = h->tr_w + (size_t)s_local * P;
+            ctx.tr_adj = h->tr_adj + (size_t)s_local * P; ctx.tr_acc = h->tr_acc + (size_t)s_local * P;
+            ctx.tr_xdot = h->tr_xdot ? h->tr_xdot + (size_t)s_local * P : nullptr;
+        }
+        if (stored) { h->cur_hist = hist_row; }
+        else { h->cur_hist = -1; h->cur_scratch = next_scratch; }
+        cur = next;
+    }
+}
 
-    // runs `n_sw` consecutive sweeps starting at local iteration it0 (block b) as one chunk
-    // blocking_on(de) (main.jl:137,162) of local iteration `it`
-    auto blocking_at = [&](int64_t it) {
-        if (B <= 1) return false;
-        const int64_t a = h->iter_offset + h->iters_done + it;
-        return a >= (int64_t)h->block_on.size() || h->block_on[(size_t)a] != 0;
-    };
-    int64_t sweeps_run = 0;
-    // DEMCMC_HOST_PROFILE=1: host seconds spent planning and launching, printed per call (stderr)
-    static const bool host_prof = [] { const char *e = getenv("DEMCMC_HOST_PROFILE"); return e && e[0] == '1'; }();
-    double host_plan_s = 0.0, host_chunk_s = 0.0;
-    auto now_s = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    auto run_chunk = [&](int64_t it0, int b0, int n_sw, bool blocked) -> int {
-        sweeps_run += n_sw;
-        const double t_chunk0 = host_prof ? now_s() : 0.0;
-        struct ChunkTimer { double &acc; double t0; bool on; std::function<double()> now; ~ChunkTimer() { if (on) acc += now() - t0; } } chunk_timer{ host_chunk_s, t_chunk0, host_prof, now_s };
-        const int64_t itg0 = h->iters_done + it0;
-        Upload &u = h->ring[h->ring_use % demcmc_handle::RING];
-        if (u.armed) BE(be::event_wait(u.copied));             // the pinned slot is free once its copies ran
-        h->ring_use++;
-        bool basedep[MAX_CHUNK];
-        Row cur = cur_row(h);
-        for (int s = 0; s < n_sw; ++s) {
-            // a chunk of blocked sweeps walks the blocks of consecutive iterations: sweep s is block (b0 + s) % B of
-            // iteration it0 + (b0 + s) / B; an unblocked chunk holds one sweep per iteration
-            const int b = blocked ? (b0 + s) % B : 0;
-            const int64_t it = it0 + (blocked ? (b0 + s) / B : s), itg = itg0 + (blocked ? (b0 + s) / B : s);
-            const bool last = !blocked || b == B - 1;             // this sweep completes its iteration
-            const int64_t s_local = it * B + b;
-            const bool inb = in_burnin_at(it);
-            basedep[s] = tape && cfg.proposal == DEMCMC_RANDOM_GAMMA && inb;
-            // destination row: the history row of the iteration on its last block, else scratch
-            // (thinning: only every k_store-th iteration has a history row; the others live in the scratch ring,
-            // whose MAX_CHUNK + 2 rows keep every row of a chunk write-once)
-            const bool stored = last && (itg + 1) % h->k_store == 0;
-            const int64_t hist_row = h->n0 + (itg + 1) / h->k_store - 1;
-            Row next;
-            int next_scratch = -1;
-            if (stored) next = row_of(h, true, hist_row);
-            else {
-                // never the row of an earlier sweep of this chunk: overlapped sweeps read each other's rows out of
-                // order (a late update of sweep t still reads row t-1 while sweep t+3 is being written)
-                next_scratch = h->scr_cursor = (h->scr_cursor + 1) % h->n_scratch;
-                if (h->cur_hist < 0 && next_scratch == h->cur_scratch) next_scratch = h->scr_cursor = (h->scr_cursor + 1) % h->n_scratch;
-                next = row_of(h, false, next_scratch);
-            }
-            SweepCtx &ctx = u.h_ctx[s];
-            memset(&ctx, 0, sizeof ctx);
-            ctx.sweep = (uint32_t)((h->iter_offset + itg) * B + b); ctx.block = blocked ? b : -1; ctx.in_burnin = inb; ctx.replay = tape != nullptr;
-            ctx.exact_base = tape != nullptr;
-            ctx.cur_theta = cur.theta; ctx.cur_w = cur.w; ctx.cur_id = cur.id;
-            ctx.next_theta = next.theta; ctx.next_w = next.w; ctx.next_id = next.id; ctx.next_acc = next.acc;
-            ctx.mutate = u.d_mut + (size_t)s * G;
-            ctx.plan = (tape || !h->plan_recs) ? nullptr : h->plan_recs + (size_t)s * P;
-            if (tape) {
-                ctx.t_kind = t_kind + (size_t)s_local * P; ctx.t_idx = t_idx + (size_t)s_local * P * 3;
-                ctx.t_g1 = t_g1 + (size_t)s_local * P; ctx.t_g2 = t_g2 + (size_t)s_local * P; ctx.t_uacc = t_uacc + (size_t)s_local * P;
-                ctx.t_noise = t_noise + (size_t)s_local * P * d; ctx.t_keep = t_keep ? t_keep + (size_t)s_local * P * d : nullptr;
-                ctx.t_idx_row = t_idx_row ? t_idx_row + (size_t)s_local * P * 3 : nullptr;
-            }
-            ctx.prop_theta = h->prop_theta; ctx.prop_prior = h->prop_prior; ctx.prop_adj = h->prop_adj; ctx.prop_inb = h->prop_inb; ctx.prop_msq = h->prop_msq;
-            ctx.ll_part = h->ll_part; ctx.ll_acc = h->ll_acc; ctx.ll_q = h->ll_q;
-            ctx.base_cw = h->base_cw; ctx.base_tot = h->base_tot;
-            // resample: donors are (row, id) cells of the rows stored before this iteration (crossover.jl:115)
-            ctx.hist_theta = ghist ? h->ghist_theta : h->hist_theta; ctx.hist_pos = ghist ? h->ghist_pos : h->hist_pos; ctx.donor_rows = stored_rows(h, itg);
-            ctx.next_pos = (stored && h->hist_pos && !ghist) ? h->hist_pos + (size_t)hist_row * P : nullptr;
-            if (h->tr_sweeps) {
-                ctx.tr_theta = h->tr_theta + (size_t)s_local * P * d; ctx.tr_w = h->tr_w + (size_t)s_local * P;
-                ctx.tr_adj = h->tr_adj + (size_t)s_local * P; ctx.tr_acc = h->tr_acc + (size_t)s_local * P;
-                ctx.tr_xdot = h->tr_xdot ? h->tr_xdot + (size_t)s_local * P : nullptr;
-            }
-            if (stored) { h->cur_hist = hist_row; }
-            else { h->cur_hist = -1; h->cur_scratch = next_scratch; }
-            cur = next;
-        }
-        // Lanes: the groups split into independent sets (groups never read each other between
-        // migrations), each planned on its own and launched as its own kernel chain on its own
-        // stream, so one lane's likelihood kernel runs while the other lane proposes / accepts.
-        // the persistent chunk kernel alternates the levels of two lanes; the level-by-level path
-        // runs the handle's lanes (default 1) as concurrent kernel chains
-        const bool skip_stream = h->suffstat && ssd_model;       // B == 0 analytically: propose -> accept, nothing streamed
-        const int persist_lanes = skip_stream ? 0 : be::chunk_persist_lanes(h->dcfg, h->dmodel);
-        const int n_lanes = persist_lanes ? persist_lanes : std::max(1, std::min(h->n_lanes, G));
-        int32_t lane_off[be::MAX_LANES + 1] = { 0 };              // entries of each lane in u.d_order
-        std::vector<uint8_t> mut((size_t)n_sw * G, 0);
-        for (int ln = 0; ln < n_lanes; ++ln) {
-            const int g0 = (ln * G + n_lanes - 1) / n_lanes, g1 = ((ln + 1) * G + n_lanes - 1) / n_lanes;   // contiguous sets of groups
-            PlanInput pin;
-            pin.seed = cfg.seed; pin.Np = Np; pin.G_local = g1 - g0; pin.group_begin = cfg.group_begin + g0; pin.G_total = Gt;
-            pin.pos_offset = g0 * Np; pin.P_stride = blocked ? P : P * B;   // consecutive sweeps of an unblocked chunk are consecutive iterations;
-                                                                            // those of a blocked one are consecutive blocks (adjacent in the tape)
-            pin.sweep_stride = blocked ? 1 : B;
-            {
-                const char *e = getenv("DEMCMC_SHAPE");       // 0 = off, else the modulus (A/B runs)
-                const int mod = e ? atoi(e) : 8;
-                pin.shape_octets = (is_ssd(h->dmodel.kind)) ? std::max(0, mod) : 0;
-                const char *ec = getenv("DEMCMC_LEVEL_CAP");
-                // levels of at most 112 updates (14 octets) for the persistent chunk kernel: measured on configs[1] against
-                // no cap / 64 / 96 / 104 / 120 / 128: 2.86 M updates/s against 2.83 / 2.64 / 2.75 / 2.82 / 2.80 / 2.83
-                pin.level_cap = persist_lanes ? (ec ? std::max(0, atoi(ec)) : 112) : 0;
-            }
-            pin.proposal = cfg.proposal; pin.beta = cfg.beta; pin.theta_snooker = cfg.theta_snooker; pin.resample = cfg.donors != 0;
-            const int64_t s_first = it0 * B + (blocked ? b0 : 0);
-            pin.t_kind = tape ? hk.data() + (size_t)s_first * P : nullptr;       // a chunk of several sweeps is unblocked: its sweeps are P_stride apart in the tape
-            pin.t_idx = tape ? hi.data() + (size_t)s_first * P * 3 : nullptr;
-            const double t_plan0 = host_prof ? now_s() : 0.0;
-            plan_chunk(pin, (uint32_t)((h->iter_offset + itg0) * B + (blocked ? b0 : 0)), n_sw, basedep, plans[ln]);
-            if (host_prof) host_plan_s += now_s() - t_plan0;
-            const ChunkPlan &pl = plans[ln];
-            memcpy(u.h_order + lane_off[ln], pl.order.data(), sizeof(int32_t) * pl.order.size());
-            lane_off[ln + 1] = lane_off[ln] + (int32_t)pl.order.size();
-            for (int s2 = 0; s2 < n_sw; ++s2)
-                for (int g = g0; g < g1; ++g) mut[(size_t)s2 * G + g] = pl.mutate[(size_t)s2 * (g1 - g0) + (g - g0)];
-        }
-        memcpy(u.h_mut, mut.data(), mut.size());
-        BE(be::h2d(u.d_blk, u.h_blk, u.off_order + sizeof(int32_t) * (size_t)n_sw * P));   // contexts, flags and entries in one copy
-        BE(be::event_record(u.copied));
-        u.armed = true;
-        if (!tape && h->plan_recs) BE(be::launch_plan(h->dcfg, u.d_ctx, n_sw));     // every state-independent draw of the chunk, one launch
+// Lanes: the groups split into independent sets (groups never read each other between migrations), each planned on
+// its own and launched as its own kernel chain on its own stream, so one lane's likelihood kernel runs while the other
+// lane proposes / accepts.
+static int plan_lanes(demcmc_handle *h, RunCall &call, Chunk &ck)
+{
+    const demcmc_config &cfg = h->cfg; const bool blocked = ck.blocked; Upload &u = ck.u;
+    const int Np = cfg.Np, G = h->G_local, P = h->P, B = h->B, n_lanes = call.n_lanes;
+    static const int shape_mod = [] { const char *e = getenv("DEMCMC_SHAPE"); return std::max(0, e ? atoi(e) : 8); }();   // 0 = off, else the modulus (A/B runs)
+    // levels of at most 112 updates (14 octets) for the persistent chunk kernel: measured on configs[1] against
+    // no cap / 64 / 96 / 104 / 120 / 128: 2.86 M updates/s against 2.83 / 2.64 / 2.75 / 2.82 / 2.80 / 2.83
+    static const int level_cap = [] { const char *e = getenv("DEMCMC_LEVEL_CAP"); return e ? std::max(0, atoi(e)) : 112; }();
+    ck.lane_off[0] = 0;
+    for (int ln = 0; ln < n_lanes; ++ln) {
+        const int g0 = (ln * G + n_lanes - 1) / n_lanes, g1 = ((ln + 1) * G + n_lanes - 1) / n_lanes;   // contiguous sets of groups
+        PlanInput pin;
+        pin.seed = cfg.seed; pin.Np = Np; pin.G_local = g1 - g0; pin.group_begin = cfg.group_begin + g0; pin.G_total = cfg.n_groups;
+        pin.pos_offset = g0 * Np; pin.P_stride = blocked ? P : P * B;   // consecutive sweeps of an unblocked chunk are consecutive iterations;
+                                                                        // those of a blocked one are consecutive blocks (adjacent in the tape)
+        pin.sweep_stride = blocked ? 1 : B;
+        pin.shape_octets = is_ssd(h->dmodel.kind) ? shape_mod : 0;
+        pin.level_cap = call.persist_lanes ? level_cap : 0;
+        pin.proposal = cfg.proposal; pin.beta = cfg.beta; pin.theta_snooker = cfg.theta_snooker; pin.resample = cfg.donors != 0;
+        const int64_t s_first = ck.it0 * B + (blocked ? ck.b0 : 0);
+        pin.t_kind = call.tape ? call.shard.hk.data() + (size_t)s_first * P : nullptr;       // a chunk of several sweeps is unblocked: its sweeps are P_stride apart in the tape
+        pin.t_idx = call.tape ? call.shard.hi.data() + (size_t)s_first * P * 3 : nullptr;
+        ChunkPlan &pl = call.plans[ln];
+        { HostTimer timer{ call.host_plan_s }; plan_chunk(pin, (uint32_t)((h->iter_offset + h->iters_done + ck.it0) * B + (blocked ? ck.b0 : 0)), ck.n_sw, ck.basedep, pl); }
+        memcpy(u.h_order + ck.lane_off[ln], pl.order.data(), sizeof(int32_t) * pl.order.size());
+        ck.lane_off[ln + 1] = ck.lane_off[ln] + (int32_t)pl.order.size();
+        for (int s2 = 0; s2 < ck.n_sw; ++s2)
+            for (int g = g0; g < g1; ++g) u.h_mut[(size_t)s2 * G + g] = pl.mutate[(size_t)s2 * (g1 - g0) + (g - g0)];
+    }
+    BE(be::h2d(u.d_blk, u.h_blk, u.off_order + sizeof(int32_t) * (size_t)ck.n_sw * P));   // contexts, flags and entries in one copy
+    BE(be::event_record(u.copied));
+    u.armed = true;
+    if (!call.tape && h->plan_recs) BE(be::launch_plan(h->dcfg, u.d_ctx, ck.n_sw));     // every state-independent draw of the chunk, one launch
+    return 0;
+}
 
-        if (needs_snapshot(it0)) {                               // n_sw == 1 here
-            bool any_cross = false;
-            for (int g = 0; g < G; ++g) any_cross |= mut[g] == 0;
-            if (any_cross) BE(be::launch_base_prep(h->dcfg, u.h_ctx[0].cur_w, h->base_th, h->base_cw, h->base_tot));
-        }
-        int max_levels = 0;
-        for (int ln = 0; ln < n_lanes; ++ln) max_levels = std::max(max_levels, plans[ln].n_levels);
-        // ---- the persistent path: the whole chunk in one launch (MVN / hierarchical) ---------------
-        // levels of the lanes alternate; a level's proposals wait for the previous level of its lane
-        if (persist_lanes) {
-            std::vector<int32_t> off, cnt, dep;
-            int last[be::MAX_LANES];
-            for (int &v : last) v = -1;
-            for (int l = 0; l < max_levels; ++l)
-                for (int ln = 0; ln < n_lanes; ++ln) {
-                    const ChunkPlan &pl = plans[ln];
-                    if (l >= pl.n_levels || pl.level_off[l + 1] == pl.level_off[l]) continue;
-                    off.push_back(lane_off[ln] + pl.level_off[l]);
-                    cnt.push_back(pl.level_off[l + 1] - pl.level_off[l]);
-                    dep.push_back(last[ln]);
-                    last[ln] = (int)off.size() - 1;
-                }
-            const bool tl = h->time_loglik && tev_ll0 + 2 * tev_ll + 1 < h->tev.size();
-            if (tl) BE(be::event_record(h->tev[tev_ll0 + 2 * tev_ll]));
-            const int rc = off.empty() ? 1 : be::launch_chunk_persist(h->dcfg, h->dmodel, u.d_order, u.d_ctx, off.data(), cnt.data(), dep.data(),
-                                                                      (int)off.size(), n_lanes > 1 ? 1 : 0, h->ll_acc, std::max(2, n_lanes));
-            if (rc < 0) return fail(DEMCMC_ECUDA, "chunk launch: %s", be::last_error());
-            if (rc == 0) {
-                if (tl) { BE(be::event_record(h->tev[tev_ll0 + 2 * tev_ll + 1])); ++tev_ll; }
-                n_levels += (int64_t)off.size();
-                ++h->ctr.persistent_chunks;
-                return 0;
-            }
-        }
-        // ---- a population of a few warps (the reference's own examples): every level of the chunk in one single-CTA launch
-        if (n_lanes == 1 && !h->time_loglik && !skip_stream) {
-            const ChunkPlan &pl = plans[0];
-            const int rc = be::launch_chunk_small(h->dcfg, h->dmodel, u.d_order, u.d_ctx, pl.level_off.data(), pl.n_levels);
-            if (rc < 0) return fail(DEMCMC_ECUDA, "chunk launch: %s", be::last_error());
-            if (rc == 0) { n_levels += pl.n_levels; return 0; }
-        }
-        BE(be::lane_fork(n_lanes));
-        int rc_launch = 0;
-        for (int l = 0; l < max_levels && !rc_launch; ++l)
-            for (int ln = 0; ln < n_lanes && !rc_launch; ++ln) {
+// Launches a planned chunk: the whole chunk in one persistent launch where that kernel takes it, else every level in
+// one single-CTA launch where that kernel takes it, else level by level.
+static int launch_chunk(demcmc_handle *h, RunCall &call, const Chunk &ck)
+{
+    const Upload &u = ck.u; const ChunkPlan *plans = call.plans; const int n_lanes = call.n_lanes;
+    if (needs_snapshot(h, call, ck.it0) && std::count(u.h_mut, u.h_mut + h->G_local, 0) > 0)    // n_sw == 1 here; a group crosses over
+        BE(be::launch_base_prep(h->dcfg, u.h_ctx[0].cur_w, h->base_th, h->base_cw, h->base_tot));
+    int max_levels = 0;
+    for (int ln = 0; ln < n_lanes; ++ln) max_levels = std::max(max_levels, plans[ln].n_levels);
+    // ---- the persistent path: the whole chunk in one launch (MVN / hierarchical) ---------------
+    // levels of the lanes alternate; a level's proposals wait for the previous level of its lane
+    if (call.persist_lanes) {
+        std::vector<int32_t> off, cnt, dep;
+        int last[be::MAX_LANES];                                 // the last level of each lane so far
+        std::fill_n(last, be::MAX_LANES, -1);
+        for (int l = 0; l < max_levels; ++l)
+            for (int ln = 0; ln < n_lanes; ++ln) {
                 const ChunkPlan &pl = plans[ln];
-                if (l >= pl.n_levels) continue;
-                Level lv;
-                lv.order = u.d_order + lane_off[ln] + pl.level_off[l];
-                lv.n = pl.level_off[l + 1] - pl.level_off[l];
-                lv.ctxs = u.d_ctx;
-                if (lv.n == 0) continue;
-                be::set_lane(ln);
-                const bool tl = h->time_loglik && tev_ll0 + 2 * tev_ll + 1 < h->tev.size();
-                if (!tl) {
-                    const int fused = be::launch_level_fused(h->dcfg, h->dmodel, lv);
-                    if (fused < 0) { rc_launch = 1; break; }
-                    if (fused == 0) { ++n_levels; continue; }
-                }
-                if (be::launch_propose(h->dcfg, h->dmodel, lv) ||
-                    (tl && be::event_record(h->tev[tev_ll0 + 2 * tev_ll])) ||
-                    (!skip_stream && be::launch_loglik(h->dcfg, h->dmodel, h->prop_theta, lv, h->ll_part, h->ll_acc)) ||
-                    (tl && be::event_record(h->tev[tev_ll0 + 2 * tev_ll + 1])) ||
-                    be::launch_accept(h->dcfg, h->dmodel, lv)) rc_launch = 1;
-                if (tl) ++tev_ll;
-                ++n_levels;
+                if (l >= pl.n_levels || pl.level_off[l + 1] == pl.level_off[l]) continue;
+                off.push_back(ck.lane_off[ln] + pl.level_off[l]);
+                cnt.push_back(pl.level_off[l + 1] - pl.level_off[l]);
+                dep.push_back(last[ln]);
+                last[ln] = (int)off.size() - 1;
             }
-        be::set_lane(0);
-        if (rc_launch) return fail(DEMCMC_ECUDA, "level launch: %s", be::last_error());
-        BE(be::lane_join(n_lanes));
-        return 0;
-    };
-    // measurement mode: one timed segment = the migration (with its NCCL exchange) plus the chunk(s)
-    // that follow it; the L2 flush in front of the segment is outside the bracket
-    auto seg_begin = [&]() -> int {
-        if (!h->flush_bytes) return 0;
-        BE(be::dfill(h->flush_buf, (int)(tev_chunks & 1), (size_t)h->flush_bytes));
-        BE(be::event_record(h->tev[2 * tev_chunks]));
-        return 0;
-    };
-    auto seg_end = [&]() -> int {
-        if (!h->flush_bytes) return 0;
-        BE(be::event_record(h->tev[2 * tev_chunks + 1]));
-        ++tev_chunks;
-        return 0;
-    };
-
-    int64_t chunks_this_call = 0;
-    for (int64_t it = 0; it < n_iter;) {
-        if (int rc = seg_begin()) { cleanup(); return rc; }
-        // ---- migration! (main.jl:85, migration.jl:11-19) on the current row, in place -----------
-        get_mig(it, ms);
-        if (ms.migrate) {
-            Row cur = cur_row(h);
-            if (ms.n < 2 || ms.n > Gt) { cleanup(); return fail(DEMCMC_EINVAL, "migration with %d groups", ms.n); }
-            MigArgs a;
-            memset(&a, 0, sizeof a);
-            a.n = ms.n;
-            bool cross = false, any_local = false;
-            std::vector<int> src(ms.n), dst(ms.n);
-            for (int i = 0; i < ms.n; ++i) {
-                a.groups[i] = ms.groups[i]; a.u_pick[i] = ms.u_pick[i];
-                if (a.groups[i] < 0 || a.groups[i] >= Gt) { cleanup(); return fail(DEMCMC_EINVAL, "migration group out of range"); }
-                dst[i] = h->group_owner[ms.groups[i]];
-                src[i] = h->group_owner[ms.groups[(i + ms.n - 1) % ms.n]];
-                a.src_rank[i] = (int8_t)src[i]; a.dst_rank[i] = (int8_t)dst[i];
-                cross |= src[i] != dst[i];
-                any_local |= dst[i] == h->rank;
-            }
-            // a cycle that spans ranks is one mailbox EVENT on every rank (the schedule is the same everywhere): slot
-            // seq % depth, published under the tag seq + 1; before a slot is used again every rank must have consumed it
-            const bool use_mbox = cross && h->mbox_on;
-            if (cross) ++h->ctr.cross_migrations;
-            if (use_mbox) ++h->ctr.mailbox_events;
-            int mb_slot = 0;
-            unsigned long long mb_tag = 0;
-            if (use_mbox) {
-                uint64_t &seq = *h->mbox_seq_p;
-                if (seq > 0 && seq % (uint64_t)h->mbox.depth == 0 && h->mbox_barrier)
-                    if (h->mbox_barrier()) { cleanup(); return fail(DEMCMC_ECOMM, "mailbox barrier: %s", be::last_error()); }
-                mb_slot = (int)(seq % (uint64_t)h->mbox.depth);
-                mb_tag = seq + 1;
-                ++seq;
-            }
-            if (any_local || cross) {
-                int32_t *picks = h->d_mig_log + it * MAX_MIG;
-                BE(be::launch_mig_pick(h->dcfg, a, cur.w, picks));
-                BE(be::launch_mig_gather(h->dcfg, a, picks, cur.theta, cur.w, cur.id, cur.acc, h->d_stage));
-                const double *incoming = h->d_stage;
-                if (use_mbox) {
-                    BE(be::launch_mig_push(h->dcfg, a, h->d_stage, h->peers, h->mbox, h->rank, mb_slot, mb_tag));
-                } else if (cross) {
-                    if (!h->comm) { cleanup(); return fail(DEMCMC_ECOMM, "migration crosses ranks but demcmc_comm_init was not called"); }
-                    BE(be::d2d(h->d_stage_recv, h->d_stage, sizeof(double) * ms.n * (d + 3)));
-                    if (be::comm_exchange(h->comm, h->rank, ms.n, src.data(), dst.data(), h->d_stage, h->d_stage_recv, d + 3)) { cleanup(); return fail(DEMCMC_ECOMM, "%s", be::last_error()); }
-                    incoming = h->d_stage_recv;
-                }
-                BE(be::launch_mig_scatter(h->dcfg, a, picks, incoming, cur.theta, cur.w, cur.id, cur.acc,
-                                          (h->hist_pos && h->cur_hist >= 0 && !ghist) ? h->hist_pos + (size_t)h->cur_hist * P : nullptr,
-                                          use_mbox ? &h->mbox : nullptr, h->rank, mb_slot, mb_tag));
-            }
-            // the migration edited a stored row: refresh its replicated copy (collective: every rank, the
-            // schedule is the same everywhere)
-            if (ghist && h->cur_hist >= 0) if (int rc = gather_row(h, h->cur_hist)) { cleanup(); return rc; }
-            mig_events.emplace_back(it, ms);
+        const bool tl = h->time_loglik && call.tev_ll0 + 2 * call.tev_ll + 1 < h->tev.size();
+        if (tl) BE(be::event_record(h->tev[call.tev_ll0 + 2 * call.tev_ll]));
+        const int rc = off.empty() ? 1 : be::launch_chunk_persist(h->dcfg, h->dmodel, u.d_order, u.d_ctx, off.data(), cnt.data(), dep.data(),
+                                                                  (int)off.size(), n_lanes > 1 ? 1 : 0, h->ll_acc, std::max(2, n_lanes));
+        if (rc < 0) return fail(DEMCMC_ECUDA, "chunk launch: %s", be::last_error());
+        if (rc == 0) {
+            if (tl) { BE(be::event_record(h->tev[call.tev_ll0 + 2 * call.tev_ll + 1])); ++call.tev_ll; }
+            call.n_levels += (int64_t)off.size();
+            ++h->ctr.persistent_chunks;
+            return 0;
         }
-
-        // ---- update! (main.jl:161-167) -------------------------------------------------------------
-        if (blocking_at(it)) {
-            // blocking (main.jl:174-179): every block is one sweep.  Consecutive block sweeps -- the blocks of this
-            // iteration and of the blocked iterations that follow it without a migration in between -- overlap on the
-            // device like the sweeps of unblocked iterations do (the tail levels of one sweep share launches with the
-            // head levels of the next).  A sweep whose select_base needs the sweep-start weights, and DE-MCz donors
-            // (rows of earlier sweeps), keep one sweep per chunk.
-            if (needs_snapshot(it) || cfg.donors || h->max_chunk <= 1) {
-                for (int b = 0; b < B; ++b) if (int rc = run_chunk(it, b, 1, true)) { cleanup(); return rc; }
-                if (ghist && h->cur_hist >= 0) if (int rc = gather_row(h, h->cur_hist)) { cleanup(); return rc; }
-                if (int rc = seg_end()) { cleanup(); return rc; }
-                ++it;
-                continue;
+    }
+    // ---- a population of a few warps (the reference's own examples): every level of the chunk in one single-CTA launch
+    if (n_lanes == 1 && !h->time_loglik && !call.skip_stream) {
+        const ChunkPlan &pl = plans[0];
+        const int rc = be::launch_chunk_small(h->dcfg, h->dmodel, u.d_order, u.d_ctx, pl.level_off.data(), pl.n_levels);
+        if (rc < 0) return fail(DEMCMC_ECUDA, "chunk launch: %s", be::last_error());
+        if (rc == 0) { call.n_levels += pl.n_levels; return 0; }
+    }
+    BE(be::lane_fork(n_lanes));
+    int rc_launch = 0;
+    for (int l = 0; l < max_levels && !rc_launch; ++l)
+        for (int ln = 0; ln < n_lanes && !rc_launch; ++ln) {
+            const ChunkPlan &pl = plans[ln];
+            if (l >= pl.n_levels || pl.level_off[l + 1] == pl.level_off[l]) continue;
+            const Level lv = { u.d_order + ck.lane_off[ln] + pl.level_off[l], pl.level_off[l + 1] - pl.level_off[l], u.d_ctx };
+            be::set_lane(ln);
+            const bool tl = h->time_loglik && call.tev_ll0 + 2 * call.tev_ll + 1 < h->tev.size();
+            if (!tl) {
+                const int fused = be::launch_level_fused(h->dcfg, h->dmodel, lv);
+                if (fused < 0) { rc_launch = 1; break; }
+                if (fused == 0) { ++call.n_levels; continue; }
             }
-            const int cap_sweeps = (int)std::min<int64_t>(h->max_chunk, (int64_t)4 << std::min<int64_t>(chunks_this_call, 8));
-            ++chunks_this_call;
-            int n_it = 1;
-            MigSchedule m2;
-            while (it + n_it < n_iter && (n_it + 1) * B <= std::max(cap_sweeps, B)) {
-                get_mig(it + n_it, m2);
-                if (m2.migrate || needs_snapshot(it + n_it) || !blocking_at(it + n_it)) break;
-                ++n_it;
-            }
-            if (n_it * B > MAX_CHUNK) {                          // more blocks than a chunk holds: one sweep per chunk
-                for (int b = 0; b < B; ++b) if (int rc = run_chunk(it, b, 1, true)) { cleanup(); return rc; }
-                n_it = 1;
-            } else if (int rc = run_chunk(it, 0, n_it * B, true)) { cleanup(); return rc; }
-            if (int rc = seg_end()) { cleanup(); return rc; }
-            it += n_it;
-            continue;
+            if (be::launch_propose(h->dcfg, h->dmodel, lv) ||
+                (tl && be::event_record(h->tev[call.tev_ll0 + 2 * call.tev_ll])) ||
+                (!call.skip_stream && be::launch_loglik(h->dcfg, h->dmodel, h->prop_theta, lv, h->ll_part, h->ll_acc)) ||
+                (tl && be::event_record(h->tev[call.tev_ll0 + 2 * call.tev_ll + 1])) ||
+                be::launch_accept(h->dcfg, h->dmodel, lv)) rc_launch = 1;
+            if (tl) ++call.tev_ll;
+            ++call.n_levels;
         }
-        // consecutive iterations without a migration and without a sweep-start snapshot overlap on
-        // the device: plan them as one chunk (planner.h)
-        int n = 1;
+    be::set_lane(0);
+    if (rc_launch) return fail(DEMCMC_ECUDA, "level launch: %s", be::last_error());
+    BE(be::lane_join(n_lanes));
+    return 0;
+}
+
+// ---- migration! (main.jl:85, migration.jl:11-19) before local iteration `it`, on the current row, in place --------
+static int migrate(demcmc_handle *h, RunCall &call, int64_t it)
+{
+    const int Gt = h->cfg.n_groups, P = h->P, d = h->d;
+    MigSchedule ms;
+    get_mig(h, call, it, ms);
+    if (!ms.migrate) return 0;
+    Row cur = cur_row(h);
+    if (ms.n < 2 || ms.n > Gt) return fail(DEMCMC_EINVAL, "migration with %d groups", ms.n);
+    MigArgs a;
+    memset(&a, 0, sizeof a);
+    a.n = ms.n;
+    bool cross = false, any_local = false;
+    std::vector<int> src(ms.n), dst(ms.n);
+    for (int i = 0; i < ms.n; ++i) {
+        a.groups[i] = ms.groups[i]; a.u_pick[i] = ms.u_pick[i];
+        if (a.groups[i] < 0 || a.groups[i] >= Gt) return fail(DEMCMC_EINVAL, "migration group out of range");
+        dst[i] = h->group_owner[ms.groups[i]];
+        src[i] = h->group_owner[ms.groups[(i + ms.n - 1) % ms.n]];
+        a.src_rank[i] = (int8_t)src[i]; a.dst_rank[i] = (int8_t)dst[i];
+        cross |= src[i] != dst[i];
+        any_local |= dst[i] == h->rank;
+    }
+    // a cycle that spans ranks is one mailbox EVENT on every rank (the schedule is the same everywhere): slot
+    // seq % depth, published under the tag seq + 1; before a slot is used again every rank must have consumed it
+    const bool use_mbox = cross && h->mbox_on;
+    if (cross) ++h->ctr.cross_migrations;
+    if (use_mbox) ++h->ctr.mailbox_events;
+    int mb_slot = 0;
+    unsigned long long mb_tag = 0;
+    if (use_mbox) {
+        uint64_t &seq = *h->mbox_seq_p;
+        if (seq > 0 && seq % (uint64_t)h->mbox.depth == 0 && h->mbox_barrier)
+            if (h->mbox_barrier()) return fail(DEMCMC_ECOMM, "mailbox barrier: %s", be::last_error());
+        mb_slot = (int)(seq % (uint64_t)h->mbox.depth);
+        mb_tag = seq + 1;
+        ++seq;
+    }
+    if (any_local || cross) {
+        int32_t *picks = h->d_mig_log + it * MAX_MIG;
+        BE(be::launch_mig_pick(h->dcfg, a, cur.w, picks));
+        BE(be::launch_mig_gather(h->dcfg, a, picks, cur.theta, cur.w, cur.id, cur.acc, h->d_stage));
+        const double *incoming = h->d_stage;
+        if (use_mbox) {
+            BE(be::launch_mig_push(h->dcfg, a, h->d_stage, h->peers, h->mbox, h->rank, mb_slot, mb_tag));
+        } else if (cross) {
+            if (!h->comm) return fail(DEMCMC_ECOMM, "migration crosses ranks but demcmc_comm_init was not called");
+            BE(be::d2d(h->d_stage_recv, h->d_stage, sizeof(double) * ms.n * (d + 3)));
+            if (be::comm_exchange(h->comm, h->rank, ms.n, src.data(), dst.data(), h->d_stage, h->d_stage_recv, d + 3)) return fail(DEMCMC_ECOMM, "%s", be::last_error());
+            incoming = h->d_stage_recv;
+        }
+        BE(be::launch_mig_scatter(h->dcfg, a, picks, incoming, cur.theta, cur.w, cur.id, cur.acc,
+                                  (h->hist_pos && h->cur_hist >= 0 && !call.ghist) ? h->hist_pos + (size_t)h->cur_hist * P : nullptr,
+                                  use_mbox ? &h->mbox : nullptr, h->rank, mb_slot, mb_tag));
+    }
+    // the migration edited a stored row: refresh its replicated copy (collective: every rank, the
+    // schedule is the same everywhere)
+    if (call.ghist && h->cur_hist >= 0) if (int rc = gather_row(h, h->cur_hist)) return rc;
+    call.mig_events.emplace_back(it, ms.n);
+    return 0;
+}
+
+// Sweeps in the chunk that starts at local iteration `it`.  Consecutive iterations without a migration, without a
+// sweep-start snapshot and in the same blocking mode overlap on the device: they are planned as one chunk (planner.h).
+// 1 for a blocked iteration: its blocks run as chunks of one sweep each.
+static int chunk_length(demcmc_handle *h, RunCall &call, int64_t it, bool blocked)
+{
+    const int B = h->B; int64_t max_it;                          // iterations the chunk may hold
+    if (blocked) {
+        // blocking (main.jl:174-179): every block is one sweep.  Consecutive block sweeps -- the blocks of this
+        // iteration and of the blocked iterations that follow it without a migration in between -- overlap on the
+        // device like the sweeps of unblocked iterations do (the tail levels of one sweep share launches with the
+        // head levels of the next).  A sweep whose select_base needs the sweep-start weights, and DE-MCz donors
+        // (rows of earlier sweeps), keep one sweep per chunk.
+        if (needs_snapshot(h, call, it) || h->cfg.donors || h->max_chunk <= 1) return 1;
+        const int cap_sweeps = (int)std::min<int64_t>(h->max_chunk, (int64_t)4 << std::min<int64_t>(call.chunks_this_call, 8));
+        max_it = std::max(cap_sweeps, B) / B;
+    } else {
         // slow start: the device idles while the host plans the first chunk of a call (49 ms for 16
         // sweeps of 32768 particles), so the first chunks are short -- 2, 4, 8 sweeps -- and the long
         // ones are planned while the device is busy with their predecessors
-        static int first_chunk = -1;
-        if (first_chunk < 0) { const char *e = getenv("DEMCMC_FIRST_CHUNK"); first_chunk = e ? std::max(1, atoi(e)) : 4; }     // 4, 8, 16 sweeps: measured against 2, 4, 8, 16 at 20 steps: +1.4 %
+        static const int first_chunk = [] { const char *e = getenv("DEMCMC_FIRST_CHUNK"); return e ? std::max(1, atoi(e)) : 4; }();     // 4, 8, 16 sweeps: measured against 2, 4, 8, 16 at 20 steps: +1.4 %
         // ... doubling from chunk to chunk; four-fold where a sweep is heavy on the device next to its planning (>= 2e6
         // observation x dimension products per particle: planning 16 sweeps of configs[1] takes 0.6 ms, the 4 sweeps it hides
         // behind 1.5 ms), so that a 20-iteration call is 4 + 16 sweeps instead of 4 + 8 + 8
-        static int growth_env = -1;
-        if (growth_env < 0) { const char *e = getenv("DEMCMC_CHUNK_GROWTH"); growth_env = e ? std::max(0, atoi(e)) : 0; }
+        static const int growth_env = [] { const char *e = getenv("DEMCMC_CHUNK_GROWTH"); return e ? std::max(0, atoi(e)) : 0; }();
         const bool heavy = (double)h->dmodel.n_obs * (double)std::max(1, (int)h->dmodel.n_dim) >= 2e6;
         const int shift = growth_env ? growth_env : (heavy ? 2 : 1);
-        const int chunk_cap = (int)std::min<int64_t>(h->max_chunk, (int64_t)first_chunk << std::min<int64_t>(shift * chunks_this_call, 8));
-        ++chunks_this_call;
-        if (!needs_snapshot(it) && h->max_chunk > 1 && !cfg.donors) {   // resample reads rows of earlier sweeps: one sweep per chunk
-            MigSchedule m2;
-            while (it + n < n_iter && n < chunk_cap) {
-                get_mig(it + n, m2);
-                if (m2.migrate || needs_snapshot(it + n) || blocking_at(it + n)) break;
-                ++n;
-            }
+        const int chunk_cap = (int)std::min<int64_t>(h->max_chunk, (int64_t)first_chunk << std::min<int64_t>(shift * call.chunks_this_call, 8));
+        // resample reads rows of earlier sweeps: one sweep per chunk
+        max_it = (needs_snapshot(h, call, it) || h->max_chunk <= 1 || h->cfg.donors) ? 1 : chunk_cap;
+    }
+    ++call.chunks_this_call;
+    int n = 1; MigSchedule m2;
+    while (it + n < call.n_iter && n < max_it) {
+        get_mig(h, call, it + n, m2);
+        if (m2.migrate || needs_snapshot(h, call, it + n) || blocking_at(h, it + n) != blocked) break;
+        ++n;
+    }
+    return !blocked ? n : n * B > MAX_CHUNK ? 1 : n * B;        // more blocks than a chunk holds: one sweep per chunk
+}
+
+static int run_impl(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter)
+{
+    if (!h || n_iter < 0) return fail(DEMCMC_EINVAL, "bad argument");
+    if (!h->has_model || !h->has_state) return fail(DEMCMC_ESTATE, "set_model and set_state must come before run");
+    BE(be::set_device(h->cfg.device));
+    const demcmc_config &cfg = h->cfg; const int Gt = cfg.n_groups, G = h->G_local, P = h->P, B = h->B;
+    if (h->n0 > 0 && !h->has_history) return fail(DEMCMC_ESTATE, "n_initial > 0: demcmc_set_history must come before run");
+    if (cfg.donors && G != Gt && h->n_ranks <= 1) return fail(DEMCMC_ESTATE, "sample = resample on a sharded job reads the history of every particle id: demcmc_comm_init must come first");
+    RunCall call;
+    call.tape = tape; call.n_iter = n_iter; call.S = n_iter * B; call.ghist = cfg.donors && h->n_ranks > 1;
+    h->dcfg.P_hist = call.ghist ? (int32_t)((int64_t)Gt * cfg.Np) : (int32_t)P;
+    if (cfg.donors && h->iter_offset > 0) return fail(DEMCMC_EUNSUPPORTED, "sample = resample draws donors from the rows of earlier iterations: a resumed handle does not hold them");
+    if (int rc = grow_history(h, stored_rows(h, h->iters_done + n_iter))) return rc;
+    if (tape) if (int rc = load_tape(h, tape, n_iter, call.shard)) return rc;
+    if (int rc = reset_call_buffers(h, call)) return rc;
+
+    const int64_t launches0 = be::launch_count();
+    call.tev_ll0 = h->flush_bytes ? 2 * (size_t)n_iter : 0;
+    const size_t tev_need = call.tev_ll0 + (h->time_loglik ? 2 * (size_t)call.S * 64 : 0);
+    while (h->tev.size() < tev_need) { void *e = be::tevent_create(); if (!e) return fail(DEMCMC_ECUDA, "event pool: %s", be::last_error()); h->tev.push_back(e); }
+    BE(be::timer_start());
+    // the persistent chunk kernel alternates the levels of two lanes; the level-by-level path runs the handle's lanes
+    // (default 1) as concurrent kernel chains
+    call.skip_stream = h->suffstat && is_ssd(h->dmodel.kind);    // B == 0 analytically: propose -> accept, nothing streamed
+    call.persist_lanes = call.skip_stream ? 0 : be::chunk_persist_lanes(h->dcfg, h->dmodel);
+    call.n_lanes = call.persist_lanes ? call.persist_lanes : std::max(1, std::min(h->n_lanes, G));
+
+    for (int64_t it = 0; it < n_iter;) {
+        // measurement mode: one timed segment = the migration (with its NCCL exchange) plus the chunk(s)
+        // that follow it; the L2 flush in front of the segment is outside the bracket
+        if (h->flush_bytes) { BE(be::dfill(h->flush_buf, (int)(call.tev_chunks & 1), (size_t)h->flush_bytes)); BE(be::event_record(h->tev[2 * call.tev_chunks])); }
+        if (int rc = migrate(h, call, it)) return rc;
+        // ---- update! (main.jl:161-167) -------------------------------------------------------------
+        const bool blocked = blocking_at(h, it);
+        const int n_sw = chunk_length(h, call, it, blocked);
+        const int n_chunks = blocked && n_sw == 1 ? B : 1;
+        for (int c = 0; c < n_chunks; ++c) {
+            call.sweeps_run += n_sw;
+            HostTimer timer{ call.host_chunk_s };
+            Chunk ck{ it, c, n_sw, blocked, h->ring[h->ring_use % demcmc_handle::RING] };
+            if (ck.u.armed) BE(be::event_wait(ck.u.copied));   // the pinned slot is free once its copies ran
+            h->ring_use++;
+            fill_sweep_contexts(h, call, ck);
+            if (int rc = plan_lanes(h, call, ck)) return rc;
+            if (int rc = launch_chunk(h, call, ck)) return rc;
         }
-        if (int rc = run_chunk(it, 0, n, false)) { cleanup(); return rc; }
-        if (ghist && h->cur_hist >= 0) if (int rc = gather_row(h, h->cur_hist)) { cleanup(); return rc; }     // n == 1 with resample
-        if (int rc = seg_end()) { cleanup(); return rc; }
-        it += n;
+        if (call.ghist && h->cur_hist >= 0) if (int rc = gather_row(h, h->cur_hist)) return rc;     // resample: one sweep per chunk
+        if (h->flush_bytes) { BE(be::event_record(h->tev[2 * call.tev_chunks + 1])); ++call.tev_chunks; }
+        it += blocked ? n_chunks * n_sw / B : n_sw;
     }
     double ms_dev = 0.0;
     BE(be::timer_stop(&ms_dev));
     BE(be::sync());
     if (h->flush_bytes) {                                   // sum of the per-segment times (migration + chunk), flushes excluded
         ms_dev = 0.0;
-        for (size_t c = 0; c < tev_chunks; ++c) { double t = 0.0; BE(be::tevent_elapsed(h->tev[2 * c], h->tev[2 * c + 1], &t)); ms_dev += t; }
+        for (size_t c = 0; c < call.tev_chunks; ++c) { double t = 0.0; BE(be::tevent_elapsed(h->tev[2 * c], h->tev[2 * c + 1], &t)); ms_dev += t; }
     }
     double ms_ll = 0.0;
-    for (size_t i = 0; i < tev_ll; ++i) { double t = 0.0; BE(be::tevent_elapsed(h->tev[tev_ll0 + 2 * i], h->tev[tev_ll0 + 2 * i + 1], &t)); ms_ll += t; }
+    for (size_t i = 0; i < call.tev_ll; ++i) { double t = 0.0; BE(be::tevent_elapsed(h->tev[call.tev_ll0 + 2 * i], h->tev[call.tev_ll0 + 2 * i + 1], &t)); ms_ll += t; }
     h->ctr.loglike_ms = ms_ll;
-    // migration log -> host
-    for (auto &ev : mig_events) {
-        std::vector<int32_t> picks(ev.second.n);
-        BE(be::d2h(picks.data(), h->d_mig_log + ev.first * MAX_MIG, sizeof(int32_t) * ev.second.n));
-        for (int i = 0; i < ev.second.n; ++i) h->last_mig_slots[ev.first * Gt + i] = picks[i];
-    }
-    cleanup();
+    for (auto &ev : call.mig_events)                        // migration log -> host
+        BE(be::d2h(h->last_mig_slots.data() + ev.first * Gt, h->d_mig_log + ev.first * MAX_MIG, sizeof(int32_t) * ev.second));
     h->iters_done += n_iter;
-    if (host_prof) fprintf(stderr, "[demcmc host] %lld iterations: chunks %.3f ms on the host (planner %.3f ms), %lld levels\n", (long long)n_iter, host_chunk_s * 1e3, host_plan_s * 1e3, (long long)n_levels);
-    h->ctr.iterations += n_iter; h->ctr.sweeps += sweeps_run; h->ctr.particle_updates += sweeps_run * P; h->ctr.loglike_evals += sweeps_run * P;
-    h->ctr.kernel_launches += be::launch_count() - launches0; h->ctr.levels += n_levels; h->ctr.device_ms = ms_dev;
+    if (host_profile()) fprintf(stderr, "[demcmc host] %lld iterations: chunks %.3f ms on the host (planner %.3f ms), %lld levels\n", (long long)n_iter, call.host_chunk_s * 1e3, call.host_plan_s * 1e3, (long long)call.n_levels);
+    h->ctr.iterations += n_iter; h->ctr.sweeps += call.sweeps_run; h->ctr.particle_updates += call.sweeps_run * P; h->ctr.loglike_evals += call.sweeps_run * P;
+    h->ctr.kernel_launches += be::launch_count() - launches0; h->ctr.levels += call.n_levels; h->ctr.device_ms = ms_dev;
     return 0;
 }
 

@@ -1063,13 +1063,20 @@ __global__ void __launch_bounds__(SC_MAX_WARPS * 32, 1) k_chunk_small(const __gr
 }
 constexpr int64_t FUSED_MAX_OBS = 256;
 
+// small pointwise models: one warp per update.  DEMCMC_NO_FUSED=1 turns that off, read per call (A/B runs in one process)
+static bool fused_eligible(const ConfigDev &cfg, const ModelDev &m)
+{
+    const char *env = getenv("DEMCMC_NO_FUSED");
+    if (env && env[0] == '1') return false;
+    if (is_ssd(m.kind) || cfg.d > 64) return false;
+    if ((m.kind == M_GAUSSIAN || m.kind == M_LNR || m.kind == M_LBA) && (m.n_obs > FUSED_MAX_OBS || m.n_osplit * m.n_ksplit != 1)) return false;
+    return m.kind == M_GAUSSIAN || m.kind == M_LNR || m.kind == M_LBA || m.kind == M_BINOMIAL || m.kind == M_RASTRIGIN;
+}
+
 // returns 1 when the level is not a small pointwise one (the caller launches the three kernels)
 int launch_level_fused(const ConfigDev &cfg, const ModelDev &m, const Level &lv)
 {
-    const char *env = getenv("DEMCMC_NO_FUSED");
-    if (env && env[0] == '1') return 1;
-    if (is_ssd(m.kind) || !lv.ctxs || cfg.d > 64) return 1;
-    if ((m.kind == M_GAUSSIAN || m.kind == M_LNR || m.kind == M_LBA) && (m.n_obs > FUSED_MAX_OBS || m.n_osplit * m.n_ksplit != 1)) return 1;
+    if (!lv.ctxs || !fused_eligible(cfg, m)) return 1;
     const int blocks = (lv.n * 32 + PA_THREADS - 1) / PA_THREADS;
     switch (m.kind) {
     case M_GAUSSIAN: CU(launch_chained(k_level_fused<M_GAUSSIAN>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
@@ -1082,15 +1089,6 @@ int launch_level_fused(const ConfigDev &cfg, const ModelDev &m, const Level &lv)
     LAUNCHED("k_level_fused");
     if (g_tl_cap > 0) ++g_tl_level;
     return 0;
-}
-
-static bool fused_eligible(const ConfigDev &cfg, const ModelDev &m)
-{
-    const char *env = getenv("DEMCMC_NO_FUSED");
-    if (env && env[0] == '1') return false;
-    if (is_ssd(m.kind) || cfg.d > 64) return false;
-    if ((m.kind == M_GAUSSIAN || m.kind == M_LNR || m.kind == M_LBA) && (m.n_obs > FUSED_MAX_OBS || m.n_osplit * m.n_ksplit != 1)) return false;
-    return m.kind == M_GAUSSIAN || m.kind == M_LNR || m.kind == M_LBA || m.kind == M_BINOMIAL || m.kind == M_RASTRIGIN;
 }
 
 // returns 1 when the chunk is not a small pointwise one (the caller launches level by level)
