@@ -2756,15 +2756,17 @@ int launch_chains(const double *rows_theta, const double *rows_w, const uint8_t 
 // ------------------------------------------------------------------------------------------------
 // streaming moments of the history: Welford per thread over the vectors of its block, Chan's merge
 // of the per-block partials in block order (deterministic; lanes run along the parameters, so the
-// reads coalesce)
+// reads coalesce).  Both work on x - x[0] (the first vector): the partial means are then of the size of
+// the spread, and the differences of them in the merge do not cancel for a parameter at a large offset
 // ------------------------------------------------------------------------------------------------
 constexpr int MOM_BLOCKS = 592, MOM_THREADS = 128;
 __global__ void __launch_bounds__(MOM_THREADS) k_moments_partial(const double *x, int64_t n, int d, double *pmean, double *pm2)
 {
     for (int k = threadIdx.x; k < d; k += MOM_THREADS) {
         double mean = 0.0, m2 = 0.0, cnt = 0.0;
+        const double shift = x[k];
         for (int64_t r = blockIdx.x; r < n; r += MOM_BLOCKS) {
-            const double v = x[r * d + k];
+            const double v = x[r * d + k] - shift;
             cnt += 1.0;
             const double dl = v - mean;
             mean += dl / cnt;
@@ -2774,7 +2776,7 @@ __global__ void __launch_bounds__(MOM_THREADS) k_moments_partial(const double *x
         pm2[(size_t)blockIdx.x * d + k] = m2;
     }
 }
-__global__ void __launch_bounds__(MOM_THREADS) k_moments_merge(const double *pmean, const double *pm2, int64_t n, int d, double *mean, double *m2)
+__global__ void __launch_bounds__(MOM_THREADS) k_moments_merge(const double *x, const double *pmean, const double *pm2, int64_t n, int d, double *mean, double *m2)
 {
     const int k = blockIdx.x * MOM_THREADS + threadIdx.x;
     if (k >= d) return;
@@ -2788,7 +2790,7 @@ __global__ void __launch_bounds__(MOM_THREADS) k_moments_merge(const double *pme
         sa += sb + dl * dl * (ca * cb / c);
         ca = c;
     }
-    mean[k] = ma; m2[k] = sa;
+    mean[k] = x[k] + ma; m2[k] = sa;
 }
 int launch_moments(const double *x, int64_t n, int32_t d, double *mean, double *m2)
 {
@@ -2796,7 +2798,7 @@ int launch_moments(const double *x, int64_t n, int32_t d, double *mean, double *
     if (!part) return -1;
     k_moments_partial<<<MOM_BLOCKS, MOM_THREADS, 0, stream()>>>(x, n, d, part, part + (size_t)MOM_BLOCKS * d);
     LAUNCHED("k_moments_partial");
-    k_moments_merge<<<(d + MOM_THREADS - 1) / MOM_THREADS, MOM_THREADS, 0, stream()>>>(part, part + (size_t)MOM_BLOCKS * d, n, d, mean, m2);
+    k_moments_merge<<<(d + MOM_THREADS - 1) / MOM_THREADS, MOM_THREADS, 0, stream()>>>(x, part, part + (size_t)MOM_BLOCKS * d, n, d, mean, m2);
     LAUNCHED("k_moments_merge");
     dfree(part);
     return 0;
@@ -2815,7 +2817,11 @@ __global__ void __launch_bounds__(256) k_diag_pos(const int32_t *rid, int64_t ro
 }
 // one block per (parameter k, group of chains): each split chain is gathered into shared memory (its draws sit at a
 // different position of every stored row: ids migrate), then thread t accumulates the lags t, t + 256, ...; the
-// block's chains are summed in order, the groups by k_diag_merge in order: deterministic
+// block's chains are summed in order, the groups by k_diag_merge in order: deterministic.
+// Every draw is taken less c_k, the draw of id 0 at row0 (the same value in every block and shard): the chain means and
+// the sums of them and of their squares are then of the size of the spread, not of the location, so the between-chain
+// variance diag_finish forms from them does not cancel for a parameter at a large offset (agg[1] and agg[2] are of the
+// shifted means; the variances and autocovariances do not depend on the shift).
 constexpr int DG_THREADS = 256, DG_GROUPS = 32, DG_MAX_LAG = 4096 /* lags per launch: 16 accumulators per thread */, DG_MAX_NH = 24576 /* 192 KB of shared memory */;
 __global__ void __launch_bounds__(DG_THREADS) k_diag_partial(DiagShards sh, const int32_t *pos, int64_t row0, int64_t n_rows, int P, int d,
                                                              int lag0, int n_lag, double *part /* [d][DG_GROUPS][3 + n_lag]: lags lag0 .. lag0 + n_lag - 1 */)
@@ -2832,6 +2838,8 @@ __global__ void __launch_bounds__(DG_THREADS) k_diag_partial(DiagShards sh, cons
     double acov[LPT];
 #pragma unroll
     for (int j = 0; j < LPT; ++j) acov[j] = 0.0;
+    const int q0 = pos[0], shard0 = q0 / sh.P_local;
+    const double shift = sh.theta[shard0][(row0 * sh.P_local + (q0 - shard0 * sh.P_local)) * d + k];
     for (int c = c0; c < c1; ++c) {
         const int id = c >> 1;
         const int64_t r0 = (c & 1) ? n_rows - nh : 0;             // second half: the LAST nh draws
@@ -2839,7 +2847,7 @@ __global__ void __launch_bounds__(DG_THREADS) k_diag_partial(DiagShards sh, cons
         for (int i = tid; i < nh; i += DG_THREADS) {
             const int64_t r = r0 + i;
             const int q = pos[r * P + id], shard = q / sh.P_local;
-            const double v = sh.theta[shard][((row0 + r) * sh.P_local + (q - shard * sh.P_local)) * d + k];
+            const double v = sh.theta[shard][((row0 + r) * sh.P_local + (q - shard * sh.P_local)) * d + k] - shift;
             xs[i] = v; s += v;
         }
         s = warp_sum(s);

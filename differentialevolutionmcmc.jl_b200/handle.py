@@ -248,8 +248,10 @@ class Handle:
 
     def moments(self, row0=0, n_rows=None):
         """Pooled posterior summary computed on the device (no download of the draws): (count, mean[d],
-        var[d] with ddof=1) over history rows [row0, row0+n_rows) and all local particles."""
-        n = self.stored_iterations - row0 if n_rows is None else n_rows
+        var[d] with ddof=1) over history rows [row0, row0+n_rows) and all local particles.  Rows count from the
+        first history row, the n_initial prior rows included (as in samples() and diagnostics()); by default
+        every stored row from row0 on."""
+        n = self.n_rows - row0 if n_rows is None else n_rows
         cnt = C.c_int64(0)
         mean, m2 = np.zeros(self.d), np.zeros(self.d)
         check(_ffi.lib().demcmc_get_moments(self._h, int(row0), int(n), C.byref(cnt), ptr(mean, _dp), ptr(m2, _dp)))

@@ -250,7 +250,8 @@ int demcmc_set_blocking_schedule(demcmc_handle *h, const uint8_t *on, int64_t n)
 int demcmc_set_weights(demcmc_handle *h, const double *w);
 /* Streaming summary on the device (SURVEY 8f-1: the history, not the compute, is what stops scaling --
  * configs[4] would hand 423 GB of draws to the host): pooled over history rows [row0, row0+n_rows) and all
- * local particles, per flattened parameter k: mean[k] and m2[k] = sum (x - mean[k])^2, with *count =
+ * local particles (rows count from the first history row, the n_initial prior rows included, as in
+ * demcmc_get_samples and demcmc_get_diagnostics), per flattened parameter k: mean[k] and m2[k] = sum (x - mean[k])^2, with *count =
  * n_rows * P_local draws, i.e. what MCMCChains' mean / std of the pooled chains reduce to
  * (var = m2 / (count - 1)).  Shards of a multi-GPU job merge (count, mean, m2) with Chan's update. */
 int demcmc_get_moments(demcmc_handle *h, int64_t row0, int64_t n_rows, int64_t *count, double *mean, double *m2);

@@ -234,10 +234,10 @@ int launch_propose(const ConfigDev &cfg, const ModelDev &m, const Level &lv)
 int launch_moments(const double *x, int64_t n, int32_t d, double *mean, double *m2)
 {
     ++g_launches;
-    for (int k = 0; k < d; ++k) {
+    for (int k = 0; k < d; ++k) {                                       // about the first vector, as the kernels
         double mu = 0.0, s = 0.0;
-        for (int64_t r = 0; r < n; ++r) { const double v = x[r * d + k], dl = v - mu; mu += dl / (double)(r + 1); s += dl * (v - mu); }
-        mean[k] = mu; m2[k] = s;
+        for (int64_t r = 0; r < n; ++r) { const double v = x[r * d + k] - x[k], dl = v - mu; mu += dl / (double)(r + 1); s += dl * (v - mu); }
+        mean[k] = x[k] + mu; m2[k] = s;
     }
     return 0;
 }
@@ -259,13 +259,15 @@ int launch_diag_aggregates(const DiagShards &sh, const int32_t *pos, int64_t row
     for (int k = 0; k < d; ++k) {
         double *a = agg + (size_t)k * (3 + n_lag);
         for (int j = 0; j < 3 + n_lag; ++j) a[j] = 0.0;
+        const int q0 = pos[0], shard0 = q0 / sh.P_local;               // the kernel's shift: the draw of id 0 at row0
+        const double shift = sh.theta[shard0][(row0 * sh.P_local + (q0 - shard0 * sh.P_local)) * d + k];
         for (int c = 0; c < 2 * P; ++c) {
             const int id = c >> 1;
             const int64_t r0 = (c & 1) ? n_rows - nh : 0;
             double mean = 0.0;
             for (int64_t i = 0; i < nh; ++i) {
                 const int q = pos[(size_t)(r0 + i) * P + id], shard = q / sh.P_local;
-                x[i] = sh.theta[shard][((row0 + r0 + i) * sh.P_local + (q - shard * sh.P_local)) * d + k];
+                x[i] = sh.theta[shard][((row0 + r0 + i) * sh.P_local + (q - shard * sh.P_local)) * d + k] - shift;
                 mean += x[i];
             }
             mean /= (double)nh;
