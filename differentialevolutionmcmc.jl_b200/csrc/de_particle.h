@@ -31,15 +31,26 @@ struct NullSink {
 };
 constexpr int PROP_PRE = 2;   // elements per lane whose state-independent inputs are fetched before the dependency wait
 
+// M_MVN_FULL: the whitened mean nu_k = sum_{j <= k} Linv[k][j] (mu_j - c_j), subtracted before the product so that the
+// offset of the data does not cancel.  Out of line on the device: the kernels that serve the other kinds as well (eval,
+// the persistent chunk kernel) keep their registers for those.
+#if defined(__CUDACC__)
+__host__ __device__ __noinline__
+#else
+inline
+#endif
+double whitened_mean(const double *linv, const double *raw_center, int n_dim, const double *theta, int k)
+{
+    const double *row = linv + (size_t)k * n_dim;
+    double nu = 0.0;
+    for (int j = 0; j <= k; ++j) nu += row[j] * (theta[j] - raw_center[j]);
+    return nu;
+}
+
 // mean of dimension k of the MVN / hierarchical likelihood, relative to the data centre
 DE_HD double centred_mean(const ModelDev &m, const double *theta, int k)
 {
-    if (m.kind == M_MVN_FULL) {                                // whitened mean nu_k = sum_{j <= k} Linv[k][j] mu_j
-        const double *row = m.linv + (size_t)k * m.n_dim;
-        double nu = 0.0;
-        for (int j = 0; j <= k; ++j) nu += row[j] * theta[j];
-        return nu - m.center[k];
-    }
+    if (m.kind == M_MVN_FULL) return whitened_mean(m.linv, m.raw_center, m.n_dim, theta, k) - m.center[k];
     return (m.kind == M_HIER ? theta[0] + theta[2 + k] : theta[k]) - m.center[k];
 }
 

@@ -33,7 +33,11 @@ struct ModelDev {
                               // A fragments (ssd_pack_index below); the host test double keeps xT[ssd_k][ssd_ld]
     const double *center;     // [ssd_k] column means removed from the data
     const double *linv;       // M_MVN_FULL: inverse of the Cholesky factor of the covariance, lower triangular [n_dim][n_dim]: the
-                              // kernel streams the WHITENED data y = Linv x against the whitened means nu = Linv mu
+                              // kernel streams the WHITENED data y = Linv (x - raw_center) against the whitened means
+                              // Linv (mu - raw_center)
+    const double *raw_center; // M_MVN_FULL: [n_dim] centre subtracted in data space, before whitening (the column means, or
+                              // demcmc_model.center): Linv x and Linv mu are both of size |Linv| |offset| and their difference
+                              // would cancel
     double logdet;            // M_MVN_FULL: log det of the covariance
     double ssd_xx;            // sum of the squared centred data
     double ssd_rowmax;        // 2 max_i |x'_i|: bounds every chain of k_xdot (the cross terms of two observation rows)

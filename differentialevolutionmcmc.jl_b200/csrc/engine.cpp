@@ -745,20 +745,35 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
                     for (int q = c; q < r; ++q) t -= (long double)L[(size_t)r * k + q] * Li[(size_t)q * k + c];
                     Li[(size_t)r * k + c] = (double)(t / L[(size_t)r * k + r]);
                 }
+            // centred in data space first, y = L^-1 (x - c), and every proposal's mean likewise as Linv (mu - c): whitening
+            // x and mu separately gives two terms of size |L^-1| |offset| whose difference, of the size of the posterior
+            // spread, loses every digit the offset takes
+            std::vector<double> c((size_t)k, 0.0);
+            if (m->center) std::copy(m->center, m->center + k, c.begin());
+            else if (m->n_obs > 0)
+                for (int r = 0; r < k; ++r) {
+                    long double s = 0.0L;
+                    for (int64_t i = 0; i < m->n_obs; ++i) s += m->x[(size_t)i * k + r];
+                    c[r] = (double)(s / (long double)m->n_obs);
+                }
             std::vector<double> y((size_t)m->n_obs * k);
             for (int64_t i = 0; i < m->n_obs; ++i) {
                 const double *xi = m->x + (size_t)i * k;
                 double *yi = y.data() + (size_t)i * k;
                 for (int r = 0; r < k; ++r) {                    // forward substitution: the same arithmetic as whitening through L
-                    long double t = xi[r];
+                    long double t = (long double)xi[r] - c[r];
                     for (int q = 0; q < r; ++q) t -= (long double)L[(size_t)r * k + q] * yi[q];
                     yi[r] = (double)(t / L[(size_t)r * k + r]);
                 }
             }
             D.linv = (const double *)upload(Li.data(), sizeof(double) * Li.size(), false);
-            if (!D.linv) return fail(DEMCMC_ENOMEM, "covariance factor upload failed");
+            D.raw_center = (const double *)upload(c.data(), sizeof(double) * c.size(), false);
+            if (!D.linv || !D.raw_center) return fail(DEMCMC_ENOMEM, "covariance factor upload failed");
             D.logdet = logdet;
-            BE(be::launch_pack_ssd(y.data(), 0, m->center, &D));
+            // the whitened data are centred on their own column means (which round to about 0), or, with an explicit
+            // centre, not at all: the cross term is then B = sum_i y_i . Linv (mu - center)
+            const std::vector<double> zero((size_t)k, 0.0);
+            BE(be::launch_pack_ssd(y.data(), 0, m->center ? zero.data() : nullptr, &D));
         } else
         BE(be::launch_pack_ssd(m->x, dev, m->center, &D));       // centres and packs the data, fills D.ssd_xx / D.ssd_rowmax
     } else {

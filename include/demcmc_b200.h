@@ -104,7 +104,12 @@ typedef struct {
                                most accurate split, and the reason no likelihood value can show whether the O(N d)
                                stream was computed correctly.  center[n_dim] (host memory) centres on THAT vector
                                instead: B is then n (mean - center).m', not zero, and demcmc_get_trace_xdot /
-                               demcmc_eval_xdot expose it, which is how the parity tests pin the DMMA kernels. */
+                               demcmc_eval_xdot expose it, which is how the parity tests pin the DMMA kernels.
+                               MVNORMAL_FULL: the centre is in data space, c = the column means or center[n_dim].  The
+                               data are centred BEFORE they are whitened, y = L^-1 (x - c), and each mean likewise,
+                               m' = L^-1 (mu - c); with NULL the y are then centred on their own column means (about 0)
+                               and B is analytically zero, with an explicit centre they are not, and
+                               B = sum_i y_i . L^-1 (mu - center). */
     const char *source;     /* CUSTOM: NUL-terminated CUDA C++ source (host memory), see DEMCMC_CUSTOM; else NULL */
 } demcmc_model;
 

@@ -755,6 +755,24 @@ def test_full_covariance_mvn_kernel():          # SURVEY 8f-4
     r, out = forced_run(case, 4, 16, 3, "replay", burnin=1, theta_snooker=0.1)
     assert out["counters"]["persistent_chunks"] > 0
     check(r, out)
+    # data 1e4 sd from 0 under a covariance of condition 1e6: the oracle whitens x_i - mu per observation, which does
+    # not cancel at the offset; the library centres before whitening for the same reason.  Crossover moves only: the
+    # snooker projection (utilities.jl:239-246) takes dot products of the UNCENTRED donor with a difference of size
+    # the spread, so at this offset the warp-order sums of the device and the oracle's sequential ones give proposals
+    # that differ by more than 1e-12 before any likelihood is evaluated (the snooker path is covered above)
+    dm = 10
+    q, _ = np.linalg.qr(rng.normal(size=(dm, dm)))
+    cov = (q * np.geomspace(1.0, 1e-6, dm)) @ q.T
+    cov = (cov + cov.T) / 2.0
+    mu = 1e4 * (1.0 + rng.uniform(size=dm))
+    x = rng.multivariate_normal(mu, cov, size=n)
+    xbar = x.mean(axis=0)
+    case = common.Case("mvn_full_offset", "mvnormal_full", dm + 1, [("flat",)] * dm + [("halfcauchy", 0, 1)],
+                       [-np.inf] * dm + [0], [np.inf] * (dm + 1),
+                       lambda r: list(rng.multivariate_normal(xbar, cov / n)) + [abs(r.normal(1, 0.05))], dict(x=x, cov=cov))
+    r, out = forced_run(case, 4, 16, 3, "replay", burnin=1, theta_snooker=0.0)
+    assert out["counters"]["persistent_chunks"] > 0
+    check(r, out)
 
 
 def test_vector_parameter_gaussian_example():   # Examples/Guassian_Example_Vector.jl
