@@ -523,6 +523,63 @@ def sample(model: DEModel, de: DE, *args, progress=False, device=0, devices=None
         h.close()
 
 
+def _comparison_handle(model: DEModel, d, device=0, devices=None):
+    """A handle bound to the model's likelihood alone, for the pointwise entry points: no sampler state, no run (they leave the
+    priors out, so every parameter gets a flat one here)."""
+    ll = model.loglike
+    if not isinstance(ll, GPULoglike):
+        raise TypeError("loglike must be a GPULoglike: only a model that runs on the device has pointwise log-likelihoods here")
+    n_dev = 1 if devices is None else max(1, len(devices))
+    h = Handle(n_dev, 3, d, [-np.inf] * d, [np.inf] * d, device=device, devices=devices)
+    try:
+        h.set_model(ll.kind, [("flat",)] * d, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov,
+                    source=ll.source)
+    except BaseException:
+        h.close()
+        raise
+    return h
+
+
+def _chain_draws(chains: Chains):
+    """The parameter draws of `chains` as theta[n_chains * n_steps][d], chain by chain."""
+    v = np.asarray(chains.value)
+    d = len(chains.names) - 2
+    n_steps, _, n_chains = v.shape
+    return np.ascontiguousarray(v[:, :d, :].transpose(2, 0, 1)).reshape(n_chains * n_steps, d), n_steps, n_chains
+
+
+def pointwise_loglikelihoods(model: DEModel, chains: Chains, device=0, devices=None):
+    """log p(y_i | theta) of every observation under every draw of `chains`, computed on the device: an array
+    (n_obs, n_steps, n_chains), the [data, step, chain] order ParetoSmooth.psis_loo takes.  Priors are left out; what an
+    observation is for each kind is stated at demcmc_eval_pointwise (include/demcmc_b200.h)."""
+    theta, n_steps, n_chains = _chain_draws(chains)
+    h = _comparison_handle(model, theta.shape[1], device, devices)
+    try:
+        out = h.eval_pointwise(theta)
+    finally:
+        h.close()
+    return out.reshape(n_chains, n_steps, -1).transpose(2, 1, 0)
+
+
+def loo(model: DEModel, chains: Chains, device=0, devices=None):
+    """PSIS-LOO and WAIC of the model over the draws of `chains` (at most 16384 draws; thin longer chains), Pareto
+    smoothing on the device (demcmc_loo, r_eff = 1).  Returns a dict: the totals elpd_loo, se_elpd_loo, p_loo, elpd_waic,
+    se_elpd_waic, p_waic and n_bad_k (observations with pareto_k > 0.7), and the per-observation arrays elpd_loo_i,
+    pareto_k, lppd_i, p_waic_i."""
+    theta, _, _ = _chain_draws(chains)
+    h = _comparison_handle(model, theta.shape[1], device, devices)
+    try:
+        elpd_i, k, lppd_i, pw_i = h.loo(theta)
+    finally:
+        h.close()
+    n = elpd_i.size
+    waic_i = lppd_i - pw_i
+    elpd = float(elpd_i.sum())
+    return {"elpd_loo": elpd, "se_elpd_loo": float(np.sqrt(n * np.var(elpd_i))), "p_loo": float(lppd_i.sum() - elpd),
+            "elpd_waic": float(waic_i.sum()), "se_elpd_waic": float(np.sqrt(n * np.var(waic_i))), "p_waic": float(pw_i.sum()),
+            "n_bad_k": int(np.sum(k > 0.7)), "elpd_loo_i": elpd_i, "pareto_k": k, "lppd_i": lppd_i, "p_waic_i": pw_i}
+
+
 class Particle:
     """What optimize returns per particle (src/structs.jl:202-223): Θ (one entry per named parameter),
     weight and id."""

@@ -55,6 +55,15 @@ int timer_stop(double *ms);
 size_t pack_ssd_doubles(const ModelDev &m);
 // center_host: nullptr = centre on the column means, else the [ssd_k] vector to centre on (host memory)
 int launch_pack_ssd(const double *x_in, int in_on_device, const double *center_host, ModelDev *m /* xT allocated */);
+// demcmc_eval_pointwise / demcmc_loo: out[i][n] = log p(y_(obs0 + i) | theta_s) for observations [obs0, obs0 + n_obs) of the
+// model and the n draws theta[n][d] (device), observation-major (k_ll_obs, k_ll_custom_obs behind ModelDev.custom)
+// Declared weak, like the custom-likelihood entry points below: the plain host-only test double does not define these
+// two, they resolve to null there, and the engine refuses the model-comparison calls with DEMCMC_EUNSUPPORTED
+// (tests/emu/emu_loo.cpp holds host versions that tests/test_loo.py builds into a test double of its own).
+int launch_pointwise(const ModelDev &m, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out_obs_major) __attribute__((weak));
+// PSIS-LOO and WAIC of each observation from ll[n_obs][n_draws] (device, 2 <= n_draws <= PSIS_MAX_DRAWS): the four outputs
+// [n_obs] (device), as include/demcmc_b200.h: demcmc_loo defines them (k_psis)
+int launch_psis(const double *ll, int64_t n_draws, int64_t n_obs, double *elpd_loo, double *pareto_k, double *lppd, double *p_waic) __attribute__((weak));
 // init_particle: weights of n particles theta[n][d] -> w[n] (also demcmc_eval)
 // xdot (MVN / hierarchical, may be nullptr): the cross term of every vector as the likelihood kernel produced it
 int launch_eval(const ConfigDev &cfg, const ModelDev &m, const double *theta, int64_t n, double *ll, double *prior,

@@ -508,4 +508,33 @@ DE_HD double binomial_ll(double N, double k, double p)
     return lc + a + b;
 }
 
+// ---- Pareto-smoothed importance sampling (include/demcmc_b200.h: demcmc_loo) ----------------------------------------
+// The scalar algebra of the generalized-Pareto fit of Zhang & Stephens (2009) as ArviZ's _gpdfit / _gpinv write it, shared
+// by k_psis and the host test double.  y[0..n) is the sorted tail, m = 30 + floor(sqrt(n)) grid points.
+// grid point j of the fit: b_j = (1 - sqrt(m / (j + 1/2))) / (3 y[q]) + 1 / y[n - 1],  q = floor(n / 4 + 1/2) - 1
+DE_HD int gpd_grid_len(int n) { return 30 + (int)sqrt((double)n); }
+DE_HD int gpd_quartile_index(int n) { return (int)((double)n / 4.0 + 0.5) - 1; }
+DE_HD double gpd_grid_b(int j, int m, double y_q, double y_max)
+{
+    return (1.0 - sqrt((double)m / ((double)(j + 1) - 0.5))) / (3.0 * y_q) + 1.0 / y_max;
+}
+// profile log-likelihood of grid point b given kbar = mean_i log1p(-b y_i): n (log(-b / kbar) - kbar - 1)
+DE_HD double gpd_profile(double b, double kbar, int n) { return (double)n * (log(-(b / kbar)) - kbar - 1.0); }
+// the weakly informative prior on k (ArviZ: prior_k = 10 pseudo-observations at k = 1/2)
+DE_HD double gpd_k_prior(double k, int n) { return ((double)n * k + 10.0 * 0.5) / ((double)n + 10.0); }
+// GPD quantile at probability p in (0, 1) with shape k and scale sigma
+DE_HD double gpd_inv(double p, double k, double sigma)
+{
+    if (!(sigma > 0.0)) return qnan();
+    const double x = fabs(k) < 2.220446049250313e-16 ? -log1p(-p) : expm1(-k * log1p(-p)) / k;
+    return x * sigma;
+}
+// tail length M = ceil(min(S / 5, 3 sqrt(S))) of S draws (r_eff = 1)
+DE_HD int psis_tail_len(int S)
+{
+    const double a = 0.2 * (double)S, b = 3.0 * sqrt((double)S);
+    return (int)ceil(a < b ? a : b);
+}
+#define DE_LOG_DBL_MIN (-708.39641853226410622)   // log(DBL_MIN): the floor of the tail cutoff
+
 } // namespace de

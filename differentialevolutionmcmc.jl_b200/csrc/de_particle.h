@@ -101,6 +101,23 @@ DE_HD double finalize_ll(const ModelDev &m, const double *theta, double total, d
     }
 }
 
+// one observation of the MVN / hierarchical kinds (demcmc_eval_pointwise): the log density is c0 - (q / s2) / 2, q the
+// squared distance of the centred observation from the centred mean -- finalize_ll's terms for a single observation
+DE_HD void ssd_obs_const(const ModelDev &m, const double *theta, double &c0, double &s2)
+{
+    const double dm = (double)m.n_dim;
+    if (m.kind == M_HIER) {
+        const double sig = theta[m.n_dim + 2];
+        s2 = sig * sig;
+        c0 = -(DE_LOG2PI / 2.0 + log(sig));
+        return;
+    }
+    const double sig = theta[m.n_dim];
+    s2 = sig * sig;
+    c0 = m.kind == M_MVN_FULL ? -(dm * DE_LOG2PI + (dm * log(s2) + m.logdet)) / 2.0 : -(dm * DE_LOG2PI + dm * log(s2)) / 2.0;
+}
+DE_HD double ssd_obs_ll(double c0, double s2, double q) { return c0 - (q / s2) / 2.0; }
+
 // in_bounds (utilities.jl:70-78) + prior_loglike of one parameter vector
 template <class C>
 DE_HD void bounds_and_prior(const C &co, const ConfigDev &cfg, const ModelDev &m, const double *theta, bool &inb, double &prior)

@@ -17,6 +17,8 @@ constexpr int PW_THREADS = 256;
 enum ModelKind { M_GAUSSIAN = 0, M_MVNORMAL = 1, M_BINOMIAL = 2, M_LNR = 3, M_LBA = 4, M_HIER = 5, M_RASTRIGIN = 6, M_MVN_FULL = 7,
                  M_CUSTOM = 8 /* user-written per-observation density compiled at run time (kernels.cu: k_ll_custom) */ };
 constexpr int CUSTOM_MAX_PAR = 256;   // d and DEMCMC_NPAR of a custom model (the per-particle values staged in shared memory)
+constexpr int PSIS_MAX_DRAWS = 16384; // draws of one demcmc_loo call: k_psis holds an observation's values in 128 KB of shared memory
+constexpr int PSIS_MAX_TAIL = 512;    // >= the tail length ceil(3 sqrt(PSIS_MAX_DRAWS)) = 384, a power of two (bitonic sort)
 // the likelihoods that are a sum of squared deviations from per-dimension means (the streamed DMMA kernels k_xdot / k_chunk_persist)
 DE_HD bool is_ssd(int kind) { return kind == M_MVNORMAL || kind == M_HIER || kind == M_MVN_FULL; }
 enum { UPDATE_MH = 0, UPDATE_MAXIMIZE = 1, UPDATE_MINIMIZE = 2 };

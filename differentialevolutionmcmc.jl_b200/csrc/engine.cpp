@@ -1773,6 +1773,77 @@ static int eval_impl(demcmc_handle *h, const double *theta, int64_t n, double *l
     return rc;
 }
 
+// ---- model comparison: pointwise log-likelihoods and PSIS-LOO / WAIC ------------------------------------------------
+static_assert(PSIS_MAX_DRAWS == DEMCMC_LOO_MAX_DRAWS, "k_psis holds DEMCMC_LOO_MAX_DRAWS values per observation");
+// observations per chunk: the ll[obs][draw] scratch stays at 256 MB whatever the data size
+static int64_t obs_chunk(int64_t n_draws) { return std::max<int64_t>(1, ((int64_t)1 << 25) / std::max<int64_t>(1, n_draws)); }
+
+// out: the caller's output, (draw, observation o) at out[draw * ld + col0 + o] (eval_pointwise), or nullptr (loo: the four
+// per-observation outputs at lo[q] + obs0, each may be nullptr)
+static int pointwise_slice(demcmc_handle *h, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out, int64_t ld,
+                           int64_t col0, double *const lo[4])
+{
+    BE(be::set_device(h->cfg.device));
+    if (n_obs <= 0) return 0;
+    const int64_t chunk = std::min(n_obs, obs_chunk(n));
+    DevBuf buf;
+    double *dt = buf.up(theta, (size_t)n * h->d), *ll = buf.up<double>(nullptr, (size_t)chunk * n);
+    double *dout = out ? nullptr : buf.up<double>(nullptr, (size_t)4 * chunk);
+    if (!dt || !ll || (!out && !dout)) return fail(DEMCMC_ENOMEM, "pointwise workspace does not fit: %s", be::last_error());
+    std::vector<double> host(out ? (size_t)chunk * n : 0);
+    for (int64_t c0 = 0; c0 < n_obs; c0 += chunk) {
+        const int64_t nc = std::min(chunk, n_obs - c0);
+        BE(be::launch_pointwise(h->dmodel, dt, n, obs0 + c0, nc, ll));
+        if (out) {
+            BE(be::d2h(host.data(), ll, sizeof(double) * nc * n));
+            for (int64_t s = 0; s < n; ++s)
+                for (int64_t o = 0; o < nc; ++o) out[s * ld + col0 + c0 + o] = host[(size_t)o * n + s];
+        } else {
+            BE(be::launch_psis(ll, n, nc, dout, dout + chunk, dout + 2 * chunk, dout + 3 * chunk));
+            for (int q = 0; q < 4; ++q)
+                if (lo[q]) BE(be::d2h(lo[q] + obs0 + c0, dout + (size_t)q * chunk, sizeof(double) * nc));
+        }
+    }
+    return 0;
+}
+
+// the checks both entry points share, then the observations split over the devices of a multi-device handle
+static int pointwise_call(demcmc_handle *h, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out, double *const lo[4])
+{
+    if (!h || !theta || n < 0) return fail(DEMCMC_EINVAL, "bad argument");
+    if (!h->has_model) return fail(DEMCMC_ESTATE, "set_model first");
+    if (!be::launch_pointwise || !be::launch_psis) return fail(DEMCMC_EUNSUPPORTED, "this backend (%s) has no pointwise kernels", be::name());
+    const int64_t N = h->dmodel.n_obs;
+    if (N <= 0) return fail(DEMCMC_EINVAL, "the model has no observations (RASTRIGIN, or CUSTOM with n_obs = 0): nothing to compare");
+    if (obs0 < 0 || n_obs < 0 || obs0 > N - n_obs)
+        return fail(DEMCMC_EINVAL, "observations [%lld, %lld) outside [0, %lld)", (long long)obs0, (long long)(obs0 + n_obs), (long long)N);
+    if (n == 0) return 0;
+    if (!h->multi) return pointwise_slice(h, theta, n, obs0, n_obs, out, n_obs, 0, lo);
+    const int64_t K = (int64_t)h->kids.size();
+    return for_kids(h, [&](demcmc_handle *k, int i) {
+        const int64_t a = n_obs * i / K, b = n_obs * (i + 1) / K;
+        return pointwise_slice(k, theta, n, obs0 + a, b - a, out, n_obs, a, lo);
+    });
+}
+
+int demcmc_eval_pointwise(demcmc_handle *h, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out)
+{
+    if (!out) return fail(DEMCMC_EINVAL, "null out");
+    double *const none[4] = { nullptr, nullptr, nullptr, nullptr };
+    return pointwise_call(h, theta, n, obs0, n_obs, out, none);
+}
+
+int demcmc_loo(demcmc_handle *h, const double *theta, int64_t n, double *elpd_loo, double *pareto_k, double *lppd, double *p_waic)
+{
+    if (h && theta && n < 2) return fail(DEMCMC_EINVAL, "PSIS needs at least 2 draws, got %lld", (long long)n);
+    if (n > DEMCMC_LOO_MAX_DRAWS)
+        return fail(DEMCMC_EUNSUPPORTED, "%lld draws: demcmc_loo takes at most %d (one observation's values are held in shared memory); "
+                    "thin the draws", (long long)n, DEMCMC_LOO_MAX_DRAWS);
+    double *const lo[4] = { elpd_loo, pareto_k, lppd, p_waic };
+    const int64_t N = (h && h->has_model) ? h->dmodel.n_obs : 0;
+    return pointwise_call(h, theta, n, 0, N, nullptr, lo);
+}
+
 
 int demcmc_op_project(int device, const double *p1, const double *p2, int32_t d, double *out)
 {

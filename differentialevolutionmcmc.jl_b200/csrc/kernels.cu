@@ -2180,6 +2180,41 @@ extern "C" __global__ void __launch_bounds__(256) k_ll_custom(const double *thet
         part[(size_t)p * n_split + split] = v;
     }
 }
+
+// demcmc_eval_pointwise / demcmc_loo: every demcmc_obs value of 32 draws (one per lane) x 64 observations (8 per warp),
+// written to out[obs][draw] instead of summed (kernels.cu: k_ll_obs).  Each draw's par row sits in dynamic shared memory,
+// its length made odd so that the lanes' rows start in different banks; the host reads the length from demcmc_custom_npar.
+#ifdef DEMCMC_NPAR
+extern "C" __device__ int demcmc_custom_npar = DEMCMC_NPAR;
+#else
+extern "C" __device__ int demcmc_custom_npar = 0;
+#endif
+extern "C" __global__ void __launch_bounds__(256) k_ll_custom_obs(const double *theta, int d, long long n, const double *x, int n_cols,
+                                                                  long long obs0, long long n_obs, double *out)
+{
+    extern __shared__ double demcmc_pars_[];
+#ifdef DEMCMC_NPAR
+    const int row = DEMCMC_NPAR | 1;
+#else
+    const int row = d | 1;
+#endif
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long s0 = (long long)blockIdx.y * 32, i0 = (long long)blockIdx.x * 64;
+#ifdef DEMCMC_NPAR
+    if (threadIdx.x < 32 && s0 + threadIdx.x < n) demcmc_prepare(theta + (size_t)(s0 + threadIdx.x) * d, demcmc_pars_ + threadIdx.x * row);
+#else
+    for (int e = threadIdx.x; e < 32 * d; e += 256) {
+        const int t = e / d, k = e - t * d;
+        if (s0 + t < n) demcmc_pars_[t * row + k] = theta[(size_t)(s0 + t) * d + k];
+    }
+#endif
+    __syncthreads();
+    if (s0 + lane >= n) return;
+    const double *par = demcmc_pars_ + lane * row;
+    const int no = (int)min(64LL, n_obs - i0);
+    for (int o = warp; o < no; o += 8)
+        out[(size_t)(i0 + o) * n + s0 + lane] = (double)demcmc_obs(par, x + (size_t)(obs0 + i0 + o) * n_cols);
+}
 )CU";
 
 struct NvrtcApi {
@@ -2250,7 +2285,7 @@ int custom_compile(const char *source)
     return custom_cubin(source, &cubin);
 }
 
-struct CustomModule { cudaLibrary_t lib; cudaKernel_t kernel; };
+struct CustomModule { cudaLibrary_t lib; cudaKernel_t kernel, obs_kernel; int npar; };
 
 int custom_load(const char *source, void **module, int *has_obs)
 {
@@ -2270,6 +2305,9 @@ int custom_load(const char *source, void **module, int *has_obs)
     size_t bytes = 0;
     if (e == cudaSuccess) e = cudaLibraryGetGlobal(&flag, &bytes, mod->lib, "demcmc_custom_has_obs");
     if (e == cudaSuccess) e = cudaMemcpy(has_obs, flag, sizeof(int), cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaLibraryGetKernel(&mod->obs_kernel, mod->lib, "k_ll_custom_obs");
+    if (e == cudaSuccess) e = cudaLibraryGetGlobal(&flag, &bytes, mod->lib, "demcmc_custom_npar");
+    if (e == cudaSuccess) e = cudaMemcpy(&mod->npar, flag, sizeof(int), cudaMemcpyDeviceToHost);
     if (e != cudaSuccess) { cudaLibraryUnload(mod->lib); delete mod; cu_fail(e, "loading k_ll_custom"); return -3; }
     *module = mod;
     return 0;
@@ -2463,6 +2501,350 @@ int launch_eval(const ConfigDev &cfg, const ModelDev &m, const double *theta, in
     k_eval_finish<<<blocks, PA_THREADS, 0, stream()>>>(cfg, m, theta, n, scratch_part, acc, q, ll, prior, w, xdot);
     LAUNCHED("k_eval_finish");
     if (acc) { cudaStreamSynchronize(stream()); dfree(acc); dfree(q); }
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// model comparison (demcmc_eval_pointwise / demcmc_loo)
+//   k_ll_obs<KIND>  the pointwise matrix out[obs][draw] of a tile of 32 draws (one per lane) x 64 observations (8 per
+//                   warp): every density is the per-observation function the summed likelihood uses (de_math.h), so a
+//                   warp reads one observation (a broadcast) and writes 32 consecutive doubles.  The streamed kinds take
+//                   the centred data x' from the packed xT and the centred means from k_ll_obs_prep, and form
+//                   |x'_i - m'|^2 directly on the CUDA cores.
+//   k_psis          one CTA per observation, its S values in dynamic shared memory: max / min / sums, a radix select of
+//                   the cutoff on order-preserving 64-bit keys, a bitonic sort of the tail, the GPD fit with its m x M
+//                   log1p terms split over the warps, the smoothing and the four outputs.  Every reduction runs in a
+//                   fixed order (per thread, warp tree, warps in order), so the outputs do not depend on the launch.
+// ------------------------------------------------------------------------------------------------
+constexpr int OB_TD = 32;            // draws per CTA, one per lane
+constexpr int OB_TO = 64;            // observations per CTA, 8 per warp
+constexpr int OB_THREADS = 256;
+constexpr int OB_KC = 32;            // dimensions of the streamed kinds staged per step
+
+// the streamed kinds: centred means transposed, mt[k][n] (lanes read consecutive draws), and the per-draw constants
+__global__ void __launch_bounds__(256) k_ll_obs_prep(ModelDev m, const double *theta, int64_t n, double *mt, double *c0, double *s2)
+{
+    const int64_t t = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (t >= n * m.ssd_k) return;
+    const int k = (int)(t / n);
+    const int64_t s = t - (int64_t)k * n;
+    const double *th = theta + (size_t)s * m.d;
+    mt[t] = centred_mean(m, th, k);
+    if (k == 0) ssd_obs_const(m, th, c0[s], s2[s]);
+}
+
+template <int KIND>
+__global__ void __launch_bounds__(OB_THREADS) k_ll_obs(const __grid_constant__ ModelDev m, const double *theta, int64_t n, int64_t obs0,
+                                                      int64_t n_obs, const double *mt, const double *c0, const double *s2, double *out)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t s0 = (int64_t)blockIdx.y * OB_TD, i0 = (int64_t)blockIdx.x * OB_TO;
+    const int64_t s = s0 + lane;
+    const int no = (int)min((int64_t)OB_TO, n_obs - i0);
+    const int64_t n_tiles = m.ssd_ld / SSD_TN;
+    if (KIND == M_MVNORMAL || KIND == M_MVN_FULL) {
+        __shared__ double xs[OB_TO][OB_KC + 1];
+        __shared__ double ms[OB_KC][OB_TD];
+        double acc[OB_TO / 8];
+#pragma unroll
+        for (int q = 0; q < OB_TO / 8; ++q) acc[q] = 0.0;
+        for (int k0 = 0; k0 < m.ssd_k; k0 += OB_KC) {
+            const int kc = min(OB_KC, m.ssd_k - k0);
+            __syncthreads();
+            for (int e = threadIdx.x; e < OB_TO * OB_KC; e += OB_THREADS) {
+                const int o = e / OB_KC, k = e % OB_KC;
+                xs[o][k] = (o < no && k < kc) ? m.xT[ssd_pack_index(obs0 + i0 + o, k0 + k, m.ksplit_len, m.ssd_nj, n_tiles, m.ssd_half)] : 0.0;
+            }
+            for (int e = threadIdx.x; e < OB_KC * OB_TD; e += OB_THREADS) {
+                const int k = e / OB_TD, t = e % OB_TD;
+                ms[k][t] = (k < kc && s0 + t < n) ? mt[(size_t)(k0 + k) * n + s0 + t] : 0.0;
+            }
+            __syncthreads();
+            for (int k = 0; k < kc; ++k) {
+                const double mk = ms[k][lane];
+#pragma unroll
+                for (int q = 0; q < OB_TO / 8; ++q) { const double dl = xs[warp + 8 * q][k] - mk; acc[q] = __fma_rn(dl, dl, acc[q]); }
+            }
+        }
+        if (s >= n) return;
+        const double a = c0[s], b = s2[s];
+#pragma unroll
+        for (int q = 0; q < OB_TO / 8; ++q) {
+            const int o = warp + 8 * q;
+            if (o < no) out[(size_t)(i0 + o) * n + s] = ssd_obs_ll(a, b, acc[q]);
+        }
+    } else if (KIND == M_HIER) {
+        if (s >= n) return;
+        const double a = c0[s], b = s2[s];
+        for (int o = warp; o < no; o += 8) {
+            const int64_t i = obs0 + i0 + o;
+            const int subj = (int)(i / m.n_per);
+            const double dl = m.xT[ssd_pack_index(i - (int64_t)subj * m.n_per, subj, m.ksplit_len, m.ssd_nj, n_tiles, m.ssd_half)] -
+                              mt[(size_t)subj * n + s];
+            out[(size_t)(i0 + o) * n + s] = ssd_obs_ll(a, b, dl * dl);
+        }
+    } else if (KIND == M_BINOMIAL) {
+        if (s < n && warp == 0) out[s] = binomial_ll(m.binom_N, m.binom_k, theta[(size_t)s * m.d]);
+    } else {
+        __shared__ double par[OB_TD][MAX_ACC + 5];
+        if (threadIdx.x < OB_TD && s0 + threadIdx.x < n) pointwise_par<KIND>(m, theta + (size_t)(s0 + threadIdx.x) * m.d, par[threadIdx.x]);
+        __syncthreads();
+        if (s >= n) return;
+        const double *sg = m.has_sigma ? m.sigma_acc : nullptr;
+        for (int o = warp; o < no; o += 8) {
+            const int64_t i = obs0 + i0 + o;
+            const double x = m.x[i];
+            double v;
+            if (KIND == M_GAUSSIAN) v = gaussian_obs(par[lane], x);
+            else if (KIND == M_LNR) v = lnr_obs(par[lane], m.n_dim, sg, x, m.choice[i] - 1);
+            else v = lba_obs(par[lane], m.n_dim, par[lane][m.n_dim + 3], m.lba_floor, x, m.choice[i] - 1);
+            out[(size_t)(i0 + o) * n + s] = v;
+        }
+    }
+}
+
+static int launch_ll_custom_obs(const ModelDev &m, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out)
+{
+    if (!m.custom) { g_be_err = "custom likelihood not loaded"; return -1; }
+    const CustomModule *mod = (const CustomModule *)m.custom;
+    const size_t smem = sizeof(double) * OB_TD * (size_t)((mod->npar > 0 ? mod->npar : m.d) | 1);
+    CU(cudaFuncSetAttribute((const void *)mod->obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int d = m.d, n_cols = m.n_cols;
+    long long nn = n, o0 = obs0, no = n_obs;
+    const double *x = m.x;
+    void *args[] = { &theta, &d, &nn, &x, &n_cols, &o0, &no, &out };
+    CU(cudaLaunchKernel((const void *)mod->obs_kernel, dim3((unsigned)((n_obs + OB_TO - 1) / OB_TO), (unsigned)((n + OB_TD - 1) / OB_TD)),
+                        dim3(OB_THREADS), args, smem, stream()));
+    LAUNCHED("k_ll_custom_obs");
+    return 0;
+}
+
+int launch_pointwise(const ModelDev &m, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out)
+{
+    if (n <= 0 || n_obs <= 0) return 0;
+    if (n > (int64_t)65535 * OB_TD) { g_be_err = "too many draws for one pointwise launch"; return -1; }
+    if (m.kind == M_CUSTOM) return launch_ll_custom_obs(m, theta, n, obs0, n_obs, out);
+    const dim3 grid((unsigned)((n_obs + OB_TO - 1) / OB_TO), (unsigned)((n + OB_TD - 1) / OB_TD));
+    double *mt = nullptr, *c0 = nullptr, *s2 = nullptr;
+    if (is_ssd(m.kind)) {
+        mt = (double *)dmalloc(sizeof(double) * (size_t)n * m.ssd_k);
+        c0 = (double *)dmalloc(sizeof(double) * (size_t)n);
+        s2 = (double *)dmalloc(sizeof(double) * (size_t)n);
+        if (!mt || !c0 || !s2) { dfree(mt); dfree(c0); dfree(s2); return -1; }
+        k_ll_obs_prep<<<(unsigned)((n * m.ssd_k + 255) / 256), 256, 0, stream()>>>(m, theta, n, mt, c0, s2);
+        ++g_launches;
+    }
+    switch (m.kind) {
+    case M_GAUSSIAN: k_ll_obs<M_GAUSSIAN><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_LNR: k_ll_obs<M_LNR><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_LBA: k_ll_obs<M_LBA><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_BINOMIAL: k_ll_obs<M_BINOMIAL><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_MVNORMAL: k_ll_obs<M_MVNORMAL><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_MVN_FULL: k_ll_obs<M_MVN_FULL><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    case M_HIER: k_ll_obs<M_HIER><<<grid, OB_THREADS, 0, stream()>>>(m, theta, n, obs0, n_obs, mt, c0, s2, out); break;
+    default: dfree(mt); dfree(c0); dfree(s2); g_be_err = "no pointwise kernel for this model kind"; return -1;
+    }
+    const cudaError_t e = cudaGetLastError();
+    ++g_launches;
+    dfree(mt); dfree(c0); dfree(s2);                 // stream-ordered: freed after the kernel has run
+    if (e != cudaSuccess) return cu_fail(e, "k_ll_obs");
+    return 0;
+}
+
+// ---- k_psis -------------------------------------------------------------------------------------
+constexpr int PS_THREADS = 256;
+constexpr int PS_WARPS = PS_THREADS / 32;
+constexpr int PS_MAX_GRID = 64;      // >= 30 + floor(sqrt(PSIS_MAX_TAIL))
+
+// fixed-order block reductions: per thread, then the warp's xor tree, then the warps in order (every thread forms the same
+// value from the same eight partials)
+struct PsSum { __device__ __forceinline__ double operator()(double a, double b) const { return a + b; } };
+struct PsMax { __device__ __forceinline__ double operator()(double a, double b) const { return fmax(a, b); } };
+struct PsMin { __device__ __forceinline__ double operator()(double a, double b) const { return fmin(a, b); } };
+template <class Op>
+__device__ __forceinline__ double ps_reduce(double v, double *red, Op op)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = op(v, __shfl_xor_sync(0xffffffffu, v, o));
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double r = red[0];
+#pragma unroll
+    for (int w = 1; w < PS_WARPS; ++w) r = op(r, red[w]);
+    __syncthreads();
+    return r;
+}
+// order-preserving 64-bit key of a double (larger value, larger key)
+__device__ __forceinline__ unsigned long long ps_key(double x)
+{
+    const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double ps_unkey(unsigned long long k)
+{
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
+__global__ void __launch_bounds__(PS_THREADS) k_psis(const double *ll, int S, double *elpd_out, double *k_out, double *lppd_out, double *pw_out)
+{
+    extern __shared__ double v[];                   // [S] the observation's log-likelihoods
+    __shared__ double tv[PSIS_MAX_TAIL];            // tail: log ratio (then its smoothed value) ...
+    __shared__ int ti[PSIS_MAX_TAIL];               // ... and its draw
+    __shared__ double ty[PSIS_MAX_TAIL];            // exp(x) - exp(cutoff)
+    __shared__ double gb[PS_MAX_GRID], gl[PS_MAX_GRID], gw[PS_MAX_GRID];
+    __shared__ unsigned hist[256];
+    __shared__ double red[PS_WARPS];
+    __shared__ int sh_digit, sh_rank, sh_nt;
+    __shared__ double sh_b;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const size_t obs = blockIdx.x;
+    const double *src = ll + obs * (size_t)S;
+    bool fin = true;
+    double mn = HUGE_VAL, mx = -HUGE_VAL, sum = 0.0;
+    for (int s = tid; s < S; s += PS_THREADS) { const double a = src[s]; v[s] = a; fin = fin && isfinite(a); mn = fmin(mn, a); mx = fmax(mx, a); sum += a; }
+    if (!__syncthreads_and(fin)) {
+        if (tid == 0) { const double q = qnan(); elpd_out[obs] = q; k_out[obs] = q; lppd_out[obs] = q; pw_out[obs] = q; }
+        return;
+    }
+    mn = ps_reduce(mn, red, PsMin());
+    mx = ps_reduce(mx, red, PsMax());
+    sum = ps_reduce(sum, red, PsSum());
+    double e = 0.0, q = 0.0;
+    const double mean = sum / (double)S;
+    for (int s = tid; s < S; s += PS_THREADS) { const double a = v[s]; e += exp(a - mx); const double dl = a - mean; q += dl * dl; }
+    e = ps_reduce(e, red, PsSum());
+    q = ps_reduce(q, red, PsSum());
+    // (M+1)-th largest log ratio x_s = mn - ll_s (= -ll_s - max(-ll)): MSB-first radix select, 8 bits a pass
+    const int M = psis_tail_len(S);
+    unsigned long long prefix = 0, mask = 0;
+    int rank = M + 1;
+    for (int shift = 56; shift >= 0; shift -= 8) {
+        hist[tid] = 0;
+        __syncthreads();
+        for (int s = tid; s < S; s += PS_THREADS) {
+            const unsigned long long k = ps_key(mn - v[s]);
+            if ((k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+        }
+        __syncthreads();
+        if (warp == 0) {                            // lane L holds bins 255 - 8L .. 248 - 8L, counted from the top
+            int c[8], tot = 0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) { c[j] = (int)hist[255 - 8 * lane - j]; tot += c[j]; }
+            int inc = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += y; }
+            const int exc = inc - tot;
+            if (exc < rank && rank <= inc) {
+                int a = exc;
+                for (int j = 0; j < 8; ++j) {
+                    if (a + c[j] >= rank) { sh_digit = 255 - 8 * lane - j; sh_rank = rank - a; break; }
+                    a += c[j];
+                }
+            }
+        }
+        __syncthreads();
+        prefix |= (unsigned long long)sh_digit << shift;
+        mask |= 0xFFull << shift;
+        rank = sh_rank;
+    }
+    const double cutoff = fmax(ps_unkey(prefix), DE_LOG_DBL_MIN);
+    // the tail, sorted by (x, draw): padding sorts last
+    if (tid == 0) sh_nt = 0;
+    for (int j = tid; j < PSIS_MAX_TAIL; j += PS_THREADS) { tv[j] = HUGE_VAL; ti[j] = 0x7fffffff; }
+    __syncthreads();
+    for (int s = tid; s < S; s += PS_THREADS) {
+        const double x = mn - v[s];
+        if (x > cutoff) { const int j = atomicAdd(&sh_nt, 1); tv[j] = x; ti[j] = s; }
+    }
+    __syncthreads();
+    const int nt = sh_nt;
+    for (int size = 2; size <= PSIS_MAX_TAIL; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = tid; t < PSIS_MAX_TAIL / 2; t += PS_THREADS) {
+                const int a = 2 * t - (t & (stride - 1)), b = a + stride;
+                const bool up = (a & size) == 0;
+                const bool gt = tv[a] > tv[b] || (tv[a] == tv[b] && ti[a] > ti[b]);
+                if (gt == up) { const double x = tv[a]; tv[a] = tv[b]; tv[b] = x; const int i = ti[a]; ti[a] = ti[b]; ti[b] = i; }
+            }
+            __syncthreads();
+        }
+    double khat = HUGE_VAL;
+    if (nt > 4) {
+        const double ec = exp(cutoff);
+        for (int j = tid; j < nt; j += PS_THREADS) ty[j] = exp(tv[j]) - ec;
+        __syncthreads();
+        const int m = gpd_grid_len(nt);
+        const double yq = ty[gpd_quartile_index(nt)], ymax = ty[nt - 1];
+        for (int g = warp; g < m; g += PS_WARPS) {
+            const double b = gpd_grid_b(g, m, yq, ymax);
+            double a = 0.0;
+            for (int j = lane; j < nt; j += 32) a += log1p(-b * ty[j]);
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+            if (lane == 0) { gb[g] = b; gl[g] = gpd_profile(b, a / (double)nt, nt); }
+        }
+        __syncthreads();
+        if (tid < m) {
+            double a = 0.0;
+            for (int h = 0; h < m; ++h) a += exp(gl[h] - gl[tid]);
+            gw[tid] = 1.0 / a;
+        }
+        __syncthreads();
+        if (tid == 0) {
+            const double floor_w = 10.0 * 2.220446049250313e-16;
+            double W = 0.0, b = 0.0;
+            for (int g = 0; g < m; ++g) if (gw[g] >= floor_w) W += gw[g];
+            for (int g = 0; g < m; ++g) if (gw[g] >= floor_w) b += gb[g] * (gw[g] / W);
+            sh_b = b;
+        }
+        __syncthreads();
+        const double b = sh_b;
+        double kp = 0.0;
+        for (int j = tid; j < nt; j += PS_THREADS) kp += log1p(-b * ty[j]);
+        kp = ps_reduce(kp, red, PsSum()) / (double)nt;
+        const double sigma = -kp / b;
+        khat = gpd_k_prior(kp, nt);
+        if (isfinite(khat))
+            for (int j = tid; j < nt; j += PS_THREADS) {
+                double t = log(gpd_inv(((double)j + 0.5) / (double)nt, khat, sigma) + ec);
+                if (t > 0.0) t = 0.0;
+                tv[j] = t;
+            }
+        __syncthreads();
+    }
+    // log weights lw = x' - logsumexp(x'), then elpd = logsumexp(lw + ll): the body draws (x <= cutoff), then the tail
+    double xm = -HUGE_VAL;
+    for (int s = tid; s < S; s += PS_THREADS) { const double x = mn - v[s]; if (!(x > cutoff)) xm = fmax(xm, x); }
+    for (int j = tid; j < nt; j += PS_THREADS) xm = fmax(xm, tv[j]);
+    xm = ps_reduce(xm, red, PsMax());
+    double se = 0.0;
+    for (int s = tid; s < S; s += PS_THREADS) { const double x = mn - v[s]; if (!(x > cutoff)) se += exp(x - xm); }
+    for (int j = tid; j < nt; j += PS_THREADS) se += exp(tv[j] - xm);
+    const double lse = xm + log(ps_reduce(se, red, PsSum()));
+    double tm = -HUGE_VAL;
+    for (int s = tid; s < S; s += PS_THREADS) { const double x = mn - v[s]; if (!(x > cutoff)) tm = fmax(tm, (x - lse) + v[s]); }
+    for (int j = tid; j < nt; j += PS_THREADS) tm = fmax(tm, (tv[j] - lse) + v[ti[j]]);
+    tm = ps_reduce(tm, red, PsMax());
+    double st = 0.0;
+    for (int s = tid; s < S; s += PS_THREADS) { const double x = mn - v[s]; if (!(x > cutoff)) st += exp(((x - lse) + v[s]) - tm); }
+    for (int j = tid; j < nt; j += PS_THREADS) st += exp(((tv[j] - lse) + v[ti[j]]) - tm);
+    st = ps_reduce(st, red, PsSum());
+    if (tid == 0) {
+        elpd_out[obs] = tm + log(st);
+        k_out[obs] = khat;
+        lppd_out[obs] = mx + log(e) - log((double)S);
+        pw_out[obs] = q / (double)(S - 1);
+    }
+}
+
+int launch_psis(const double *ll, int64_t n_draws, int64_t n_obs, double *elpd, double *khat, double *lppd, double *p_waic)
+{
+    if (n_obs <= 0) return 0;
+    if (n_draws < 2 || n_draws > PSIS_MAX_DRAWS) { g_be_err = "k_psis takes 2 .. 16384 draws"; return -1; }
+    const size_t smem = sizeof(double) * (size_t)n_draws;
+    CU(cudaFuncSetAttribute(k_psis, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * PSIS_MAX_DRAWS)));
+    k_psis<<<(unsigned)n_obs, PS_THREADS, smem, stream()>>>(ll, (int)n_draws, elpd, khat, lppd, p_waic);
+    LAUNCHED("k_psis");
     return 0;
 }
 

@@ -62,6 +62,7 @@ class Handle:
         self.P_total = n_groups * Np
         self.B = max(1, nb)
         self.n_initial = n_initial
+        self.n_obs = 0                                      # observations of the bound model (set_model)
         self.store_every = max(1, int(store_every))
         self.iterations = 0
         self._last_iters = 0
@@ -151,6 +152,7 @@ class Handle:
                        int(n_cols or 0), ptr(cv, _dp), ptr(cen, _dp), src)
         self._keep = [xs, cs, sg, pr, cen, cv, src]
         check(_ffi.lib().demcmc_set_model(self._h, C.byref(m)))
+        self.n_obs = int(n_obs)
 
     # ---- state ---------------------------------------------------------------------------------
     def set_history(self, rows):
@@ -326,6 +328,23 @@ class Handle:
         pr = np.zeros(n)
         check(_ffi.lib().demcmc_eval(self._h, ptr(th, _dp), n, ptr(ll, _dp), ptr(pr, _dp)))
         return ll, pr
+
+    def eval_pointwise(self, theta, obs0=0, n_obs=None):
+        """log p(y_i | theta_s) for the draws theta[n][d] and observations [obs0, obs0 + n_obs) of the bound model (all from
+        obs0 by default): an array [n, n_obs] (demcmc_eval_pointwise; priors are left out)."""
+        th = f8(theta).reshape(-1, self.d)
+        n_obs = self.n_obs - obs0 if n_obs is None else int(n_obs)
+        out = np.empty((th.shape[0], max(n_obs, 0)))
+        check(_ffi.lib().demcmc_eval_pointwise(self._h, ptr(th, _dp), th.shape[0], int(obs0), n_obs, ptr(out, _dp)))
+        return out
+
+    def loo(self, theta):
+        """PSIS-LOO and WAIC of every observation over the draws theta[n][d] (demcmc_loo, 2 <= n <= 16384): the arrays
+        (elpd_loo, pareto_k, lppd, p_waic), each [n_obs]."""
+        th = f8(theta).reshape(-1, self.d)
+        out = [np.empty(self.n_obs) for _ in range(4)]
+        check(_ffi.lib().demcmc_loo(self._h, ptr(th, _dp), th.shape[0], *(ptr(a, _dp) for a in out)))
+        return tuple(out)
 
     def comm_init(self, uid: bytes, rank: int, n_ranks: int):
         buf = np.frombuffer(uid, dtype=np.uint8).copy()

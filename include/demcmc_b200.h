@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define DEMCMC_ABI_VERSION 5
+#define DEMCMC_ABI_VERSION 6
 
 enum { DEMCMC_OK = 0, DEMCMC_EINVAL = -1, DEMCMC_ENODEVICE = -2, DEMCMC_ECUDA = -3, DEMCMC_ENOMEM = -4,
        DEMCMC_ESTATE = -5, DEMCMC_EUNSUPPORTED = -6, DEMCMC_ECOMM = -7 };
@@ -315,6 +315,46 @@ int demcmc_eval_xdot(demcmc_handle *h, const double *theta, int64_t n, double *x
  * "loglike evals incl.", i.e. every observation streamed for every particle; bench.py reports this mode
  * separately (value_sufficient_stat).  Refused when the model was given an explicit center. */
 int demcmc_set_sufficient_stat(demcmc_handle *h, int32_t on);
+
+/* Model comparison: pointwise log-likelihoods, PSIS-LOO and WAIC on the device.
+ *
+ * An observation is what demcmc_model.n_obs counts: GAUSSIAN x_i; MVNORMAL / MVNORMAL_FULL row x_i, with the log density
+ * logpdf(MvNormal(mu, sigma^2 I or sigma^2 Sigma), x_i); HIER_NORMAL y_sj in the subject-major order of demcmc_model.x
+ * (n_obs = n_dim * n_per); LNR / LBA one trial; BINOMIAL the single (N, k) (n_obs = 1); CUSTOM row x_i, its log density
+ * the value demcmc_obs returns for it.
+ * Priors are left out, and so is the demcmc_particle term of a CUSTOM model (it belongs to no observation).  A model
+ * without observations (RASTRIGIN, CUSTOM with n_obs = 0) is refused with DEMCMC_EINVAL; so is an observation range
+ * outside [0, n_obs).  Before demcmc_set_model: DEMCMC_ESTATE.
+ *
+ * demcmc_loo is PSIS as in Vehtari, Simpson, Gelman, Yao & Gabry (2024), written as ArviZ's psislw / _gpdfit / _gpinv
+ * with relative efficiency r_eff = 1.  For each observation i, with ll_s = log p(y_i | theta_s), s < S = n:
+ *   1. log ratios r_s = -ll_s, shifted by their maximum: x_s = r_s - max r (so max x = 0);
+ *   2. tail length M = ceil(min(S / 5, 3 sqrt(S))); cutoff c = max(the (M+1)-th largest x_s, log(DBL_MIN)); the tail is the
+ *      n_t draws with x_s > c (n_t = M unless values tie at the cutoff), in increasing (x_s, s) order;
+ *   3. n_t <= 4: no smoothing and k-hat = +Inf;
+ *   4. otherwise the Zhang & Stephens (2009) fit to the sorted y_j = exp(x_j) - exp(c), j < n_t: m = 30 + floor(sqrt(n_t))
+ *      grid points b_g = (1 - sqrt(m / (g + 1/2))) / (3 y_q) + 1 / y_(n_t - 1), g < m, q = floor(n_t / 4 + 1/2) - 1;
+ *      kbar_g = mean_j log1p(-b_g y_j); profile l_g = n_t (log(-b_g / kbar_g) - kbar_g - 1); weight w_g = 1 / sum_h
+ *      exp(l_h - l_g); weights below 10 DBL_EPSILON are dropped and the rest normalised to sum 1; b = sum_g w_g b_g;
+ *      k = mean_j log1p(-b y_j), sigma = -k / b, and the prior adjustment k-hat = (n_t k + 5) / (n_t + 10);
+ *   5. if k-hat is finite, the tail value of rank j becomes log(F^-1((j + 1/2) / n_t) + exp(c)), F^-1 the GPD quantile
+ *      sigma (expm1(-k-hat log1p(-p)) / k-hat) (sigma (-log1p(-p)) when |k-hat| < DBL_EPSILON), and then every value
+ *      above 0 is set to 0;
+ *   6. log weights lw_s = x_s - logsumexp(x);
+ *   7. elpd_loo[i] = logsumexp_s(lw_s + ll_s), lppd[i] = logsumexp_s(ll_s) - log S, p_waic[i] = sum_s (ll_s - mean ll)^2 / (S - 1),
+ *      pareto_k[i] = k-hat.
+ * If any of an observation's S values is not finite, its four outputs are NaN (the call still returns 0).  Every sum is
+ * formed in a fixed order, so every output is the same bits from run to run and on any number of devices.  A multi-device
+ * handle gives each device a contiguous slice of the observations; a rank of a sharded job holds all the data and
+ * computes locally. */
+/* log p(y_i | theta_j) for n parameter vectors theta[n][d] and observations [obs0, obs0 + n_obs) of the bound model:
+ * out[n][n_obs] (Julia: n_obs x n, data fastest, the [data, draw] order ParetoSmooth.psis_loo takes) */
+int demcmc_eval_pointwise(demcmc_handle *h, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out);
+/* PSIS-LOO and WAIC per observation over the n draws theta[n][d], all observations of the bound model; each output
+ * [n_obs] may be NULL.  2 <= n <= DEMCMC_LOO_MAX_DRAWS (DEMCMC_EINVAL below, DEMCMC_EUNSUPPORTED above: thin the draws) */
+int demcmc_loo(demcmc_handle *h, const double *theta, int64_t n, double *elpd_loo, double *pareto_k,
+               double *lppd, double *p_waic);
+#define DEMCMC_LOO_MAX_DRAWS 16384
 
 /* Particle algebra on the device, for the reference's known-answer tests (test/utility_tests.jl):
  * project (utilities.jl:239-246), reset! (crossover.jl:336-352), random_gamma body

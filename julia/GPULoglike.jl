@@ -23,7 +23,7 @@
 # GPU path with a closure throws an ArgumentError -- there is no silent CPU fallback.
 
 const LIBDEMCMC = get(ENV, "LIBDEMCMC_B200", "libdemcmc_b200.so")
-const DEMCMC_ABI_VERSION = Int32(5)
+const DEMCMC_ABI_VERSION = Int32(6)
 
 const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7, custom = 8)
 const GPU_PRIORS = (flat = 0, normal = 1, halfcauchy = 2, uniform = 3, beta = 4, normal_ref = 5)
@@ -246,6 +246,26 @@ function sample(model::DEModel{<:GPULoglike}, de::DE, ::MCMCThreads, n_iter::Int
     return _sample_gpu(model, de, n_iter; device, devices, store_every, seed)    # every group is always updated concurrently on the device(s)
 end
 
+# demcmc_model's n_dim, n_per, n_obs, n_cols of a GPULoglike with d flattened parameters
+function model_geometry(ll::GPULoglike, d)
+    x = ll.data.x
+    n_dim, n_per, n_obs, n_cols = 0, 0, length(x), 0
+    if ll.kind == :custom
+        n_cols, n_obs = size(x)
+    elseif ll.kind == :mvnormal || ll.kind == :mvnormal_full
+        n_dim, n_obs = size(x)
+    elseif ll.kind == :hier_normal
+        n_per, n_dim = size(x); n_obs = n_dim * n_per
+    elseif ll.kind == :lnr
+        n_dim = d - 1
+    elseif ll.kind == :lba
+        n_dim = d - 3
+    elseif ll.kind == :binomial
+        n_obs = 1
+    end
+    return n_dim, n_per, n_obs, n_cols
+end
+
 function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_every = 1, return_particles = false)
     store_every == 1 || return_particles === false || throw(ArgumentError("optimize keeps every row"))
     store_every == 1 || return _sample_gpu_thinned(model, de, n_iter; device, devices, store_every, seed)
@@ -277,22 +297,9 @@ function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_e
     priors = prior_table(model, Θ1)
     x = ll.data.x
     choice = ll.data.choice
-    n_dim, n_per, n_obs, n_cols = 0, 0, length(x), 0
+    n_dim, n_per, n_obs, n_cols = model_geometry(ll, d)
     covm = ll.cov
     src = ll.source
-    if ll.kind == :custom
-        n_cols, n_obs = size(x)
-    elseif ll.kind == :mvnormal || ll.kind == :mvnormal_full
-        n_dim, n_obs = size(x)
-    elseif ll.kind == :hier_normal
-        n_per, n_dim = size(x); n_obs = n_dim * n_per
-    elseif ll.kind == :lnr
-        n_dim = d - 1
-    elseif ll.kind == :lba
-        n_dim = d - 3
-    elseif ll.kind == :binomial
-        n_obs = 1
-    end
     h = Ref{Ptr{Cvoid}}(C_NULL)
     n_rows = n_iter + de.n_initial
     samples = zeros(Float64, n_rows, d, P)          # Julia order == the library's output order
@@ -461,3 +468,62 @@ function optimize(model::DEModel{<:GPULoglike}, de::DE, n_iter::Int; progress = 
     return particles
 end
 optimize(model::DEModel{<:GPULoglike}, de::DE, ::MCMCThreads, n_iter::Int; kwargs...) = optimize(model, de, n_iter; kwargs...)
+
+# ---- model comparison ------------------------------------------------------------------------------------------------
+# log p(y_i | θ) of every observation under every draw, and PSIS-LOO / WAIC, on the device (demcmc_eval_pointwise /
+# demcmc_loo, include/demcmc_b200.h).  Both leave the priors out and need no run: the handle is bound to the likelihood
+# alone.  `f(h, theta, n, n_obs)` runs on that handle with the draws of `chains` as theta[d][n], chain by chain.
+function _with_likelihood(f, model::DEModel{<:GPULoglike}, chains; device = 0)
+    v = Array(chains.value)                                  # Ns × (d + 2) × n_chains; acceptance and lp last
+    d = size(v, 2) - 2
+    theta = reshape(permutedims(v[:, 1:d, :], (2, 1, 3)), d, :)
+    ll = model.loglike
+    n_dim, n_per, n_obs, n_cols = model_geometry(ll, d)
+    x, choice, covm, src = ll.data.x, ll.data.choice, ll.cov, ll.source
+    sig = ll.sigma === nothing ? Float64[] : ll.sigma
+    lo, hi = fill(-Inf, d), fill(Inf, d)
+    priors = [CPrior(Int32(GPU_PRIORS.flat), Int32(0), 0.0, 0.0) for _ in 1:d]
+    h = Ref{Ptr{Cvoid}}(C_NULL)
+    GC.@preserve theta x choice sig covm src lo hi priors begin
+        cfg = CConfig(DEMCMC_ABI_VERSION, 1, 3, d, 0, 0, 0.0, 0.0, 0.001, 0.05, 1.0, 0.0, Int32(0), 0, C_NULL, pointer(lo), pointer(hi),
+            UInt64(0), device, 0, 0, 0, 0, 1, 0, 0, 0, C_NULL)
+        demcmc_check(ccall((:demcmc_create, LIBDEMCMC), Cint, (Ref{CConfig}, Ref{Ptr{Cvoid}}), cfg, h))
+        try
+            m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), choice === nothing ? C_NULL : pointer(choice),
+                isempty(sig) ? C_NULL : pointer(sig), ll.lba_floor, pointer(priors), 0, n_cols, isempty(covm) ? C_NULL : pointer(covm), C_NULL,
+                isempty(src) ? C_NULL : pointer(src))
+            demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
+            return f(h[], theta, size(theta, 2), n_obs), size(v, 1), size(v, 3)
+        finally
+            ccall((:demcmc_destroy, LIBDEMCMC), Cint, (Ptr{Cvoid},), h[])
+        end
+    end
+end
+
+# n_obs × n_steps × n_chains, the [data, step, chain] array ParetoSmooth.psis_loo takes:
+#   psis_loo(pointwise_loglikelihoods(model, chains))
+function pointwise_loglikelihoods(model::DEModel{<:GPULoglike}, chains; device = 0)
+    out, Ns, nc = _with_likelihood(model, chains; device) do h, theta, n, n_obs
+        ll = zeros(Float64, n_obs, n)                         # Julia n_obs × n == C out[n][n_obs]
+        GC.@preserve ll demcmc_check(ccall((:demcmc_eval_pointwise, LIBDEMCMC), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}), h, theta, n, 0, n_obs, ll))
+        ll
+    end
+    return reshape(out, :, Ns, nc)
+end
+
+# PSIS-LOO and WAIC with Pareto smoothing on the device (at most DEMCMC_LOO_MAX_DRAWS = 16384 draws: thin longer chains)
+function loo(model::DEModel{<:GPULoglike}, chains; device = 0)
+    (elpd_i, k, lppd_i, pw_i), _, _ = _with_likelihood(model, chains; device) do h, theta, n, n_obs
+        o = ntuple(_ -> zeros(Float64, n_obs), 4)
+        GC.@preserve o demcmc_check(ccall((:demcmc_loo, LIBDEMCMC), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}), h, theta, n, o[1], o[2], o[3], o[4]))
+        o
+    end
+    N = length(elpd_i)
+    waic_i = lppd_i .- pw_i
+    se(a) = sqrt(N * sum(abs2, a .- sum(a) / N) / N)
+    return (elpd_loo = sum(elpd_i), se_elpd_loo = se(elpd_i), p_loo = sum(lppd_i) - sum(elpd_i), elpd_waic = sum(waic_i),
+            se_elpd_waic = se(waic_i), p_waic = sum(pw_i), n_bad_k = count(>(0.7), k), elpd_loo_i = elpd_i, pareto_k = k,
+            lppd_i = lppd_i, p_waic_i = pw_i)
+end
