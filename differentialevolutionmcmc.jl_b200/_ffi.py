@@ -13,7 +13,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(_HERE, "libdemcmc_b200.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int32)
@@ -34,7 +34,8 @@ class Model(C.Structure):
     _fields_ = [("kind", C.c_int32), ("d", C.c_int32), ("n_obs", C.c_int64), ("n_dim", C.c_int32),
                 ("n_per", C.c_int32), ("x", C.c_void_p), ("choice", C.c_void_p), ("sigma", _dp),
                 ("lba_floor", C.c_double), ("prior", C.POINTER(Prior)), ("data_on_device", C.c_int32),
-                ("n_cols", C.c_int32), ("cov", _dp), ("center", _dp), ("source", C.c_char_p)]
+                ("n_cols", C.c_int32), ("cov", _dp), ("center", _dp), ("source", C.c_char_p), ("n_sim", C.c_int32),
+                ("sim_floor", C.c_double)]
 
 
 class Config(C.Structure):
@@ -65,9 +66,9 @@ class Counters(C.Structure):
 # every symbol include/demcmc_b200.h declares (tests check the library exports all of them)
 SYMBOLS = [
     "demcmc_last_error", "demcmc_abi_version", "demcmc_device_count", "demcmc_backend_name", "demcmc_create",
-    "demcmc_destroy", "demcmc_set_model", "demcmc_compile_loglike", "demcmc_set_history", "demcmc_set_state", "demcmc_run", "demcmc_replay", "demcmc_get_samples",
+    "demcmc_destroy", "demcmc_set_model", "demcmc_compile_loglike", "demcmc_compile_simulator", "demcmc_set_history", "demcmc_set_state", "demcmc_run", "demcmc_replay", "demcmc_get_samples",
     "demcmc_get_accept", "demcmc_get_lp", "demcmc_get_chains", "demcmc_get_moments", "demcmc_set_iteration", "demcmc_set_weights", "demcmc_set_blocking_schedule", "demcmc_get_history_by_slot", "demcmc_get_state", "demcmc_get_trace",
-    "demcmc_get_trace_xdot", "demcmc_eval_xdot", "demcmc_set_sufficient_stat", "demcmc_get_diagnostics",
+    "demcmc_get_trace_xdot", "demcmc_eval_xdot", "demcmc_eval_simulated", "demcmc_set_sufficient_stat", "demcmc_get_diagnostics",
     "demcmc_get_migration", "demcmc_get_counters", "demcmc_set_timing", "demcmc_set_max_chunk", "demcmc_set_lanes", "demcmc_eval", "demcmc_eval_pointwise", "demcmc_loo", "demcmc_op_project", "demcmc_op_reset",
     "demcmc_op_de_proposal", "demcmc_op_snooker", "demcmc_op_accept", "demcmc_op_select", "demcmc_comm_unique_id",
     "demcmc_comm_init", "demcmc_fp64_peak", "demcmc_fp64_peaks", "demcmc_copy_peak",
@@ -88,6 +89,7 @@ def _declare(L):
     L.demcmc_destroy.argtypes = [C.c_void_p]
     L.demcmc_set_model.argtypes = [C.c_void_p, C.POINTER(Model)]
     L.demcmc_compile_loglike.argtypes = [C.c_char_p, C.c_char_p, C.c_int64]
+    L.demcmc_compile_simulator.argtypes = [C.c_char_p, C.c_char_p, C.c_int64]
     L.demcmc_set_history.argtypes = [C.c_void_p, _dp]
     L.demcmc_set_state.argtypes = [C.c_void_p, _dp, _ip]
     L.demcmc_run.argtypes = [C.c_void_p, C.c_int64]
@@ -106,6 +108,7 @@ def _declare(L):
     L.demcmc_get_diagnostics.argtypes = [C.c_void_p, C.c_int64, C.c_int64, _dp, _dp]
     L.demcmc_get_trace_xdot.argtypes = [C.c_void_p, _dp]
     L.demcmc_eval_xdot.argtypes = [C.c_void_p, _dp, C.c_int64, _dp]
+    L.demcmc_eval_simulated.argtypes = [C.c_void_p, _dp, C.c_int64, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), _dp, _dp]
     L.demcmc_set_sufficient_stat.argtypes = [C.c_void_p, C.c_int32]
     L.demcmc_get_migration.argtypes = [C.c_void_p, _ip]
     L.demcmc_get_counters.argtypes = [C.c_void_p, C.POINTER(Counters)]

@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from .handle import Handle, compile_loglike
+from .handle import Handle, compile_loglike, compile_simulator
 
 
 # ---- registered priors (replace prior_loglike closures) -----------------------------------------
@@ -95,12 +95,17 @@ class GPULoglike:
     GPULoglike("custom", X, source=src)          sum_i demcmc_obs(par, X[i]) + demcmc_particle(θ): a likelihood written as
                                                  CUDA C++ (include/demcmc_b200.h: DEMCMC_CUSTOM), compiled here for
                                                  sm_100a; X is a vector, an n_obs × n_cols matrix, or None (no data)
+    GPULoglike("simulated", X, source=src, n_sim=M, floor=1e-10)
+                                                 a likelihood estimated from M simulations per proposal of the CUDA C++
+                                                 simulator demcmc_simulate (include/demcmc_b200.h: DEMCMC_SIMULATED): a
+                                                 Gaussian kernel density per label; X is a vector of values or an n_obs × 2
+                                                 matrix of (label 1..8, value) rows
     (Examples/Guassian_Example_Vector.jl is the "gaussian" kernel: its loglike(data, θ...) destructures μ, σ)
     """
-    KINDS = ("gaussian", "mvnormal", "binomial", "lnr", "lba", "hier_normal", "rastrigin", "mvnormal_full", "custom")
+    KINDS = ("gaussian", "mvnormal", "binomial", "lnr", "lba", "hier_normal", "rastrigin", "mvnormal_full", "custom", "simulated")
 
     def __init__(self, kind, x=None, *, choice=None, rt=None, N=None, k=None, sigma=None, lba_floor=1e-10, cov=None,
-                 source=None):
+                 source=None, n_sim=None, floor=1e-10):
         kind = str(kind).lstrip(":")
         if kind not in self.KINDS:
             raise ValueError(f"no registered kernel for {kind!r}; registered: {self.KINDS}")
@@ -110,7 +115,31 @@ class GPULoglike:
         self.lba_floor = lba_floor
         self.cov = None if cov is None else np.ascontiguousarray(cov, dtype=np.float64)   # mvnormal_full: the known covariance
         self.source = None
-        if kind == "custom":
+        self.n_sim, self.sim_floor = 0, 1e-10
+        if kind == "simulated":
+            if not isinstance(source, (str, bytes)) or not source:
+                raise ValueError("simulated needs source=: CUDA C++ text that defines demcmc_simulate (include/demcmc_b200.h)")
+            if x is None:
+                raise ValueError("simulated needs data: a vector of values or an n_obs x 2 matrix of (label, value) rows")
+            self.x = np.ascontiguousarray(x, dtype=np.float64)
+            if self.x.ndim not in (1, 2) or (self.x.ndim == 2 and self.x.shape[1] not in (1, 2)):
+                raise ValueError("simulated data must be a vector (n_cols = 1) or an n_obs x 2 matrix of (label, value) rows (n_cols = 2)")
+            if self.x.shape[0] < 1:
+                raise ValueError("simulated data need at least one observation")
+            vals = self.x if self.x.ndim == 1 else self.x[:, -1]
+            if not np.all(np.isfinite(vals)):
+                raise ValueError("simulated data values must be finite")
+            if self.x.ndim == 2 and self.x.shape[1] == 2:
+                lab = self.x[:, 0]
+                if not np.all((lab == np.floor(lab)) & (lab >= 1) & (lab <= 8)):
+                    raise ValueError("simulated data labels must be integers in 1..8")
+            if n_sim is None or not 16 <= int(n_sim) <= 16384:
+                raise ValueError(f"simulated needs n_sim in [16, 16384] simulations per proposal, got {n_sim}")
+            if not float(floor) > 0.0:
+                raise ValueError(f"simulated needs floor > 0, got {floor}")
+            compile_simulator(source)        # a source that does not compile fails here, with the compiler log
+            self.source, self.n_sim, self.sim_floor = source, int(n_sim), float(floor)
+        elif kind == "custom":
             if not isinstance(source, (str, bytes)) or not source:
                 raise ValueError("custom needs source=: CUDA C++ text that defines demcmc_obs (include/demcmc_b200.h)")
             self.x = None if x is None else np.ascontiguousarray(x, dtype=np.float64)
@@ -470,7 +499,8 @@ def build_handle(model: DEModel, de: DE, device=0, trace=False, group_begin=0, g
     table = _prior_table(model, shapes, needed=de.evaluate_fitness is not evaluate_fun)
 
     def bind():
-        h.set_model(ll.kind, table, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov, source=ll.source)
+        h.set_model(ll.kind, table, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov, source=ll.source,
+                    n_sim=ll.n_sim, sim_floor=ll.sim_floor)
     if background_model:
         return h, shapes, d, _Background(bind)
     bind()
@@ -533,7 +563,7 @@ def _comparison_handle(model: DEModel, d, device=0, devices=None):
     h = Handle(n_dev, 3, d, [-np.inf] * d, [np.inf] * d, device=device, devices=devices)
     try:
         h.set_model(ll.kind, [("flat",)] * d, x=ll.x, choice=ll.choice, sigma=ll.sigma, lba_floor=ll.lba_floor, cov=ll.cov,
-                    source=ll.source)
+                    source=ll.source, n_sim=ll.n_sim, sim_floor=ll.sim_floor)
     except BaseException:
         h.close()
         raise

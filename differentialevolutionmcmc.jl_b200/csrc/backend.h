@@ -89,6 +89,15 @@ int launch_accept(const ConfigDev &cfg, const ModelDev &m, const Level &lv);
 int custom_compile(const char *source) __attribute__((weak));
 int custom_load(const char *source, void **module, int *has_obs /* the source defines demcmc_obs */) __attribute__((weak));
 void custom_unload(void *module) __attribute__((weak));
+// simulation-based likelihoods (M_SIMULATED): sim_compile / sim_load are custom_compile / custom_load for a DEMCMC_SIMULATED
+// source (its own kernel text k_ll_sim / k_ll_sim_obs; cached apart from a custom source of the same text); the module is
+// freed with custom_unload.  launch_loglik and launch_pointwise run it for ModelDev.custom = *module, with the keys of
+// include/demcmc_b200.h: DEMCMC_SIMULATED.  launch_eval_sim is launch_eval (ll, prior) with the explicit keys (sweep[n],
+// unit[n]) (device) and, when sims is not nullptr, the simulations sims[n][n_sim][n_cols] (device).  Weak, like custom_*.
+int sim_compile(const char *source) __attribute__((weak));
+int sim_load(const char *source, void **module) __attribute__((weak));
+int launch_eval_sim(const ConfigDev &cfg, const ModelDev &m, const double *theta, int64_t n, const uint32_t *sweep, const uint32_t *unit,
+                    double *ll, double *prior, double *sims, double *scratch_part) __attribute__((weak));
 // small pointwise problems: propose + likelihood + accept of a level in one launch, one warp per
 // particle; returns 1 when the model / size does not qualify (launch the three kernels instead)
 int launch_level_fused(const ConfigDev &cfg, const ModelDev &m, const Level &lv);

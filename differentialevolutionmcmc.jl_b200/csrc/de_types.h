@@ -15,9 +15,13 @@ constexpr int PW_TP = 8;          // particles per tile of the pointwise kernels
 constexpr int PW_THREADS = 256;
 
 enum ModelKind { M_GAUSSIAN = 0, M_MVNORMAL = 1, M_BINOMIAL = 2, M_LNR = 3, M_LBA = 4, M_HIER = 5, M_RASTRIGIN = 6, M_MVN_FULL = 7,
-                 M_CUSTOM = 8 /* user-written per-observation density compiled at run time (kernels.cu: k_ll_custom) */ };
+                 M_CUSTOM = 8 /* user-written per-observation density compiled at run time (kernels.cu: k_ll_custom) */,
+                 M_SIMULATED = 9 /* kernel density of user-written simulations compiled at run time (kernels.cu: k_ll_sim) */ };
 constexpr int CUSTOM_MAX_PAR = 256;   // d and DEMCMC_NPAR of a custom model (the per-particle values staged in shared memory)
 constexpr int PSIS_MAX_DRAWS = 16384; // draws of one demcmc_loo call: k_psis holds an observation's values in 128 KB of shared memory
+constexpr int SIM_MAX_DRAWS = 16384;  // simulations per proposal: k_ll_sim sorts them in 144 KB of shared memory
+constexpr int SIM_MAX_LABELS = 8;     // labels of n_cols = 2 data (= MAX_ACC)
+constexpr uint32_t SIM_SWEEP_EVAL = 0xFFFFFFFFu;   // the sweep of the simulation keys outside a run
 constexpr int PSIS_MAX_TAIL = 512;    // >= the tail length ceil(3 sqrt(PSIS_MAX_DRAWS)) = 384, a power of two (bitonic sort)
 // the likelihoods that are a sum of squared deviations from per-dimension means (the streamed DMMA kernels k_xdot / k_chunk_persist)
 DE_HD bool is_ssd(int kind) { return kind == M_MVNORMAL || kind == M_HIER || kind == M_MVN_FULL; }
@@ -68,7 +72,11 @@ struct ModelDev {
     int32_t n_osplit, n_ksplit, split_len, ksplit_len;
     uint32_t ksplit_magic;    // ceil(2^32 / ksplit_len): k / ksplit_len = umulhi(k, magic) for every dimension index k < 2^32 / ksplit_len
     int32_t n_cols;           // M_CUSTOM: values per observation, x[n_obs][n_cols]
-    void *custom;             // M_CUSTOM: the module loaded on this device (be::custom_load), host-side handle
+    void *custom;             // M_CUSTOM / M_SIMULATED: the module loaded on this device (be::custom_load / sim_load), host-side handle
+    int32_t n_sim;            // M_SIMULATED: simulations per proposal
+    int32_t n_lab;            // M_SIMULATED: labels K (n_cols = 2: the largest label of the data; n_cols = 1: 1)
+    double sim_floor;         // M_SIMULATED: density floor
+    uint64_t sim_seed;        // M_SIMULATED: the handle's seed, the Philox key of the simulations (launch_pointwise has no ConfigDev)
 };
 
 // Packed layout of the centred data for k_xdot: element (observation i, dimension k) lives in the

@@ -8,6 +8,7 @@
 #include <string.h>
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <condition_variable>
 #include <functional>
 #include <mutex>
@@ -615,6 +616,16 @@ int demcmc_destroy(demcmc_handle *h)
 
 static_assert(CUSTOM_MAX_PAR == DEMCMC_CUSTOM_MAX_PAR, "k_ll_custom stages DEMCMC_CUSTOM_MAX_PAR values per particle");
 static const char NO_CUSTOM[] = "custom likelihoods need the CUDA backend (this backend has no run-time compiler)";
+static const char NO_SIM[] = "simulated likelihoods need the CUDA backend (this backend has no run-time compiler)";
+static_assert(SIM_MAX_DRAWS == DEMCMC_SIM_MAX_DRAWS && SIM_MAX_LABELS == DEMCMC_SIM_MAX_LABELS && SIM_MAX_LABELS == MAX_ACC &&
+              SIM_SWEEP_EVAL == DEMCMC_SIM_SWEEP_EVAL, "k_ll_sim's limits are the header's");
+// observations per split of a simulated model.  Every CTA of a proposal regenerates and sorts all M simulations before it
+// scores its split, so a split must be long enough that this repetition is a small share of its split_len * M kernel terms:
+// the setup is about log2(M)^2 / 4 compare-exchanges of the bitonic sort plus one simulation per j, by estimate (not
+// measured separately) a few dozen kernel terms' worth per simulation, which 1024 observations make a few per cent of the
+// split's work (a label's observations meet only that label's share of the M).  Below 1024 observations there is
+// one split, one CTA per proposal of the level.  The splits are the y dimension of k_ll_sim's grid, hence at most 65535.
+constexpr int64_t SIM_SPLIT = 1024;
 
 int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
 {
@@ -660,6 +671,19 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         if (m->d < 1 || m->d > DEMCMC_CUSTOM_MAX_PAR) return fail(DEMCMC_EUNSUPPORTED, "a custom likelihood takes 1..%d parameters, got d = %d", DEMCMC_CUSTOM_MAX_PAR, m->d);
         if (!m->source) return fail(DEMCMC_EINVAL, "a custom likelihood needs model.source");
         if (m->n_obs > 0 && m->n_cols < 1) return fail(DEMCMC_EINVAL, "a custom likelihood with observations needs n_cols >= 1, got %d", m->n_cols);
+        want_d = m->d;
+        break;
+    case DEMCMC_SIMULATED:
+        if (!be::sim_load || !be::launch_eval_sim) return fail(DEMCMC_EUNSUPPORTED, "%s", NO_SIM);
+        if (m->d < 1 || m->d > DEMCMC_CUSTOM_MAX_PAR) return fail(DEMCMC_EUNSUPPORTED, "a simulated likelihood takes 1..%d parameters, got d = %d", DEMCMC_CUSTOM_MAX_PAR, m->d);
+        if (!m->source) return fail(DEMCMC_EINVAL, "a simulated likelihood needs model.source (a demcmc_simulate)");
+        if (m->n_cols != 1 && m->n_cols != 2) return fail(DEMCMC_EINVAL, "a simulated likelihood takes n_cols = 1 (a value) or 2 (label, value), got %d", m->n_cols);
+        if (m->n_obs < 1) return fail(DEMCMC_EINVAL, "a simulated likelihood needs at least one observation");
+        if (m->n_obs > SIM_SPLIT * 65535)
+            return fail(DEMCMC_EUNSUPPORTED, "a simulated likelihood takes at most %lld observations, got %lld", (long long)(SIM_SPLIT * 65535), (long long)m->n_obs);
+        if (m->n_sim < 16 || m->n_sim > DEMCMC_SIM_MAX_DRAWS) return fail(DEMCMC_EINVAL, "n_sim must be in [16, %d], got %d", DEMCMC_SIM_MAX_DRAWS, m->n_sim);
+        if (!(m->sim_floor > 0.0)) return fail(DEMCMC_EINVAL, "sim_floor must be > 0, got %g", m->sim_floor);
+        if (m->data_on_device) return fail(DEMCMC_EINVAL, "a simulated likelihood checks its data on the host: pass host data, not device pointers");
         want_d = m->d;
         break;
     default: return fail(DEMCMC_EUNSUPPORTED, "no registered kernel for model kind %d: arbitrary closures are not supported and there is no CPU fallback", m->kind);
@@ -780,7 +804,19 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         // the pointwise kinds, and DEMCMC_CUSTOM: x[n_obs][n_cols], through the same observation splits (k_ll_custom).
         // A custom model never qualifies for the fused / small-chunk / persistent kernels (their densities are the
         // registered ones): every level runs propose -> k_ll_custom -> accept
-        const int64_t n_val = m->n_obs * (m->kind == DEMCMC_CUSTOM ? (int64_t)m->n_cols : 1);
+        const int64_t n_val = m->n_obs * (m->kind == DEMCMC_CUSTOM || m->kind == DEMCMC_SIMULATED ? (int64_t)m->n_cols : 1);
+        if (m->kind == DEMCMC_SIMULATED) {                     // DEMCMC_SIMULATED: labels integers in 1..8, values finite
+            D.n_lab = 1;
+            for (int64_t i = 0; i < m->n_obs; ++i) {
+                const double *xi = m->x + (size_t)i * m->n_cols;
+                if (!std::isfinite(xi[m->n_cols - 1])) return fail(DEMCMC_EINVAL, "observation %lld: the value %g is not finite", (long long)i, xi[m->n_cols - 1]);
+                if (m->n_cols == 2) {
+                    if (!(xi[0] >= 1.0 && xi[0] <= DEMCMC_SIM_MAX_LABELS && xi[0] == floor(xi[0])))
+                        return fail(DEMCMC_EINVAL, "observation %lld: the label %g is not an integer in 1..%d", (long long)i, xi[0], DEMCMC_SIM_MAX_LABELS);
+                    D.n_lab = std::max(D.n_lab, (int32_t)xi[0]);
+                }
+            }
+        }
         D.x = (const double *)upload(m->x, sizeof(double) * n_val, dev);
         if (!D.x) return fail(DEMCMC_ENOMEM, "data upload failed");
         if (m->kind == DEMCMC_CUSTOM) {
@@ -795,6 +831,14 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
                             "__device__ double demcmc_obs(const double *par, const double *x)", (long long)m->n_obs);
             D.custom = h->custom_mod;
         }
+        if (m->kind == DEMCMC_SIMULATED) {
+            D.n_cols = m->n_cols; D.n_sim = m->n_sim; D.sim_floor = m->sim_floor; D.sim_seed = h->cfg.seed;
+            if (int rc = be::sim_load(m->source, &h->custom_mod)) {
+                g_err = be::last_error();
+                return rc == -1 ? DEMCMC_EINVAL : rc == -2 ? DEMCMC_EUNSUPPORTED : DEMCMC_ECUDA;
+            }
+            D.custom = h->custom_mod;
+        }
         if (m->choice) { D.choice = (const int32_t *)upload(m->choice, sizeof(int32_t) * m->n_obs, dev); if (!D.choice) return fail(DEMCMC_ENOMEM, "data upload failed"); }
         if (m->sigma) { D.has_sigma = 1; for (int r = 0; r < m->n_dim && r < MAX_ACC; ++r) D.sigma_acc[r] = m->sigma[r]; }
         const int64_t chunk = PW_THREADS;
@@ -802,6 +846,10 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         const int64_t per = std::max<int64_t>(1, (chunks + 147) / 148);
         D.split_len = (int32_t)(per * chunk);
         D.n_osplit = (int32_t)std::max<int64_t>(1, (m->n_obs + D.split_len - 1) / D.split_len);
+        if (m->kind == DEMCMC_SIMULATED) {                     // balanced splits of at most SIM_SPLIT observations
+            D.n_osplit = (int32_t)((m->n_obs + SIM_SPLIT - 1) / SIM_SPLIT);
+            D.split_len = (int32_t)((m->n_obs + D.n_osplit - 1) / D.n_osplit);
+        }
     }
     const size_t n_split = (size_t)D.n_osplit * D.n_ksplit;
     h->ll_part = (double *)be::dmalloc(sizeof(double) * std::max<size_t>(1, (size_t)h->P * n_split));
@@ -817,6 +865,18 @@ int demcmc_compile_loglike(const char *source, char *log, int64_t log_cap)
     if (!source) return fail(DEMCMC_EINVAL, "null source");
     if (!be::custom_compile) return fail(DEMCMC_EUNSUPPORTED, "%s", NO_CUSTOM);
     const int rc = be::custom_compile(source);
+    if (rc == 0) return 0;
+    g_err = be::last_error();                                // the whole compiler log (fail() would cut it)
+    if (log && log_cap > 0) { const size_t n = std::min(g_err.size(), (size_t)log_cap - 1); memcpy(log, g_err.data(), n); log[n] = 0; }
+    return rc == -2 ? DEMCMC_EUNSUPPORTED : DEMCMC_EINVAL;
+}
+
+int demcmc_compile_simulator(const char *source, char *log, int64_t log_cap)
+{
+    if (log && log_cap > 0) log[0] = 0;
+    if (!source) return fail(DEMCMC_EINVAL, "null source");
+    if (!be::sim_compile) return fail(DEMCMC_EUNSUPPORTED, "%s", NO_SIM);
+    const int rc = be::sim_compile(source);
     if (rc == 0) return 0;
     g_err = be::last_error();                                // the whole compiler log (fail() would cut it)
     if (log && log_cap > 0) { const size_t n = std::min(g_err.size(), (size_t)log_cap - 1); memcpy(log, g_err.data(), n); log[n] = 0; }
@@ -1751,6 +1811,37 @@ int demcmc_eval_xdot(demcmc_handle *h, const double *theta, int64_t n, double *x
     if (h && h->has_model && !is_ssd(h->dmodel.kind)) return fail(DEMCMC_EINVAL, "only MVNORMAL / HIER_NORMAL have a cross term");
     return eval_impl(h, theta, n, nullptr, nullptr, xdot);
 }
+// a simulated model under explicit keys (demcmc_eval: the eval sweep and the vector's index)
+static int eval_sim_impl(demcmc_handle *h, const double *theta, int64_t n, const uint32_t *sweep, const uint32_t *unit, double *loglike,
+                         double *prior, double *sims)
+{
+    BE(be::set_device(h->cfg.device));
+    if (n == 0) return 0;
+    const ModelDev &M = h->dmodel;
+    DevBuf buf;
+    double *dt = buf.up(theta, (size_t)n * h->d), *dl = buf.up<double>(nullptr, (size_t)n), *dp = buf.up<double>(nullptr, (size_t)n);
+    double *part = buf.up<double>(nullptr, (size_t)n * M.n_osplit);
+    uint32_t *ds = buf.up(sweep, (size_t)n), *du = buf.up(unit, (size_t)n);
+    const size_t n_sims = (size_t)n * M.n_sim * M.n_cols;
+    double *dsim = sims ? buf.up<double>(nullptr, n_sims) : nullptr;
+    if (!dt || !dl || !dp || !part || !ds || !du || (sims && !dsim)) return fail(DEMCMC_ENOMEM, "eval staging does not fit: %s", be::last_error());
+    if (be::sync() || be::launch_eval_sim(h->dcfg, M, dt, n, ds, du, dl, dp, dsim, part) ||
+        (loglike && be::d2h(loglike, dl, sizeof(double) * n)) || (prior && be::d2h(prior, dp, sizeof(double) * n)) ||
+        (sims && be::d2h(sims, dsim, sizeof(double) * n_sims)))
+        return fail(DEMCMC_ECUDA, "eval: %s", be::last_error());
+    return 0;
+}
+
+int demcmc_eval_simulated(demcmc_handle *h, const double *theta, int64_t n, const uint32_t *sweep, const uint32_t *unit, double *loglike,
+                          double *sims)
+{
+    if (!h || !theta || n < 0 || (n > 0 && (!sweep || !unit))) return fail(DEMCMC_EINVAL, "bad argument");
+    if (!h->has_model) return fail(DEMCMC_ESTATE, "set_model first");
+    if (h->dmodel.kind != M_SIMULATED) return fail(DEMCMC_EINVAL, "demcmc_eval_simulated needs a DEMCMC_SIMULATED model");
+    if (h->multi) return demcmc_eval_simulated(h->kids[0], theta, n, sweep, unit, loglike, sims);
+    return eval_sim_impl(h, theta, n, sweep, unit, loglike, nullptr, sims);
+}
+
 static int eval_impl(demcmc_handle *h, const double *theta, int64_t n, double *loglike, double *prior, double *xdot)
 {
     if (!h || !theta || n < 0) return fail(DEMCMC_EINVAL, "bad argument");
@@ -1758,6 +1849,11 @@ static int eval_impl(demcmc_handle *h, const double *theta, int64_t n, double *l
     if (h->multi) return eval_impl(h->kids[0], theta, n, loglike, prior, xdot);
     BE(be::set_device(h->cfg.device));
     if (n == 0) return 0;
+    if (h->dmodel.kind == M_SIMULATED) {
+        std::vector<uint32_t> sweep((size_t)n, SIM_SWEEP_EVAL), unit((size_t)n);
+        for (int64_t i = 0; i < n; ++i) unit[(size_t)i] = (uint32_t)i;
+        return eval_sim_impl(h, theta, n, sweep.data(), unit.data(), loglike, prior, nullptr);
+    }
     const size_t d = h->d, ns = (size_t)h->dmodel.n_osplit * h->dmodel.n_ksplit;
     double *dt = (double *)be::dmalloc(sizeof(double) * n * d), *dl = (double *)be::dmalloc(sizeof(double) * n),
            *dp = (double *)be::dmalloc(sizeof(double) * n), *part = (double *)be::dmalloc(sizeof(double) * n * ns),

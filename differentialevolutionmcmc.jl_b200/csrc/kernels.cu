@@ -13,6 +13,7 @@
 //   k_mig_*        migration picks and the cyclic shift
 //   k_history      by-slot rows -> the reference's samples[n_rows, d, P] layout
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <dlfcn.h>
 #include <nvrtc.h>
 #include <stdio.h>
@@ -2217,6 +2218,302 @@ extern "C" __global__ void __launch_bounds__(256) k_ll_custom_obs(const double *
 }
 )CU";
 
+// ------------------------------------------------------------------------------------------------
+// simulation-based likelihoods (M_SIMULATED): the caller's simulator (include/demcmc_b200.h: DEMCMC_SIMULATED) is compiled
+// at run time into two kernels around it, k_ll_sim (a level's proposals, writing the ll_part slots k_ll_custom writes, so
+// accept, k_eval_finish and finalize_ll are unchanged) and k_ll_sim_obs (out[obs][draw] for launch_pointwise).  A CTA takes
+// one parameter vector and one range of observations: it regenerates that vector's M simulations from their counter-based
+// streams into shared memory (no global staging, no inter-CTA sync), sorts them by (label, value) with k_psis's
+// order-preserving keys and bitonic network (spelled out again here: the run-time module cannot link the library's device
+// code), takes each label's moments and quartiles, and streams its observations against their own label's group, one
+// observation per warp.  Both kernels call the same two functions with the same 256 threads, so an observation's value is
+// the same bits in either.  Plain launches (no programmatic dependent launch), like k_ll_custom.  The README's LBA
+// simulator (DEMCMC_NPAR 5) compiled by libnvrtc 12.9 with this file's options plus --ptxas-options=-v: both kernels 64
+// registers, no spills, 320 bytes of static shared memory (2336 without DEMCMC_NPAR: par[] is then 256 doubles); k_ll_sim
+// has a 16-byte stack frame (y[2], passed to demcmc_simulate).  Dynamic shared memory: 9 bytes per simulation, padded to a
+// power of two (144 KB at M = 16384).  The inner loop of demcmc_sim_obs_ issues 24 fp64 instructions per term (16 DFMA,
+// 4 DMUL, 3 DADD, 1 DSETP; unrolled by 8 in the SASS).
+// ------------------------------------------------------------------------------------------------
+static_assert(offsetof(SweepCtx, sweep) == 0, "k_ll_sim reads a level's sweep as the first word of its SweepCtx");
+static_assert(SIM_MAX_LABELS == 8 && SIM_SWEEP_EVAL == 0xFFFFFFFFu, "k_ll_sim's source spells these out");
+
+// dynamic shared memory of k_ll_sim / k_ll_sim_obs: a key and a label per simulation, padded to a power of two (>= 16)
+static size_t sim_smem(int M) { int p = 16; while (p < M) p <<= 1; return (size_t)p * (sizeof(unsigned long long) + 1); }
+
+// ahead of the user's text: the random streams, and a stand-in demcmc_simulate whose return type tells the kernel source
+// that the user wrote none (a definition in the source matches the argument types exactly, the stand-in needs conversions)
+static const char SIM_PRELUDE[] = R"CU(
+#define DEMCMC_INF __longlong_as_double(0x7ff0000000000000LL)
+#define DEMCMC_NAN __longlong_as_double(0x7ff8000000000000LL)
+struct demcmc_rng { unsigned c, unit, sweep, stream, k0, k1; int has_u, has_z; double u, z; };
+struct demcmc_u4_ { unsigned x, y, z, w; };
+__device__ inline demcmc_u4_ demcmc_philox_(demcmc_u4_ c, unsigned k0, unsigned k1)
+{
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const unsigned hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const unsigned hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        demcmc_u4_ n;
+        n.x = hi1 ^ c.y ^ k0; n.y = lo1; n.z = hi0 ^ c.w ^ k1; n.w = lo0;
+        c = n;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    return c;
+}
+__device__ inline double demcmc_u53_(unsigned lo, unsigned hi)
+{
+    const unsigned long long b = (((unsigned long long)hi << 32) | lo) >> 11;
+    return b ? (double)b * 0x1.0p-53 : 0x1.0p-54;
+}
+__device__ inline double demcmc_uniform(demcmc_rng *r)
+{
+    if (r->has_u) { r->has_u = 0; return r->u; }
+    demcmc_u4_ c; c.x = r->c++; c.y = r->unit; c.z = r->sweep; c.w = r->stream;
+    const demcmc_u4_ o = demcmc_philox_(c, r->k0, r->k1);
+    r->u = demcmc_u53_(o.z, o.w); r->has_u = 1;
+    return demcmc_u53_(o.x, o.y);
+}
+__device__ inline double demcmc_normal(demcmc_rng *r)
+{
+    if (r->has_z) { r->has_z = 0; return r->z; }
+    const double u1 = demcmc_uniform(r), u2 = demcmc_uniform(r);
+    const double rad = sqrt(-2.0 * log(u1));
+    double s, c;
+    sincospi(2.0 * u2, &s, &c);
+    r->z = rad * s; r->has_z = 1;
+    return rad * c;
+}
+struct demcmc_missing_ {};
+struct demcmc_any_cptr_ { __device__ demcmc_any_cptr_(const double *) {} };
+struct demcmc_any_rng_ { __device__ demcmc_any_rng_(demcmc_rng *) {} };
+struct demcmc_any_ptr_ { __device__ demcmc_any_ptr_(double *) {} };
+__device__ inline demcmc_missing_ demcmc_simulate(demcmc_any_cptr_, demcmc_any_rng_, demcmc_any_ptr_) { return demcmc_missing_(); }
+#line 1 "user.cu"
+)CU";
+
+static const char SIM_KERNEL[] = R"CU(
+#line 1 "demcmc_sim_kernel.cu"
+template <class T> struct demcmc_is_void_ { enum { value = 0 }; };
+template <> struct demcmc_is_void_<void> { enum { value = 1 }; };
+static_assert(demcmc_is_void_<decltype(demcmc_simulate((const double *)0, (demcmc_rng *)0, (double *)0))>::value,
+              "the source must define  __device__ void demcmc_simulate(const double *par, demcmc_rng *rng, double *y)");
+#ifdef DEMCMC_NPAR
+static_assert(DEMCMC_NPAR >= 1, "DEMCMC_NPAR must be at least 1");
+static_assert(DEMCMC_NPAR <= 256, "DEMCMC_NPAR is above DEMCMC_CUSTOM_MAX_PAR (256)");
+#define DEMCMC_PAR_LEN_ (DEMCMC_NPAR)
+#else
+#define DEMCMC_PAR_LEN_ 256
+#endif
+
+// exp(x) for x <= 0 (de_math.h: de_exp_nonpos, the LBA kernel's): 2^k Taylor_13(r), |r| <= ln2 / 2; 0 below -708
+__constant__ double demcmc_exp_c_[14] = {
+    1.0, 1.0, 0.5, 1.0 / 6.0, 1.0 / 24.0, 1.0 / 120.0, 1.0 / 720.0, 1.0 / 5040.0, 1.0 / 40320.0, 1.0 / 362880.0, 1.0 / 3628800.0,
+    1.0 / 39916800.0, 1.0 / 479001600.0, 1.0 / 6227020800.0
+};
+__device__ __forceinline__ double demcmc_exp_nonpos_(double x)
+{
+    const double kd = __dadd_rn(__fma_rn(x, 1.4426950408889634074, 6755399441055744.0), -6755399441055744.0);
+    double r = __fma_rn(kd, -6.93147180369123816490e-01, x);
+    r = __fma_rn(kd, -1.90821492927058770002e-10, r);
+    double p = demcmc_exp_c_[13];
+#pragma unroll
+    for (int j = 12; j >= 0; --j) p = __fma_rn(p, r, demcmc_exp_c_[j]);
+    const int k = (int)kd;
+    const double scale = __hiloint2double((k + 1023) << 20, 0);
+    return x < -708.0 ? 0.0 : p * scale;
+}
+// order-preserving 64-bit key of a double (kernels.cu: ps_key)
+__device__ __forceinline__ unsigned long long demcmc_key_(double x)
+{
+    const unsigned long long u = (unsigned long long)__double_as_longlong(x);
+    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double demcmc_unkey_(unsigned long long k)
+{
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+// fixed-order CTA sum: the warp's xor tree, then the 8 warps in order; every thread gets the value
+__device__ __forceinline__ double demcmc_cta_sum_(double v, double *red)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double r = red[0];
+#pragma unroll
+    for (int w = 1; w < 8; ++w) r += red[w];
+    __syncthreads();
+    return r;
+}
+// linearly interpolated quantile of sorted v[0..m) (numpy's and Julia's default)
+__device__ __forceinline__ double demcmc_quantile_(const double *v, int m, double p)
+{
+    const double h = (double)(m - 1) * p;
+    const int lo = (int)floor(h);
+    const int hi = lo + 1 < m ? lo + 1 : lo;
+    return v[lo] + (h - (double)lo) * (v[hi] - v[lo]);
+}
+// per label c = 1..8: first index and size of its sorted group, 1/h_c and 1/(sqrt(2 pi) M h_c) (ih = 0: no density)
+struct demcmc_groups_ { int beg[9], m[9]; double ih[9], scale[9]; };
+
+__device__ __forceinline__ int demcmc_pow2_(int M) { int p = 16; while (p < M) p <<= 1; return p; }
+
+// the M simulations of one key into key[] / lab[] (P2 entries, dynamic shared memory), sorted by (label, value); then the
+// values in place of the keys and the groups' bandwidths.  Label 255 = in no group (and the padding up to P2).
+__device__ void demcmc_sim_prepare_(const double *par, unsigned sweep, unsigned unit, unsigned long long seed, int M, int n_cols,
+                                    int K, unsigned long long *key, unsigned char *lab, demcmc_groups_ &g, double *red, double *sims)
+{
+    const int tid = threadIdx.x, P2 = demcmc_pow2_(M);
+    for (int j = tid; j < P2; j += 256) {
+        unsigned char l = 255;
+        unsigned long long k = ~0ull;
+        if (j < M) {
+            demcmc_rng r;
+            r.c = 0; r.unit = unit; r.sweep = sweep; r.stream = 8u + 16u * (unsigned)j;
+            r.k0 = (unsigned)seed; r.k1 = (unsigned)(seed >> 32); r.has_u = 0; r.has_z = 0; r.u = 0.0; r.z = 0.0;
+            double y[2] = { 0.0, 0.0 };
+            demcmc_simulate(par, &r, y);
+            if (sims) for (int c = 0; c < n_cols; ++c) sims[(size_t)j * n_cols + c] = y[c];
+            const double val = n_cols == 2 ? y[1] : y[0];
+            if (isfinite(val)) {
+                if (n_cols == 1) l = 1;
+                else if (y[0] >= 1.0 && y[0] <= (double)K && y[0] == floor(y[0])) l = (unsigned char)y[0];
+            }
+            k = demcmc_key_(val);
+        }
+        key[j] = k; lab[j] = l;
+    }
+    if (tid < 9) g.m[tid] = 0;
+    __syncthreads();
+    for (int size = 2; size <= P2; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = tid; t < P2 / 2; t += 256) {
+                const int a = 2 * t - (t & (stride - 1)), b = a + stride;
+                const bool up = (a & size) == 0;
+                const unsigned char la = lab[a], lb = lab[b];
+                const unsigned long long ka = key[a], kb = key[b];
+                if ((la > lb || (la == lb && ka > kb)) == up) { lab[a] = lb; lab[b] = la; key[a] = kb; key[b] = ka; }
+            }
+            __syncthreads();
+        }
+    double *v = (double *)key;
+    for (int j = tid; j < M; j += 256) {
+        const unsigned char l = lab[j];
+        if (l != 255) { atomicAdd(&g.m[l], 1); v[j] = demcmc_unkey_(key[j]); }
+    }
+    __syncthreads();
+    if (tid == 0) { int b = 0; for (int c = 1; c <= K; ++c) { g.beg[c] = b; b += g.m[c]; } }
+    __syncthreads();
+    for (int c = 1; c <= K; ++c) {
+        const int m = g.m[c], b = g.beg[c];
+        double ih = 0.0, sc = 0.0;
+        if (m >= 2) {
+            double s = 0.0;
+            for (int j = tid; j < m; j += 256) s += v[b + j];
+            const double mean = demcmc_cta_sum_(s, red) / (double)m;
+            double q = 0.0;
+            for (int j = tid; j < m; j += 256) { const double dl = v[b + j] - mean; q += dl * dl; }
+            const double sd = sqrt(demcmc_cta_sum_(q, red) / (double)(m - 1));
+            const double iqr = demcmc_quantile_(v + b, m, 0.75) - demcmc_quantile_(v + b, m, 0.25);
+            const double a = iqr > 0.0 ? fmin(sd, iqr / 1.34) : sd;
+            const double h = 0.9 * a * pow((double)m, -0.2);
+            if (h > 0.0 && isfinite(h)) { ih = 1.0 / h; sc = 0.39894228040143267794 / ((double)M * h); }
+        }
+        if (tid == 0) { g.ih[c] = ih; g.scale[c] = sc; }
+    }
+    __syncthreads();
+}
+
+// log-likelihood of one observation (label c, value t), computed by one whole warp: lane-strided over the group, xor tree
+__device__ __forceinline__ double demcmc_sim_obs_(const double *v, const demcmc_groups_ &g, int c, double t, double floor_)
+{
+    const double ih = g.ih[c];
+    if (!(ih > 0.0)) return log(floor_);
+    const int b = g.beg[c], m = g.m[c];
+    double s = 0.0;
+    for (int j = (int)(threadIdx.x & 31); j < m; j += 32) {
+        const double z = (t - v[b + j]) * ih;
+        s += demcmc_exp_nonpos_(-0.5 * (z * z));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const double f = s * g.scale[c];
+    return log(f > floor_ ? f : floor_);
+}
+
+__device__ __forceinline__ void demcmc_sim_par_(const double *th, int d, double *par)
+{
+#ifdef DEMCMC_NPAR
+    if (threadIdx.x == 0) demcmc_prepare(th, par);
+#else
+    for (int k = threadIdx.x; k < d; k += 256) par[k] = th[k];
+#endif
+    __syncthreads();
+}
+
+// one CTA per (proposal, observation split): part[p][split] = sum of the split's ll_i.  Keys: (key_sweep[p], key_unit[p])
+// when given (the test hook), else (the sweep of the entry's SweepCtx, or the eval sweep without contexts; unit_base + p)
+extern "C" __global__ void __launch_bounds__(256) k_ll_sim(const double *theta, int d, const int *order, const char *ctxs, int ctx_stride,
+                                                           unsigned unit_base, const unsigned *key_sweep, const unsigned *key_unit,
+                                                           const double *x, int n_cols, long long n_obs, int split_len, int n_split,
+                                                           double *part, unsigned long long seed, int M, int K, double floor_, double *sims)
+{
+    extern __shared__ unsigned long long demcmc_keys_[];
+    __shared__ double par[DEMCMC_PAR_LEN_];
+    __shared__ double red[8];
+    __shared__ demcmc_groups_ g;
+    unsigned char *lab = (unsigned char *)(demcmc_keys_ + demcmc_pow2_(M));
+    const int split = blockIdx.y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned e = order ? (unsigned)order[blockIdx.x] : blockIdx.x;
+    const int p = (int)(e & 0xFFFFFFu);
+    unsigned sweep, unit;
+    if (key_sweep) { sweep = key_sweep[p]; unit = key_unit[p]; }
+    else { sweep = ctxs ? *(const unsigned *)(ctxs + (size_t)(e >> 24) * ctx_stride) : 0xFFFFFFFFu; unit = unit_base + (unsigned)p; }
+    demcmc_sim_par_(theta + (size_t)p * d, d, par);
+    demcmc_sim_prepare_(par, sweep, unit, seed, M, n_cols, K, demcmc_keys_, lab, g, red,
+                        (sims && split == 0) ? sims + (size_t)p * M * n_cols : nullptr);
+    const double *v = (const double *)demcmc_keys_;
+    const long long i0 = (long long)split * split_len, i1 = min(n_obs, i0 + (long long)split_len);
+    double acc = 0.0;
+    for (long long i = i0 + warp; i < i1; i += 8) {
+        const double *xi = x + (size_t)i * n_cols;
+        acc += demcmc_sim_obs_(v, g, n_cols == 2 ? (int)xi[0] : 1, xi[n_cols - 1], floor_);
+    }
+    if (lane == 0) red[warp] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) s += red[w];
+        part[(size_t)p * n_split + split] = s;
+    }
+}
+
+// demcmc_eval_pointwise / demcmc_loo: one CTA per (draw s, chunk of observations), key (eval sweep, s);
+// out[o][s] = ll of observation obs0 + o
+extern "C" __global__ void __launch_bounds__(256) k_ll_sim_obs(const double *theta, int d, long long n, const double *x, int n_cols,
+                                                               long long obs0, long long n_obs, int chunk_len, unsigned long long seed,
+                                                               int M, int K, double floor_, double *out)
+{
+    extern __shared__ unsigned long long demcmc_keys_[];
+    __shared__ double par[DEMCMC_PAR_LEN_];
+    __shared__ double red[8];
+    __shared__ demcmc_groups_ g;
+    unsigned char *lab = (unsigned char *)(demcmc_keys_ + demcmc_pow2_(M));
+    const long long s = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    demcmc_sim_par_(theta + (size_t)s * d, d, par);
+    demcmc_sim_prepare_(par, 0xFFFFFFFFu, (unsigned)s, seed, M, n_cols, K, demcmc_keys_, lab, g, red, nullptr);
+    const double *v = (const double *)demcmc_keys_;
+    const long long o0 = (long long)blockIdx.y * chunk_len, o1 = min(n_obs, o0 + (long long)chunk_len);
+    for (long long o = o0 + warp; o < o1; o += 8) {
+        const double *xi = x + (size_t)(obs0 + o) * n_cols;
+        const double ll = demcmc_sim_obs_(v, g, n_cols == 2 ? (int)xi[0] : 1, xi[n_cols - 1], floor_);
+        if (lane == 0) out[(size_t)o * n + s] = ll;
+    }
+}
+)CU";
+
 struct NvrtcApi {
     void *lib = nullptr;
     decltype(&nvrtcCreateProgram) CreateProgram = nullptr;
@@ -2230,7 +2527,7 @@ struct NvrtcApi {
 };
 static NvrtcApi g_nvrtc;
 static std::mutex g_custom_mu;                                   // the NVRTC table and the cubin cache
-static std::map<std::string, std::string> g_custom_cubin;        // source text -> sm_100a cubin
+static std::map<std::pair<int, std::string>, std::string> g_custom_cubin;   // (1 = simulator, source text) -> sm_100a cubin
 
 static int nvrtc_load()                                          // under g_custom_mu
 {
@@ -2247,13 +2544,14 @@ static int nvrtc_load()                                          // under g_cust
     return 0;
 }
 
-// the cubin of `source`, compiled on the first request (under g_custom_mu)
-static int custom_cubin(const char *source, const std::string **cubin)
+// the cubin of a custom (sim = 0) or simulator (sim = 1) `source`, compiled on the first request (under g_custom_mu)
+static int custom_cubin(const char *source, const std::string **cubin, int sim = 0)
 {
-    auto it = g_custom_cubin.find(source);
+    const std::pair<int, std::string> key(sim, source);
+    auto it = g_custom_cubin.find(key);
     if (it != g_custom_cubin.end()) { *cubin = &it->second; return 0; }
     if (int rc = nvrtc_load()) return rc;
-    const std::string text = std::string(CUSTOM_PRELUDE) + source + "\n" + CUSTOM_KERNEL;
+    const std::string text = sim ? std::string(SIM_PRELUDE) + source + "\n" + SIM_KERNEL : std::string(CUSTOM_PRELUDE) + source + "\n" + CUSTOM_KERNEL;
     nvrtcProgram prog = nullptr;
     nvrtcResult r = g_nvrtc.CreateProgram(&prog, text.c_str(), "demcmc_custom.cu", 0, nullptr, nullptr);
     if (r != NVRTC_SUCCESS) { g_be_err = std::string("nvrtcCreateProgram: ") + g_nvrtc.GetErrorString(r); return -1; }
@@ -2265,7 +2563,7 @@ static int custom_cubin(const char *source, const std::string **cubin)
         std::string log;
         if (g_nvrtc.GetProgramLogSize(prog, &n) == NVRTC_SUCCESS && n > 1) { log.resize(n); g_nvrtc.GetProgramLog(prog, &log[0]); log.resize(n - 1); }
         g_nvrtc.DestroyProgram(&prog);
-        g_be_err = "custom likelihood does not compile (" + std::string(g_nvrtc.GetErrorString(r)) + "):\n" + log;
+        g_be_err = std::string(sim ? "simulator" : "custom likelihood") + " does not compile (" + std::string(g_nvrtc.GetErrorString(r)) + "):\n" + log;
         return log.find("DEMCMC_NPAR is above") != std::string::npos ? -2 : -1;
     }
     size_t n = 0;
@@ -2274,7 +2572,7 @@ static int custom_cubin(const char *source, const std::string **cubin)
     if (r == NVRTC_SUCCESS) { bin.resize(n); r = g_nvrtc.GetCUBIN(prog, &bin[0]); }
     g_nvrtc.DestroyProgram(&prog);
     if (r != NVRTC_SUCCESS) { g_be_err = std::string("nvrtcGetCUBIN: ") + g_nvrtc.GetErrorString(r); return -1; }
-    *cubin = &(g_custom_cubin[source] = std::move(bin));
+    *cubin = &(g_custom_cubin[key] = std::move(bin));
     return 0;
 }
 
@@ -2321,6 +2619,59 @@ void custom_unload(void *module)
     delete mod;
 }
 
+int sim_compile(const char *source)
+{
+    std::lock_guard<std::mutex> lk(g_custom_mu);
+    const std::string *cubin = nullptr;
+    return custom_cubin(source, &cubin, 1);
+}
+
+// a simulator module: k_ll_sim as CustomModule.kernel, k_ll_sim_obs as obs_kernel
+int sim_load(const char *source, void **module)
+{
+    *module = nullptr;
+    std::string cubin;
+    {
+        std::lock_guard<std::mutex> lk(g_custom_mu);
+        const std::string *c = nullptr;
+        if (int rc = custom_cubin(source, &c, 1)) return rc;
+        cubin = *c;
+    }
+    CustomModule *mod = new CustomModule();
+    cudaError_t e = cudaLibraryLoadData(&mod->lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+    if (e != cudaSuccess) { delete mod; cu_fail(e, "cudaLibraryLoadData (simulator)"); return -3; }
+    e = cudaLibraryGetKernel(&mod->kernel, mod->lib, "k_ll_sim");
+    if (e == cudaSuccess) e = cudaLibraryGetKernel(&mod->obs_kernel, mod->lib, "k_ll_sim_obs");
+    const size_t smem = sim_smem(SIM_MAX_DRAWS);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)mod->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute((const void *)mod->obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) { cudaLibraryUnload(mod->lib); delete mod; cu_fail(e, "loading k_ll_sim"); return -3; }
+    *module = mod;
+    return 0;
+}
+
+// k_ll_sim over the entries of lv; keys from key_sweep / key_unit (device, [lv.n]) when given
+static int launch_ll_sim(const ConfigDev &cfg, const ModelDev &m, const double *theta, const Level &lv, const uint32_t *key_sweep,
+                         const uint32_t *key_unit, double *ll_part, double *sims)
+{
+    if (!m.custom) { g_be_err = "simulator not loaded"; return -1; }
+    const CustomModule *mod = (const CustomModule *)m.custom;
+    int d = m.d, n_cols = m.n_cols, split_len = m.split_len, n_split = m.n_osplit, M = m.n_sim, K = m.n_lab;
+    int ctx_stride = (int)sizeof(SweepCtx);
+    unsigned unit_base = (unsigned)(cfg.group_begin * cfg.Np);
+    long long n_obs = m.n_obs;
+    unsigned long long seed = m.sim_seed;
+    double floor_ = m.sim_floor;
+    const int *order = lv.order;
+    const char *ctxs = (const char *)lv.ctxs;
+    const double *x = m.x;
+    void *args[] = { &theta, &d, &order, &ctxs, &ctx_stride, &unit_base, &key_sweep, &key_unit, &x, &n_cols, &n_obs, &split_len, &n_split,
+                     &ll_part, &seed, &M, &K, &floor_, &sims };
+    CU(cudaLaunchKernel((const void *)mod->kernel, dim3((unsigned)lv.n, (unsigned)n_split), dim3(256), args, sim_smem(M), stream()));
+    LAUNCHED("k_ll_sim");
+    return 0;
+}
+
 static int launch_ll_custom(const ModelDev &m, const double *theta, const Level &lv, double *ll_part)
 {
     if (!m.custom) { g_be_err = "custom likelihood not loaded"; return -1; }
@@ -2346,6 +2697,7 @@ int launch_loglik(const ConfigDev &cfg, const ModelDev &m, const double *theta, 
         return launch_xdot(m, xs, lv, ll_acc);
     }
     if (m.kind == M_CUSTOM) return launch_ll_custom(m, theta, lv, ll_part);
+    if (m.kind == M_SIMULATED) return launch_ll_sim(cfg, m, theta, lv, nullptr, nullptr, ll_part, nullptr);
     dim3 grid((lv.n + PW_TP - 1) / PW_TP, m.n_osplit);
     if (m.kind == M_GAUSSIAN) k_ll_pointwise<M_GAUSSIAN><<<grid, PW_THREADS, 0, stream()>>>(m, theta, lv, ll_part);
     else if (m.kind == M_LNR) k_ll_pointwise<M_LNR><<<grid, PW_THREADS, 0, stream()>>>(m, theta, lv, ll_part);
@@ -2504,6 +2856,18 @@ int launch_eval(const ConfigDev &cfg, const ModelDev &m, const double *theta, in
     return 0;
 }
 
+int launch_eval_sim(const ConfigDev &cfg, const ModelDev &m, const double *theta, int64_t n, const uint32_t *sweep, const uint32_t *unit,
+                    double *ll, double *prior, double *sims, double *scratch_part)
+{
+    if (n <= 0) return 0;
+    Level lv; lv.order = nullptr; lv.n = (int32_t)n; lv.ctxs = nullptr;
+    if (launch_ll_sim(cfg, m, theta, lv, sweep, unit, scratch_part, sims)) return -1;
+    const int blocks = (int)((n * 32 + PA_THREADS - 1) / PA_THREADS);
+    k_eval_finish<<<blocks, PA_THREADS, 0, stream()>>>(cfg, m, theta, n, scratch_part, nullptr, nullptr, ll, prior, nullptr, nullptr);
+    LAUNCHED("k_eval_finish");
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // model comparison (demcmc_eval_pointwise / demcmc_loo)
 //   k_ll_obs<KIND>  the pointwise matrix out[obs][draw] of a tile of 32 draws (one per lane) x 64 observations (8 per
@@ -2619,11 +2983,29 @@ static int launch_ll_custom_obs(const ModelDev &m, const double *theta, int64_t 
     return 0;
 }
 
+static int launch_ll_sim_obs(const ModelDev &m, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out)
+{
+    if (!m.custom) { g_be_err = "simulator not loaded"; return -1; }
+    const CustomModule *mod = (const CustomModule *)m.custom;
+    int d = m.d, n_cols = m.n_cols, chunk_len = m.split_len, M = m.n_sim, K = m.n_lab;
+    long long nn = n, o0 = obs0, no = n_obs;
+    unsigned long long seed = m.sim_seed;
+    double floor_ = m.sim_floor;
+    const double *x = m.x;
+    const int64_t n_chunks = (n_obs + chunk_len - 1) / chunk_len;
+    if (n_chunks > 65535) { g_be_err = "too many observations for one k_ll_sim_obs launch"; return -1; }
+    void *args[] = { &theta, &d, &nn, &x, &n_cols, &o0, &no, &chunk_len, &seed, &M, &K, &floor_, &out };
+    CU(cudaLaunchKernel((const void *)mod->obs_kernel, dim3((unsigned)n, (unsigned)n_chunks), dim3(256), args, sim_smem(M), stream()));
+    LAUNCHED("k_ll_sim_obs");
+    return 0;
+}
+
 int launch_pointwise(const ModelDev &m, const double *theta, int64_t n, int64_t obs0, int64_t n_obs, double *out)
 {
     if (n <= 0 || n_obs <= 0) return 0;
     if (n > (int64_t)65535 * OB_TD) { g_be_err = "too many draws for one pointwise launch"; return -1; }
     if (m.kind == M_CUSTOM) return launch_ll_custom_obs(m, theta, n, obs0, n_obs, out);
+    if (m.kind == M_SIMULATED) return launch_ll_sim_obs(m, theta, n, obs0, n_obs, out);
     const dim3 grid((unsigned)((n_obs + OB_TO - 1) / OB_TO), (unsigned)((n + OB_TD - 1) / OB_TD));
     double *mt = nullptr, *c0 = nullptr, *s2 = nullptr;
     if (is_ssd(m.kind)) {

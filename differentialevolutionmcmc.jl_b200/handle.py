@@ -11,7 +11,7 @@ from . import _ffi
 from ._ffi import _bp, _dp, _ip, check, f8, ptr
 
 KINDS = {"gaussian": 0, "mvnormal": 1, "binomial": 2, "lnr": 3, "lba": 4, "hier_normal": 5, "rastrigin": 6, "mvnormal_full": 7,
-         "custom": 8}
+         "custom": 8, "simulated": 9}
 UPDATES = {"mh": 0, "maximize": 1, "minimize": 2}
 FITNESS = {"posterior": 0, "fun": 1}
 PRIORS = {"flat": 0, "normal": 1, "halfcauchy": 2, "uniform": 3, "beta": 4, "normal_ref": 5}
@@ -90,12 +90,15 @@ class Handle:
 
     # ---- model ---------------------------------------------------------------------------------
     def set_model(self, kind, prior, x=None, choice=None, sigma=None, lba_floor=1e-10, device_ptrs=None, n_obs=None,
-                  n_dim=0, n_per=0, center=None, cov=None, source=None, n_cols=None):
+                  n_dim=0, n_per=0, center=None, cov=None, source=None, n_cols=None, n_sim=0, sim_floor=1e-10):
         """Bind a registered likelihood kernel.  `prior` is a list of (name, a, b, ref) per
         flattened parameter.  `device_ptrs=(x_ptr, choice_ptr)` passes data already in HBM.
         kind="custom": `source` is the CUDA C++ text of the likelihood (include/demcmc_b200.h: DEMCMC_CUSTOM) and x an
         n_obs-vector (n_cols = 1), an n_obs x n_cols matrix, or None (no observations); with device pointers pass
         n_obs and n_cols.
+        kind="simulated": `source` is the CUDA C++ text of the simulator (include/demcmc_b200.h: DEMCMC_SIMULATED), x an
+        n_obs-vector of values (n_cols = 1) or an n_obs x 2 matrix of (label, value) rows, n_sim the simulations per proposal
+        and sim_floor the density floor.
         `center` (mvnormal / hier_normal, test hook): centre the data on this vector instead of on their
         column means, which makes the streamed cross term non-zero (demcmc_model.center)."""
         d = self.d
@@ -127,7 +130,7 @@ class Handle:
                 n_obs = 1
             elif kind == "rastrigin":
                 n_obs = 0
-            elif kind == "custom":
+            elif kind in ("custom", "simulated"):
                 if x is None:
                     n_obs, n_cols = 0, 0
                 elif xs.ndim == 1:
@@ -135,7 +138,7 @@ class Handle:
                 elif xs.ndim == 2:
                     n_obs, n_cols = xs.shape
                 else:
-                    raise ValueError("custom data must be a vector or an n_obs x n_cols matrix")
+                    raise ValueError(f"{kind} data must be a vector or an n_obs x n_cols matrix")
             else:
                 n_obs = xs.shape[0]
                 if kind in ("lnr", "lba") and not n_dim:
@@ -149,10 +152,11 @@ class Handle:
             raise ValueError("mvnormal_full needs cov of shape (n_dim, n_dim)")
         src = None if source is None else source.encode() if isinstance(source, str) else bytes(source)
         m = _ffi.Model(kind_id, d, int(n_obs), int(n_dim), int(n_per), xp, cp, ptr(sg, _dp), float(lba_floor), pr, on_dev,
-                       int(n_cols or 0), ptr(cv, _dp), ptr(cen, _dp), src)
+                       int(n_cols or 0), ptr(cv, _dp), ptr(cen, _dp), src, int(n_sim), float(sim_floor))
         self._keep = [xs, cs, sg, pr, cen, cv, src]
         check(_ffi.lib().demcmc_set_model(self._h, C.byref(m)))
         self.n_obs = int(n_obs)
+        self.n_cols, self.n_sim = int(n_cols or 0), int(n_sim)
 
     # ---- state ---------------------------------------------------------------------------------
     def set_history(self, rows):
@@ -329,6 +333,19 @@ class Handle:
         check(_ffi.lib().demcmc_eval(self._h, ptr(th, _dp), n, ptr(ll, _dp), ptr(pr, _dp)))
         return ll, pr
 
+    def eval_simulated(self, theta, sweep, unit, sims=False):
+        """Test hook of a simulated model (demcmc_eval_simulated): the log-likelihoods of theta[n][d] under the explicit
+        simulation keys (sweep[i], unit[i]), and with sims=True also the simulations, an array [n, n_sim, n_cols]."""
+        th = f8(theta).reshape(-1, self.d)
+        n = th.shape[0]
+        sw = np.ascontiguousarray(np.broadcast_to(np.asarray(sweep, dtype=np.uint32), (n,)))
+        un = np.ascontiguousarray(np.broadcast_to(np.asarray(unit, dtype=np.uint32), (n,)))
+        ll = np.zeros(n)
+        out = np.zeros((n, self.n_sim, self.n_cols)) if sims else None
+        u32 = C.POINTER(C.c_uint32)
+        check(_ffi.lib().demcmc_eval_simulated(self._h, ptr(th, _dp), n, ptr(sw, u32), ptr(un, u32), ptr(ll, _dp), ptr(out, _dp)))
+        return (ll, out) if sims else ll
+
     def eval_pointwise(self, theta, obs0=0, n_obs=None):
         """log p(y_i | theta_s) for the draws theta[n][d] and observations [obs0, obs0 + n_obs) of the bound model (all from
         obs0 by default): an array [n, n_obs] (demcmc_eval_pointwise; priors are left out)."""
@@ -357,6 +374,16 @@ def compile_loglike(source):
     src = source.encode() if isinstance(source, str) else bytes(source)
     log = C.create_string_buffer(1 << 16)
     rc = _ffi.lib().demcmc_compile_loglike(src, log, len(log))
+    if rc != 0:
+        raise _ffi.DemcmcError(rc, log.value.decode(errors="replace") or _ffi.lib().demcmc_last_error().decode(errors="replace"))
+
+
+def compile_simulator(source):
+    """Compiles a simulated-likelihood source (DEMCMC_SIMULATED) for sm_100a (demcmc_compile_simulator; no device needed).
+    Raises DemcmcError with the compiler log when it does not compile; the result is cached for later set_model calls."""
+    src = source.encode() if isinstance(source, str) else bytes(source)
+    log = C.create_string_buffer(1 << 16)
+    rc = _ffi.lib().demcmc_compile_simulator(src, log, len(log))
     if rc != 0:
         raise _ffi.DemcmcError(rc, log.value.decode(errors="replace") or _ffi.lib().demcmc_last_error().decode(errors="replace"))
 

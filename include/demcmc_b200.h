@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define DEMCMC_ABI_VERSION 6
+#define DEMCMC_ABI_VERSION 7
 
 enum { DEMCMC_OK = 0, DEMCMC_EINVAL = -1, DEMCMC_ENODEVICE = -2, DEMCMC_ECUDA = -3, DEMCMC_ENOMEM = -4,
        DEMCMC_ESTATE = -5, DEMCMC_EUNSUPPORTED = -6, DEMCMC_ECOMM = -7 };
@@ -39,7 +39,9 @@ enum { DEMCMC_GAUSSIAN = 0, DEMCMC_MVNORMAL = 1, DEMCMC_BINOMIAL = 2, DEMCMC_LNR
                                    whitened once through the Cholesky factor (y = L^-1 x), every proposal's mean is whitened
                                    when it is staged (nu = L^-1 mu), and the isotropic kernels stream y against nu */,
        DEMCMC_CUSTOM = 8        /* a likelihood the caller writes in CUDA C++ (demcmc_model.source), compiled at run time for
-                                   sm_100a; see the source contract below */ };
+                                   sm_100a; see the source contract below */,
+       DEMCMC_SIMULATED = 9     /* a likelihood estimated from a simulator the caller writes in CUDA C++ (demcmc_model.source):
+                                   a Gaussian kernel density of demcmc_model.n_sim simulations per proposal; see below */ };
 /* DEMCMC_CUSTOM source contract.  demcmc_model.source is CUDA C++ text (no #include) that defines
  *   demcmc_obs       required (unless n_obs == 0): __device__ double, arguments (const double *par, const double *x): the
  *                    log density of ONE observation; x = that observation's n_cols values (row i of demcmc_model.x)
@@ -55,6 +57,49 @@ enum { DEMCMC_GAUSSIAN = 0, DEMCMC_MVNORMAL = 1, DEMCMC_BINOMIAL = 2, DEMCMC_LNR
  * DEMCMC_NAN are defined.  A custom model takes the level-by-level path only: the fused and persistent kernels are
  * specialised to the registered kinds. */
 #define DEMCMC_CUSTOM_MAX_PAR 256
+/* DEMCMC_SIMULATED source contract: a probability density approximation (PDA) of a model that can only be simulated
+ * (Turner & Sederberg 2014; Holmes 2015; the reference's Binomial_ABC.jl, KDE_Example.jl, Predator_Prey_Example.jl).
+ * demcmc_model.source is CUDA C++ text (no #include) that defines
+ *   demcmc_simulate  required: __device__ void, arguments (const double *par, demcmc_rng *rng, double *y): ONE synthetic
+ *                    observation y[n_cols] drawn under par, its random numbers taken from rng only
+ *   DEMCMC_NPAR      optional, with demcmc_prepare, exactly as for DEMCMC_CUSTOM
+ * and the text is given demcmc_rng and two generators:
+ *   demcmc_uniform   double, argument (demcmc_rng *): uniform on the open interval (0, 1): 53 random bits b, u = b 2^-53
+ *                    (b = 0, of probability 2^-53, gives 2^-54)
+ *   demcmc_normal    double, argument (demcmc_rng *): standard normal (Box-Muller on two uniforms; the second value of a
+ *                    pair is kept for the next call)
+ * The data are x[n_obs][n_cols], n_obs >= 1: n_cols = 1, one continuous value per observation; n_cols = 2, (label, value)
+ * with the label an integer-valued double in 1..K, K = the largest label of the data <= DEMCMC_SIM_MAX_LABELS (the
+ * (choice, RT) form of the sequential-sampling models).  The data are checked on the host (labels integers in range, values
+ * finite), so data_on_device is refused.  d and DEMCMC_NPAR are at most DEMCMC_CUSTOM_MAX_PAR.
+ *
+ * The estimator, for a proposal theta with key (sweep, unit):
+ *   1. simulations y_j = demcmc_simulate of (par, rng_j), j < M = demcmc_model.n_sim (16 <= M <= DEMCMC_SIM_MAX_DRAWS).  rng_j
+ *      is the Philox4x32-10 stream with key = the handle's seed and counter (c, unit, sweep, 8 + 16 j), c = 0, 1, ... counting
+ *      the Philox calls of the stream (two uniforms each): a function of (seed, sweep, unit, j) alone -- not of the level,
+ *      the launch geometry, the path or the device count -- and disjoint from the sampler's own streams (their last
+ *      counter word is 1..7).  In a run the key is (the sweep, the particle's global position group_begin * Np + j), the
+ *      unit of the proposal noise; the initial weights of demcmc_set_state use (DEMCMC_SIM_SWEEP_EVAL, global position),
+ *      demcmc_eval, demcmc_eval_pointwise and demcmc_loo use (DEMCMC_SIM_SWEEP_EVAL, index of the vector);
+ *   2. groups: G_c = { j : label of y_j is exactly c and the value of y_j is finite }, c = 1..K (n_cols = 1: one group, the
+ *      finite values).  Simulations outside every group still count in M, so the density is DEFECTIVE: label c's density
+ *      integrates to m_c / M (m_c = |G_c|);
+ *   3. bandwidth: a group with m_c >= 2 gets Silverman's rule, the default of KernelDensity.jl:
+ *      h_c = 0.9 min(s_c, IQR_c / 1.34) m_c^(-1/5), s_c the sample sd (ddof 1), IQR_c from linearly interpolated quantiles
+ *      (numpy's and Julia's default), s_c alone when IQR_c = 0.  A group with m_c < 2, or with h_c zero or not finite, has
+ *      no density;
+ *   4. density of an observation (c, t): f = sum_{j in G_c} phi((t - v_j) / h_c) / (M h_c), phi the standard normal density
+ *      and v_j the value of y_j; ll_i = log(max(f, sim_floor)), or log(sim_floor) when G_c has no density;
+ *   5. the log-likelihood is sum_i ll_i.
+ * This is the EXACT Gaussian kernel sum over all m_c simulations, not KernelDensity.jl's binned FFT approximation.  Every
+ * sum is formed in a fixed order (the group values sorted, per lane, then the warp's xor tree, then the observations in a
+ * fixed order), so a value is the same bits from run to run, on any number of devices and whichever kernel computes it.
+ * Pseudo-marginal semantics: only proposals are simulated.  The current particle keeps the estimate it was accepted with,
+ * as the reference's stored Particle.weight does; it is never re-evaluated.  A simulated model takes the level-by-level
+ * path only. */
+#define DEMCMC_SIM_MAX_DRAWS 16384
+#define DEMCMC_SIM_MAX_LABELS 8
+#define DEMCMC_SIM_SWEEP_EVAL 0xFFFFFFFFu   /* the sweep of every key outside a run (a run never reaches this sweep) */
 /* (Examples/Guassian_Example_Vector.jl is the Gaussian model with `loglike(data, theta...)` destructuring its arguments:
  * DEMCMC_GAUSSIAN is its kernel, d = 2 whether the two parameters are named separately or as one 2-vector.) */
 /* de.update_particle! (src/utilities.jl:201-226): mh_update!, or the greedy maximize! / minimize! of
@@ -110,7 +155,10 @@ typedef struct {
                                m' = L^-1 (mu - c); with NULL the y are then centred on their own column means (about 0)
                                and B is analytically zero, with an explicit centre they are not, and
                                B = sum_i y_i . L^-1 (mu - center). */
-    const char *source;     /* CUSTOM: NUL-terminated CUDA C++ source (host memory), see DEMCMC_CUSTOM; else NULL */
+    const char *source;     /* CUSTOM / SIMULATED: NUL-terminated CUDA C++ source (host memory), see DEMCMC_CUSTOM /
+                               DEMCMC_SIMULATED; else NULL */
+    int32_t n_sim;          /* SIMULATED: simulations per proposal M, 16 <= M <= DEMCMC_SIM_MAX_DRAWS */
+    double sim_floor;       /* SIMULATED: density floor, > 0 (1e-10 by default, as lba_floor) */
 } demcmc_model;
 
 /* Mirrors the DE sampler struct field by field (src/structs.jl:57-131). */
@@ -206,6 +254,8 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *model);
  * NULL) and into demcmc_last_error(); DEMCMC_EUNSUPPORTED when libnvrtc.so.12 cannot be loaded or DEMCMC_NPAR is above
  * DEMCMC_CUSTOM_MAX_PAR. */
 int demcmc_compile_loglike(const char *source, char *log, int64_t log_cap);
+/* The same for a DEMCMC_SIMULATED source (cached apart from a DEMCMC_CUSTOM source of the same text). */
+int demcmc_compile_simulator(const char *source, char *log, int64_t log_cap);
 /* initialize_samples (src/utilities.jl:29-41) when n_initial > 0: rows[n_initial][P][d], row i = the
  * i-th sample_prior() draw of every particle id; they become rows 1..n_initial of de.samples.  A sharded
  * job passes the rows of its own particles, [n_initial][P_local][d] -- unless sample = resample: then (after
@@ -309,6 +359,11 @@ int demcmc_set_lanes(demcmc_handle *h, int32_t n_lanes);
 int demcmc_eval(demcmc_handle *h, const double *theta, int64_t n, double *loglike, double *prior);
 /* the cross term B (see demcmc_get_trace_xdot) of n arbitrary parameter vectors theta[n][d], through k_xdot */
 int demcmc_eval_xdot(demcmc_handle *h, const double *theta, int64_t n, double *xdot);
+/* DEMCMC_SIMULATED test hook: loglike[n] of n vectors theta[n][d] under the explicit keys (sweep[i], unit[i]) of
+ * DEMCMC_SIMULATED step 1 (the value a run computes for a proposal with that key), and, when sims is not NULL, the
+ * simulations sims[n][n_sim][n_cols] in j order */
+int demcmc_eval_simulated(demcmc_handle *h, const double *theta, int64_t n, const uint32_t *sweep, const uint32_t *unit,
+                          double *loglike, double *sims);
 /* SURVEY hard part 7: with the data centred on their column means the cross term is analytically zero, so the
  * MVNORMAL / HIER_NORMAL likelihood follows from O(d) sufficient statistics alone.  on = 1 skips the O(N d) stream
  * (k_xdot / k_chunk_persist are not launched; B is taken as 0).  Off by default: the headline metric counts
@@ -321,7 +376,8 @@ int demcmc_set_sufficient_stat(demcmc_handle *h, int32_t on);
  * An observation is what demcmc_model.n_obs counts: GAUSSIAN x_i; MVNORMAL / MVNORMAL_FULL row x_i, with the log density
  * logpdf(MvNormal(mu, sigma^2 I or sigma^2 Sigma), x_i); HIER_NORMAL y_sj in the subject-major order of demcmc_model.x
  * (n_obs = n_dim * n_per); LNR / LBA one trial; BINOMIAL the single (N, k) (n_obs = 1); CUSTOM row x_i, its log density
- * the value demcmc_obs returns for it.
+ * the value demcmc_obs returns for it; SIMULATED row x_i, its log density ll_i of DEMCMC_SIMULATED step 4 (draw j simulated
+ * under the key (DEMCMC_SIM_SWEEP_EVAL, j), so a row sums to the demcmc_eval value of the draw up to the summation order).
  * Priors are left out, and so is the demcmc_particle term of a CUSTOM model (it belongs to no observation).  A model
  * without observations (RASTRIGIN, CUSTOM with n_obs = 0) is refused with DEMCMC_EINVAL; so is an observation range
  * outside [0, n_obs).  Before demcmc_set_model: DEMCMC_ESTATE.

@@ -23,9 +23,9 @@
 # GPU path with a closure throws an ArgumentError -- there is no silent CPU fallback.
 
 const LIBDEMCMC = get(ENV, "LIBDEMCMC_B200", "libdemcmc_b200.so")
-const DEMCMC_ABI_VERSION = Int32(6)
+const DEMCMC_ABI_VERSION = Int32(7)
 
-const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7, custom = 8)
+const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7, custom = 8, simulated = 9)
 const GPU_PRIORS = (flat = 0, normal = 1, halfcauchy = 2, uniform = 3, beta = 4, normal_ref = 5)
 
 """
@@ -41,6 +41,14 @@ per-subject vectors / `n_per × n_subj` matrix (`:hier_normal`).
 A likelihood written as CUDA C++ (`source`, the DEMCMC_CUSTOM contract of include/demcmc_b200.h: `demcmc_obs`, and
 optionally `demcmc_particle` / `DEMCMC_NPAR` + `demcmc_prepare`), compiled by the library for sm_100a.  `X` is a vector
 (one value per observation), an `n_cols × n_obs` matrix (one column per observation), or `nothing` (no data).
+
+    GPULoglike(:simulated, X; source, n_sim, floor = 1e-10)
+
+A likelihood estimated on the device from `n_sim` simulations per proposal of a simulator written as CUDA C++ (`source`,
+the DEMCMC_SIMULATED contract of include/demcmc_b200.h: `demcmc_simulate(par, rng, y)` with `demcmc_uniform` /
+`demcmc_normal`, and optionally `DEMCMC_NPAR` + `demcmc_prepare`): a Gaussian kernel density per label, Silverman's
+bandwidth, floored at `floor`.  `X` is a vector of values, or a `2 × n_obs` matrix of (label 1..8, value) columns.  Only
+proposals are simulated: a particle keeps the estimate it was accepted with (pseudo-marginal).
 """
 struct GPULoglike{D}
     kind::Symbol
@@ -48,7 +56,9 @@ struct GPULoglike{D}
     sigma::Union{Nothing, Vector{Float64}}
     lba_floor::Float64
     cov::Matrix{Float64}   # :mvnormal_full: the known covariance Σ of MvNormal(μ, σ²Σ); empty otherwise
-    source::String         # :custom: the CUDA C++ source of the likelihood; empty otherwise
+    source::String         # :custom / :simulated: the CUDA C++ source of the likelihood / simulator; empty otherwise
+    n_sim::Int32           # :simulated: simulations per proposal; 0 otherwise
+    sim_floor::Float64     # :simulated: density floor
 end
 
 function GPULoglike(kind::Symbol; x = nothing, choice = nothing, rt = nothing, N = nothing, k = nothing,
@@ -64,17 +74,25 @@ function GPULoglike(kind::Symbol; x = nothing, choice = nothing, rt = nothing, N
         (x = Array{Float64}(x), choice = nothing)
     end
     kind == :mvnormal_full && size(cov) != (size(data.x, 1), size(data.x, 1)) && throw(ArgumentError(":mvnormal_full needs cov, n_dim × n_dim"))
-    return GPULoglike(kind, data, sigma === nothing ? nothing : Vector{Float64}(sigma), Float64(lba_floor), Matrix{Float64}(cov), "")
+    return GPULoglike(kind, data, sigma === nothing ? nothing : Vector{Float64}(sigma), Float64(lba_floor), Matrix{Float64}(cov), "", Int32(0), 1e-10)
 end
 
 # the source is compiled when the model is bound (demcmc_set_model caches the cubin per source text); a source that
-# does not compile raises there, with the compiler log as the library's error message
-function GPULoglike(kind::Symbol, X; source::AbstractString)
-    kind == :custom || throw(ArgumentError("GPULoglike(kind, X; source) is the :custom form"))
-    isempty(source) && throw(ArgumentError(":custom needs the CUDA source of demcmc_obs"))
-    x = X === nothing ? zeros(0, 0) : X isa AbstractVector ? Matrix{Float64}(reshape(X, 1, :)) : Matrix{Float64}(X)
-    (X !== nothing && size(x, 1) == 0) && throw(ArgumentError(":custom data need at least one value per observation"))
-    return GPULoglike(kind, (x = x, choice = nothing), nothing, 1e-10, zeros(0, 0), String(source))
+# does not compile raises there, with the compiler log as the library's error message.  :simulated data and arguments are
+# checked again by demcmc_set_model.
+function GPULoglike(kind::Symbol, X; source::AbstractString, n_sim::Integer = 0, floor::Real = 1e-10)
+    kind in (:custom, :simulated) || throw(ArgumentError("GPULoglike(kind, X; source) is the :custom / :simulated form"))
+    isempty(source) && throw(ArgumentError(":$kind needs the CUDA source of " * (kind == :custom ? "demcmc_obs" : "demcmc_simulate")))
+    if kind == :custom
+        x = X === nothing ? zeros(0, 0) : X isa AbstractVector ? Matrix{Float64}(reshape(X, 1, :)) : Matrix{Float64}(X)
+        (X !== nothing && size(x, 1) == 0) && throw(ArgumentError(":custom data need at least one value per observation"))
+        return GPULoglike(kind, (x = x, choice = nothing), nothing, 1e-10, zeros(0, 0), String(source), Int32(0), 1e-10)
+    end
+    16 <= n_sim <= 16384 || throw(ArgumentError(":simulated needs 16 <= n_sim <= 16384, got $n_sim"))
+    floor > 0 || throw(ArgumentError(":simulated needs floor > 0, got $floor"))
+    x = X isa AbstractVector ? Matrix{Float64}(reshape(X, 1, :)) : Matrix{Float64}(X)
+    size(x, 1) in (1, 2) || throw(ArgumentError(":simulated data are values or (label, value) columns"))
+    return GPULoglike(kind, (x = x, choice = nothing), nothing, 1e-10, zeros(0, 0), String(source), Int32(n_sim), Float64(floor))
 end
 
 # the device evaluates it; calling it on the host is an error, never a fallback
@@ -146,7 +164,9 @@ struct CModel
     n_cols::Int32          # :custom: values per observation (rows of the n_cols × n_obs data matrix)
     cov::Ptr{Float64}      # :mvnormal_full: the known covariance, n_dim × n_dim
     center::Ptr{Float64}   # C_NULL: centre the data on their column means (the product default)
-    source::Ptr{UInt8}     # :custom: NUL-terminated CUDA source (a Julia String's pointer), else C_NULL
+    source::Ptr{UInt8}     # :custom / :simulated: NUL-terminated CUDA source (a Julia String's pointer), else C_NULL
+    n_sim::Int32           # :simulated: simulations per proposal
+    sim_floor::Float64     # :simulated: density floor
 end
 
 struct CConfig
@@ -250,7 +270,7 @@ end
 function model_geometry(ll::GPULoglike, d)
     x = ll.data.x
     n_dim, n_per, n_obs, n_cols = 0, 0, length(x), 0
-    if ll.kind == :custom
+    if ll.kind == :custom || ll.kind == :simulated
         n_cols, n_obs = size(x)
     elseif ll.kind == :mvnormal || ll.kind == :mvnormal_full
         n_dim, n_obs = size(x)
@@ -321,7 +341,7 @@ function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_e
         try
             m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), choice === nothing ? C_NULL : pointer(choice),
                 isempty(sig) ? C_NULL : pointer(sig), ll.lba_floor, pointer(priors), 0, n_cols, isempty(covm) ? C_NULL : pointer(covm), C_NULL,
-                isempty(src) ? C_NULL : pointer(src))
+                isempty(src) ? C_NULL : pointer(src), ll.n_sim, ll.sim_floor)
             demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
             if n_blocks > 0 && !all(!iszero, block_on)         # block updating in some iterations only
                 GC.@preserve block_on demcmc_check(ccall((:demcmc_set_blocking_schedule, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Int64), h[], block_on, length(block_on)))
@@ -387,7 +407,7 @@ function _sample_gpu_thinned(model, de, n_iter; device, devices, store_every, se
             pointer(lo), pointer(hi), seed, device, 0, 0, 0, 0, store_every, 0, 0, length(devs), isempty(devs) ? C_NULL : pointer(devs))
         demcmc_check(ccall((:demcmc_create, LIBDEMCMC), Cint, (Ref{CConfig}, Ref{Ptr{Cvoid}}), cfg, h))
         try
-            m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), C_NULL, C_NULL, ll.lba_floor, pointer(priors), 0, 0, C_NULL, C_NULL, C_NULL)
+            m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), C_NULL, C_NULL, ll.lba_floor, pointer(priors), 0, 0, C_NULL, C_NULL, C_NULL, Int32(0), 1e-10)
             demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
             demcmc_check(ccall((:demcmc_set_state, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}), h[], theta0, C_NULL))
             demcmc_check(ccall((:demcmc_run, LIBDEMCMC), Cint, (Ptr{Cvoid}, Int64), h[], n_iter))
@@ -491,7 +511,7 @@ function _with_likelihood(f, model::DEModel{<:GPULoglike}, chains; device = 0)
         try
             m = CModel(GPU_KINDS[ll.kind], d, n_obs, n_dim, n_per, pointer(x), choice === nothing ? C_NULL : pointer(choice),
                 isempty(sig) ? C_NULL : pointer(sig), ll.lba_floor, pointer(priors), 0, n_cols, isempty(covm) ? C_NULL : pointer(covm), C_NULL,
-                isempty(src) ? C_NULL : pointer(src))
+                isempty(src) ? C_NULL : pointer(src), ll.n_sim, ll.sim_floor)
             demcmc_check(ccall((:demcmc_set_model, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ref{CModel}), h[], m))
             return f(h[], theta, size(theta, 2), n_obs), size(v, 1), size(v, 3)
         finally
