@@ -10,4 +10,4 @@ from .handle import (Handle, comm_unique_id, copy_peak, fp64_peak, fp64_peaks, o
                      op_reset, op_select, op_snooker)
 from .api import (DE, DEModel, GPUDEModel, Beta, Chains, Flat, GPULoglike, GPUPrior, HalfCauchy, MCMCThreads, Normal,  # noqa: F401
                   NormalRef, Particle, Uniform, compute_posterior, evaluate_fun, fixed_gamma, get_optimal, maximize,
-                  mh_update, minimize, optimize, pointwise_loglikelihoods, loo, random_gamma, resample, sample, variable_gamma)
+                  mh_update, minimize, optimize, pointwise_loglikelihoods, loo, power_posterior, random_gamma, resample, sample, variable_gamma)

@@ -13,7 +13,7 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DEFAULT_LIB = os.path.join(_HERE, "libdemcmc_b200.so")
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int32)
@@ -63,13 +63,19 @@ class Counters(C.Structure):
                 ("mailbox_events", C.c_int64), ("cross_migrations", C.c_int64)]
 
 
+class Evidence(C.Structure):
+    _fields_ = [("n_rungs", C.c_int32), ("log_z_ti", C.c_double), ("log_z_ti2", C.c_double), ("log_z_ss", C.c_double),
+                ("se_ti", C.c_double), ("se_ss", C.c_double)]
+
+
 # every symbol include/demcmc_b200.h declares (tests check the library exports all of them)
 SYMBOLS = [
     "demcmc_last_error", "demcmc_abi_version", "demcmc_device_count", "demcmc_backend_name", "demcmc_create",
     "demcmc_destroy", "demcmc_set_model", "demcmc_compile_loglike", "demcmc_compile_simulator", "demcmc_set_history", "demcmc_set_state", "demcmc_run", "demcmc_replay", "demcmc_get_samples",
     "demcmc_get_accept", "demcmc_get_lp", "demcmc_get_chains", "demcmc_get_moments", "demcmc_set_iteration", "demcmc_set_weights", "demcmc_set_blocking_schedule", "demcmc_get_history_by_slot", "demcmc_get_state", "demcmc_get_trace",
     "demcmc_get_trace_xdot", "demcmc_eval_xdot", "demcmc_eval_simulated", "demcmc_set_sufficient_stat", "demcmc_get_diagnostics",
-    "demcmc_get_migration", "demcmc_get_counters", "demcmc_set_timing", "demcmc_set_max_chunk", "demcmc_set_lanes", "demcmc_eval", "demcmc_eval_pointwise", "demcmc_loo", "demcmc_op_project", "demcmc_op_reset",
+    "demcmc_get_migration", "demcmc_get_counters", "demcmc_set_timing", "demcmc_set_max_chunk", "demcmc_set_lanes", "demcmc_eval", "demcmc_eval_pointwise", "demcmc_loo",
+    "demcmc_set_temperatures", "demcmc_get_loglike", "demcmc_power_posterior", "demcmc_op_project", "demcmc_op_reset",
     "demcmc_op_de_proposal", "demcmc_op_snooker", "demcmc_op_accept", "demcmc_op_select", "demcmc_comm_unique_id",
     "demcmc_comm_init", "demcmc_fp64_peak", "demcmc_fp64_peaks", "demcmc_copy_peak",
 ]
@@ -118,6 +124,9 @@ def _declare(L):
     L.demcmc_eval.argtypes = [C.c_void_p, _dp, C.c_int64, _dp, _dp]
     L.demcmc_eval_pointwise.argtypes = [C.c_void_p, _dp, C.c_int64, C.c_int64, C.c_int64, _dp]
     L.demcmc_loo.argtypes = [C.c_void_p, _dp, C.c_int64, _dp, _dp, _dp, _dp]
+    L.demcmc_set_temperatures.argtypes = [C.c_void_p, _dp, C.c_int32]
+    L.demcmc_get_loglike.argtypes = [C.c_void_p, _dp, C.c_int64]
+    L.demcmc_power_posterior.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.POINTER(Evidence), _dp, _dp, _dp, _dp, _dp, _dp]
     L.demcmc_op_project.argtypes = [C.c_int, _dp, _dp, C.c_int32, _dp]
     L.demcmc_op_reset.argtypes = [C.c_int, _dp, _dp, _bp, C.c_int32, _dp]
     L.demcmc_op_de_proposal.argtypes = [C.c_int, _dp, _dp, _dp, _dp, C.c_double, C.c_double, _dp, C.c_int32, _dp]

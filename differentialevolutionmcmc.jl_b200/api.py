@@ -507,6 +507,28 @@ def build_handle(model: DEModel, de: DE, device=0, trace=False, group_begin=0, g
     return h, shapes, d
 
 
+def _init_state(h, model: DEModel, de: DE, d, binding, temperatures=None):
+    """The particles of sample_init, once the model is bound; temperatures (per group of the job) temper the handle first."""
+    P = de.n_groups * de.Np
+    rows = theta0 = None
+    if de.n_initial > 0:
+        # initialize_samples (src/utilities.jl:29-41): for every particle id, n_initial sample_prior()
+        # draws; init_particle then starts each particle from samples[1, :, id] (utilities.jl:15)
+        rows = np.empty((de.n_initial, P, d))
+        for p in range(P):
+            for i in range(de.n_initial):
+                _fill_flat(model.sample_prior(), rows[i, p])
+    else:
+        # sample_init (src/main.jl:263-271): one sample_prior() per particle, id order -- drawn while the data upload runs
+        theta0 = _draw_states(model.sample_prior, P, d)
+    binding.join()                                       # the data set is on the device and packed
+    if temperatures is not None:
+        h.set_temperatures(temperatures)
+    if rows is not None:
+        h.set_history(rows)
+    h.set_state(theta0)
+
+
 def sample(model: DEModel, de: DE, *args, progress=False, device=0, devices=None, store_every=1, **kwargs):
     """sample(model, de, n_iter) / sample(model, de, MCMCThreads(), n_iter): runs all n_iter
     iterations on the device in ONE library call and returns the chains (src/main.jl:19-71).
@@ -520,22 +542,7 @@ def sample(model: DEModel, de: DE, *args, progress=False, device=0, devices=None
         raise TypeError("sample(model, de, n_iter) or sample(model, de, MCMCThreads(), n_iter)")
     h, shapes, d, binding = build_handle(model, de, device=device, n_iter=n_iter, devices=devices, store_every=store_every, background_model=True)
     try:
-        P = de.n_groups * de.Np
-        if de.n_initial > 0:
-            # initialize_samples (src/utilities.jl:29-41): for every particle id, n_initial sample_prior()
-            # draws; init_particle then starts each particle from samples[1, :, id] (utilities.jl:15)
-            rows = np.empty((de.n_initial, P, d))
-            for p in range(P):
-                for i in range(de.n_initial):
-                    _fill_flat(model.sample_prior(), rows[i, p])
-            binding.join()                                   # the data set is on the device and packed
-            h.set_history(rows)
-            h.set_state(None)
-        else:
-            # sample_init (src/main.jl:263-271): one sample_prior() per particle, id order -- drawn while the data upload runs
-            theta0 = _draw_states(model.sample_prior, P, d)
-            binding.join()
-            h.set_state(theta0)
+        _init_state(h, model, de, d, binding)
         h.run(n_iter)
         de.iter = n_iter + de.n_initial
         # bundle_samples (src/main.jl:222-250) runs on the device: one gather, one download, and the
@@ -548,6 +555,43 @@ def sample(model: DEModel, de: DE, *args, progress=False, device=0, devices=None
     finally:
         try:
             binding.join()                                   # (an exception above: let the upload finish before the handle goes)
+        except BaseException:                                # noqa: BLE001
+            pass
+        h.close()
+
+
+def power_posterior(model: DEModel, de: DE, n_iter, temperatures=None, n_temperatures=32, power=5.0, device=0, devices=None,
+                    store_every=1):
+    """The marginal likelihood log p(y) by power posteriors, in ONE run: rung k is de.n_groups groups of de.Np particles whose
+    weights are prior + t_k loglike, t_k = (k / (K - 1))^power by default (Friel & Pettitt 2008), all K rungs in one handle of
+    K * de.n_groups groups.  Burn-in is dropped as sample() drops it.  Returns a dict: the totals log_z_ti (trapezoid rule),
+    log_z_ti2 (corrected trapezoid), log_z_ss (stepping stones) and their standard errors se_ti, se_ss; the per-rung arrays
+    t, mean_ll, var_ll, ess_ll, rhat_ll, log_ratio (include/demcmc_b200.h: demcmc_power_posterior); and chains, the t = 1
+    rung's Chains, a posterior sample like sample()'s."""
+    import copy
+    t = np.asarray([(k / (n_temperatures - 1)) ** power for k in range(n_temperatures)] if temperatures is None else temperatures, dtype=np.float64)
+    K = t.size
+    if de.α > 0 and K * de.n_groups > 1:
+        raise ValueError("power_posterior runs every rung as groups of one handle, and migration would move particles between "
+                         "temperatures: pass DE(α = 0)")
+    job = copy.copy(de)
+    job.n_groups = K * de.n_groups
+    n_iter = int(n_iter)
+    h, shapes, d, binding = build_handle(model, job, device=device, n_iter=n_iter, devices=devices, store_every=store_every, background_model=True)
+    try:
+        _init_state(h, model, job, d, binding, temperatures=np.repeat(t, de.n_groups))
+        h.run(n_iter)
+        offset = (de.burnin // h.store_every) if de.discard_burnin else 0
+        row0 = max(offset, de.n_initial)
+        out = h.power_posterior(row0, h.n_rows - row0)
+        arr = h.chains(offset, max(n_iter // h.store_every - offset, 0))
+        top = arr[(K - 1) * de.n_groups * de.Np:]           # the particles of the t = 1 rung
+        names = _flat_names(model.names, shapes) + ["acceptance", "lp"]
+        out["chains"] = Chains(top.transpose(2, 1, 0), names, [str(n) for n in model.names])
+        return out
+    finally:
+        try:
+            binding.join()
         except BaseException:                                # noqa: BLE001
             pass
         h.close()

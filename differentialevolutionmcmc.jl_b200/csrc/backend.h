@@ -157,6 +157,17 @@ int launch_moments(const double *x, int64_t n, int32_t d, double *mean, double *
 // split-R-hat and ESS (engine.cpp: diag_finish).
 int launch_diag_pos(const int32_t *rows_id, int64_t row0, int64_t n_rows, int32_t P_local, int32_t id_base, int32_t P_ids, int32_t pos_base, int32_t *pos);
 int launch_diag_aggregates(const DiagShards &sh, const int32_t *pos, int64_t row0, int64_t n_rows, int32_t P_ids, int32_t d, int32_t lag0, int32_t n_lag, double *agg);   // lags [lag0, lag0 + n_lag)
+// Power posteriors.  Declared weak, like launch_pointwise: a backend without them (the plain host-only test double) leaves
+// them null, and the engine refuses demcmc_set_temperatures with DEMCMC_EUNSUPPORTED (tests/emu/emu_power_posterior.cpp
+// holds host versions that tests/test_power_posterior.py builds into a test double of its own).
+// k_power_posterior: the stored untempered log-likelihoods ll_rows[row][P_local] of rows [row0, row0 + n_rows), cut into
+// slices of PP_ROWS rows of one local group; part[G_local][n_slices][PP_OUT] (device) gets each slice's
+// [count, mean, m2, max, sum e, sum e^2], e = exp(delta.v[g] (ll - slice max)) (de_types.h: PP_OUT).
+int launch_power_posterior(const double *ll_rows, int64_t row0, int64_t n_rows, int32_t P_local, int32_t Np, int32_t G_local,
+                           const PPDelta &delta, double *part) __attribute__((weak));
+// k_temper_weights: the initial weights of a tempered handle, w[p] = prior[p] + tempered_ll(group of p, ll[p]), or -Inf
+// where prior[p] is -Inf (out of bounds: launch_eval's prior output), for the n = P_local particles by local position
+int launch_temper_weights(const ConfigDev &cfg, const double *prior, const double *ll, int64_t n, double *w) __attribute__((weak));
 int diag_max_half();   // longest split chain (stored rows / 2) one call can hold, and
 int diag_max_lags();   // the most lags one call computes
 // particle algebra known-answer ops (single warp each)

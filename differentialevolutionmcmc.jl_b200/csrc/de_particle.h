@@ -346,8 +346,9 @@ DE_PRAGMA_UNROLL
 }
 
 // compute_posterior! tail + mh_update! (utilities.jl:92-99, 201-210) + the row write that replaces
-// store_samples! (utilities.jl:161-180)
-template <class C>
+// store_samples! (utilities.jl:161-180).  TEMPER = false compiles the power-posterior terms out (ConfigDev.temp and
+// SweepCtx.next_ll must then be NULL): the kernels that are tight on registers take it for untempered handles.
+template <class C, bool TEMPER = true>
 DE_HD void accept_particle(const C &co, const ConfigDev &cfg, const ModelDev &m, const SweepCtx &ctx, int p)
 {
     const int d = cfg.d, Np = cfg.Np;
@@ -372,11 +373,13 @@ DE_HD void accept_particle(const C &co, const ConfigDev &cfg, const ModelDev &m,
     // compute_posterior! (utilities.jl:92-99), or evaluate_fun! (utilities.jl:113-120): the kernel
     // alone, and out of bounds loses every comparison
     const double wprop = cfg.fitness == FITNESS_FUN ? (inb ? ll : (cfg.update == UPDATE_MAXIMIZE ? -inf() : inf()))
-                                                    : (inb ? add(ctx.prop_prior[p], ll) : -inf());
+                                                    : (inb ? add(ctx.prop_prior[p], TEMPER ? tempered_ll(cfg, cfg.group_begin + g, ll) : ll) : -inf());
     const double adj = ctx.prop_adj[p];
     const double wcur = ctx.cur_w[p];
     // mh_update! (utilities.jl:201-210), maximize! / minimize! (utilities.jl:212-226)
     const bool acc = cfg.update == UPDATE_MAXIMIZE ? wprop > wcur : cfg.update == UPDATE_MINIMIZE ? wprop < wcur : accept(wprop, wcur, adj, u);
+    // (written here, not with the other lane-0 stores below: ll then dies before the row copy, which needs the registers)
+    if (TEMPER && ctx.next_ll && co.lane() == 0) ctx.next_ll[p] = acc ? ll : ctx.cur_ll[p];
     double *dst = ctx.next_theta + (size_t)p * d;
     const double *src = acc ? prop : tcur;                     // (uniform over the lanes: only the row that is kept is read)
     {

@@ -104,6 +104,8 @@ struct ConfigDev {
     const double *lo, *hi;    // [d]
     const uint8_t *blocks;    // [n_blocks][d]
     uint64_t seed;
+    const double *temp;       // [n_groups] power-posterior temperature of each global group (demcmc_set_temperatures), or
+                              // NULL: untempered
 };
 
 // The state-independent draws of one particle update (kind, donor slots, gammas, the select_base and accept uniforms):
@@ -150,6 +152,8 @@ struct SweepCtx {
     // trace rows of this sweep or NULL
     double *tr_theta, *tr_w, *tr_adj; uint8_t *tr_acc;
     double *tr_xdot;          // MVN / hierarchical: the cross term the likelihood kernel produced for the proposal
+    // tempered handle (ConfigDev.temp): the untempered log-likelihood of each particle, kept with theta; else NULL
+    const double *cur_ll; double *next_ll;
 };
 
 // One launch: the (sweep slot, local position) updates of one dependency level.  Entry encoding:
@@ -177,5 +181,20 @@ struct Mbox { double *rows; unsigned long long *flags; int32_t depth, max_rows, 
 // of shard q / P_local
 struct DiagShards { const double *theta[MAX_RANKS]; int32_t n, P_local; };
 struct PeerTable { double *rows[MAX_RANKS]; unsigned long long *flags[MAX_RANKS]; };
+// k_power_posterior: the stored log-likelihoods of one group over PP_ROWS consecutive rows are one slice; its six
+// partials are [count, mean, m2 = sum (ll - mean)^2, max, sum e, sum e^2], e = exp(delta (ll - max)).  The slices depend
+// on the group and the row range alone, so the partials are the same on any number of devices.
+constexpr int PP_ROWS = 256;
+constexpr int PP_OUT = 6;
+struct PPDelta { double v[MAX_MIG]; };   // delta = t_(k+1) - t_k of the rung k of each local group (0 on the last rung)
+
+// the weight's likelihood term of a particle of global group g: t_g loglike, or loglike itself when untempered.  At t = 0
+// the term is 0 whatever the likelihood (the prior alone, as L^0 = 1 reads even where L = 0).
+DE_HD double tempered_ll(const ConfigDev &cfg, int g, double ll)
+{
+    if (!cfg.temp) return ll;
+    const double t = cfg.temp[g];
+    return t == 0.0 ? 0.0 : mul(t, ll);
+}
 
 } // namespace de

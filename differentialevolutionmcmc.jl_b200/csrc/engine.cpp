@@ -41,7 +41,7 @@ static int fail(int code, const char *fmt, ...)
 
 namespace {
 
-struct Row { double *theta; double *w; int32_t *id; uint8_t *acc; };
+struct Row { double *theta; double *w; int32_t *id; uint8_t *acc; double *ll; /* untempered log-likelihood, tempered handles only */ };
 
 struct Upload {            // pinned staging + device copy of one sweep's schedule
     // ONE pinned block and ONE device block per slot, copied with one cudaMemcpyAsync per chunk:
@@ -139,6 +139,11 @@ struct demcmc_handle {
     int64_t flush_bytes = 0;
     bool time_loglik = false;
     bool suffstat = false;                              // demcmc_set_sufficient_stat: the O(N d) stream is skipped
+    // power posteriors (demcmc_set_temperatures): the temperature of every group of the job, on the host and the device,
+    // and the untempered log-likelihood of every state row (history and scratch, [row][P]); all empty when untempered
+    std::vector<double> temper;
+    std::vector<int32_t> prior_kind;                    // DEMCMC_PRIOR_* of each parameter of the bound model
+    double *d_temp = nullptr, *hist_ll = nullptr, *scr_ll = nullptr;
     void *flush_buf = nullptr;
     std::vector<void *> tev;                            // pool of timing events
 };
@@ -147,8 +152,8 @@ static Row row_of(demcmc_handle *h, bool hist, int64_t idx)
 {
     const size_t P = h->P, d = h->d;
     Row r;
-    if (hist) { r.theta = h->hist_theta + idx * P * d; r.w = h->hist_w + idx * P; r.id = h->hist_id + idx * P; r.acc = h->hist_acc + idx * P; }
-    else { r.theta = h->scr_theta + idx * P * d; r.w = h->scr_w + idx * P; r.id = h->scr_id + idx * P; r.acc = h->scr_acc + idx * P; }
+    if (hist) { r.theta = h->hist_theta + idx * P * d; r.w = h->hist_w + idx * P; r.id = h->hist_id + idx * P; r.acc = h->hist_acc + idx * P; r.ll = h->hist_ll ? h->hist_ll + idx * P : nullptr; }
+    else { r.theta = h->scr_theta + idx * P * d; r.w = h->scr_w + idx * P; r.id = h->scr_id + idx * P; r.acc = h->scr_acc + idx * P; r.ll = h->scr_ll ? h->scr_ll + idx * P : nullptr; }
     return r;
 }
 // history rows held after `iters` iterations of this handle: the n_initial prior rows + every k_store-th iteration
@@ -170,13 +175,16 @@ static int grow_history(demcmc_handle *h, int64_t need)
     int32_t *ni = (int32_t *)be::dmalloc(sizeof(int32_t) * cap * P);
     uint8_t *na = (uint8_t *)be::dmalloc(cap * P);
     int32_t *np = h->cfg.donors ? (int32_t *)be::dmalloc(sizeof(int32_t) * cap * P) : nullptr;
-    if (!nt || !nw || !ni || !na || (h->cfg.donors && !np)) return fail(DEMCMC_ENOMEM, "history of %lld rows does not fit on the device", (long long)cap);
+    const bool tempered = !h->temper.empty();
+    double *nl = tempered ? (double *)be::dmalloc(sizeof(double) * cap * P) : nullptr;
+    if (!nt || !nw || !ni || !na || (h->cfg.donors && !np) || (tempered && !nl)) return fail(DEMCMC_ENOMEM, "history of %lld rows does not fit on the device", (long long)cap);
     if (have > 0) {
         BE(be::d2d(nt, h->hist_theta, sizeof(double) * have * P * d));
         BE(be::d2d(nw, h->hist_w, sizeof(double) * have * P));
         BE(be::d2d(ni, h->hist_id, sizeof(int32_t) * have * P));
         BE(be::d2d(na, h->hist_acc, have * P));
         if (np) BE(be::d2d(np, h->hist_pos, sizeof(int32_t) * have * P));
+        if (nl && h->hist_ll) BE(be::d2d(nl, h->hist_ll, sizeof(double) * have * P));
         BE(be::sync());
     }
     if (h->cfg.donors && h->n_ranks > 1) {
@@ -193,7 +201,8 @@ static int grow_history(demcmc_handle *h, int64_t need)
         be::dfree(h->ghist_theta); be::dfree(h->ghist_pos);
         h->ghist_theta = gt; h->ghist_pos = gp;
     }
-    be::dfree(h->hist_theta); be::dfree(h->hist_w); be::dfree(h->hist_id); be::dfree(h->hist_acc); be::dfree(h->hist_pos);
+    be::dfree(h->hist_theta); be::dfree(h->hist_w); be::dfree(h->hist_id); be::dfree(h->hist_acc); be::dfree(h->hist_pos); be::dfree(h->hist_ll);
+    h->hist_ll = nl;
     h->hist_theta = nt; h->hist_w = nw; h->hist_id = ni; h->hist_acc = na; h->hist_pos = np; h->hist_cap = cap;
     return 0;
 }
@@ -395,7 +404,8 @@ static int multi_interleave(demcmc_handle *p, T *out, int64_t rows, size_t w, F 
     return 0;
 }
 
-static int multi_history_out(demcmc_handle *p, double *samples, double *lp, uint8_t *accept, int64_t n_rows)
+// ll_col: the lp output takes the stored untempered log-likelihoods instead of the weights (demcmc_get_loglike)
+static int multi_history_out(demcmc_handle *p, double *samples, double *lp, uint8_t *accept, int64_t n_rows, bool ll_col)
 {
     demcmc_handle *k0 = p->kids[0];
     if (n_rows != stored_rows(k0)) return fail(DEMCMC_EINVAL, "n_rows %lld != the %lld stored rows (iterations run / store_every + n_initial)", (long long)n_rows, (long long)stored_rows(k0));
@@ -415,7 +425,7 @@ static int multi_history_out(demcmc_handle *p, double *samples, double *lp, uint
             if (rc) break;
             if (be::set_device(k->cfg.device) ||
                 (stored_rows(k) > 0 && (k->n0 == 0 || k->has_history) &&
-                 be::launch_history_by_id(k->hist_theta, k->hist_w, k->hist_acc, k->hist_id, stored_rows(k), 0, n_rows, (int32_t)k->P, (int32_t)d, 0, ds, lp_written ? dl : nullptr, da, (int32_t)Pt)) ||
+                 be::launch_history_by_id(k->hist_theta, ll_col ? k->hist_ll : k->hist_w, k->hist_acc, k->hist_id, stored_rows(k), 0, n_rows, (int32_t)k->P, (int32_t)d, 0, ds, lp_written ? dl : nullptr, da, (int32_t)Pt)) ||
                 be::sync()) rc = DEMCMC_ECUDA;
         }
         if (!rc && be::set_device(k0->cfg.device)) rc = DEMCMC_ECUDA;
@@ -606,7 +616,8 @@ int demcmc_destroy(demcmc_handle *h)
     if (h->custom_mod) be::custom_unload(h->custom_mod);
     void *ptrs[] = { h->hist_theta, h->hist_w, h->hist_id, h->hist_acc, h->hist_pos, h->scr_theta, h->scr_w, h->scr_id, h->scr_acc,
                      h->prop_theta, h->prop_prior, h->prop_adj, h->prop_msq, h->prop_inb, h->ll_acc, h->ll_q, h->base_th, h->base_cw, h->base_tot, h->ll_part, h->d_lo, h->d_hi, h->d_blocks,
-                     h->plan_recs, h->d_picks, h->d_stage, h->d_stage_recv, h->d_mig_log, h->tr_theta, h->tr_w, h->tr_adj, h->tr_xdot, h->tr_acc, h->flush_buf };
+                     h->plan_recs, h->d_picks, h->d_stage, h->d_stage_recv, h->d_mig_log, h->tr_theta, h->tr_w, h->tr_adj, h->tr_xdot, h->tr_acc, h->flush_buf,
+                     h->d_temp, h->hist_ll, h->scr_ll };
     for (void *e : h->tev) be::tevent_destroy(e);
     for (void *p : ptrs) be::dfree(p);
     for (auto &u : h->ring) { be::hfree_pinned(u.h_blk); be::dfree(u.d_blk); be::event_destroy(u.copied); }
@@ -632,7 +643,7 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
     if (!h || !m || !m->prior) return fail(DEMCMC_EINVAL, "null argument");
     if (h->multi) {
         const int rc = for_kids(h, [&](demcmc_handle *k, int) { return demcmc_set_model(k, m); });
-        if (!rc) { h->has_model = true; h->dmodel = h->kids[0]->dmodel; }
+        if (!rc) { h->has_model = true; h->dmodel = h->kids[0]->dmodel; h->prior_kind = h->kids[0]->prior_kind; }
         return rc;
     }
     if (m->d != h->d) return fail(DEMCMC_EINVAL, "model.d %d != config.d %d", m->d, h->d);
@@ -684,6 +695,8 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         if (m->n_sim < 16 || m->n_sim > DEMCMC_SIM_MAX_DRAWS) return fail(DEMCMC_EINVAL, "n_sim must be in [16, %d], got %d", DEMCMC_SIM_MAX_DRAWS, m->n_sim);
         if (!(m->sim_floor > 0.0)) return fail(DEMCMC_EINVAL, "sim_floor must be > 0, got %g", m->sim_floor);
         if (m->data_on_device) return fail(DEMCMC_EINVAL, "a simulated likelihood checks its data on the host: pass host data, not device pointers");
+        for (double t : h->temper)
+            if (t != 1.0) return fail(DEMCMC_EINVAL, "a simulated likelihood cannot be tempered (t = %g): a power of a noisy estimate breaks the pseudo-marginal target", t);
         want_d = m->d;
         break;
     default: return fail(DEMCMC_EUNSUPPORTED, "no registered kernel for model kind %d: arbitrary closures are not supported and there is no CPU fallback", m->kind);
@@ -702,6 +715,8 @@ int demcmc_set_model(demcmc_handle *h, const demcmc_model *m)
         if (pr[k].kind == PRIOR_NORMAL_REF) D.prior_has_ref = 1;
         prior_constants(pr[k]);
     }
+    h->prior_kind.resize(m->d);
+    for (int k = 0; k < m->d; ++k) h->prior_kind[k] = m->prior[k].kind;
     D.prior = (const Prior *)upload(pr.data(), sizeof(Prior) * pr.size(), false);
     if (!D.prior) return fail(DEMCMC_ENOMEM, "prior upload failed");
     const bool dev = m->data_on_device != 0;
@@ -883,6 +898,44 @@ int demcmc_compile_simulator(const char *source, char *log, int64_t log_cap)
     return rc == -2 ? DEMCMC_EUNSUPPORTED : DEMCMC_EINVAL;
 }
 
+int demcmc_set_temperatures(demcmc_handle *h, const double *t, int32_t n)
+{
+    if (!h || !t) return fail(DEMCMC_EINVAL, "null argument");
+    if (n != h->cfg.n_groups) return fail(DEMCMC_EINVAL, "%d temperatures for the %d groups of the job", n, h->cfg.n_groups);
+    for (int32_t g = 0; g < n; ++g)
+        if (!(t[g] >= 0.0 && t[g] <= 1.0)) return fail(DEMCMC_EINVAL, "temperature %g of group %d is not in [0, 1]", t[g], g);
+    if (!be::launch_power_posterior || !be::launch_temper_weights) return fail(DEMCMC_EUNSUPPORTED, "this backend (%s) has no power-posterior kernels", be::name());
+    if (!h->has_model) return fail(DEMCMC_ESTATE, "set_model must come before set_temperatures");
+    if (h->has_state) return fail(DEMCMC_ESTATE, "set_temperatures must come before set_state (the initial weights are tempered)");
+    if (h->cfg.n_groups > 1 && h->cfg.alpha > 0.0)
+        return fail(DEMCMC_EINVAL, "a tempered handle has no migration (it would move particles between temperatures): create it with alpha = 0");
+    if (h->cfg.donors) return fail(DEMCMC_EINVAL, "a tempered handle draws its donors from the current group: sample = resample is not supported");
+    if (h->cfg.update != DEMCMC_UPDATE_MH || h->cfg.fitness != DEMCMC_FITNESS_POSTERIOR)
+        return fail(DEMCMC_EINVAL, "temperatures temper a posterior: update must be mh_update! and fitness compute_posterior!");
+    if (h->dmodel.kind == M_SIMULATED)
+        for (int32_t g = 0; g < n; ++g)
+            if (t[g] != 1.0) return fail(DEMCMC_EINVAL, "a simulated likelihood cannot be tempered (t = %g): a power of a noisy estimate breaks the pseudo-marginal target", t[g]);
+    if (h->multi) {
+        const int rc = for_kids(h, [&](demcmc_handle *k, int) { return demcmc_set_temperatures(k, t, n); }, false);
+        if (!rc) h->temper.assign(t, t + n);
+        return rc;
+    }
+    BE(be::set_device(h->cfg.device));
+    const size_t P = h->P;
+    if (!h->d_temp) h->d_temp = (double *)be::dmalloc(sizeof(double) * n);
+    if (!h->scr_ll) h->scr_ll = (double *)be::dmalloc(sizeof(double) * h->n_scratch * P);
+    if (h->hist_cap > 0 && !h->hist_ll) {                  // demcmc_set_history came first: its prior rows carry no log-likelihood
+        h->hist_ll = (double *)be::dmalloc(sizeof(double) * h->hist_cap * P);
+        if (h->hist_ll) BE(be::dfill(h->hist_ll, 0xFF, sizeof(double) * h->hist_cap * P));
+    }
+    if (!h->d_temp || !h->scr_ll || (h->hist_cap > 0 && !h->hist_ll)) return fail(DEMCMC_ENOMEM, "log-likelihood rows do not fit on the device");
+    BE(be::h2d(h->d_temp, t, sizeof(double) * n));
+    BE(be::sync());
+    h->temper.assign(t, t + n);
+    h->dcfg.temp = h->d_temp;
+    return 0;
+}
+
 int demcmc_set_history(demcmc_handle *h, const double *rows)
 {
     if (!h || !rows) return fail(DEMCMC_EINVAL, "null argument");
@@ -956,8 +1009,13 @@ int demcmc_set_state(demcmc_handle *h, const double *theta, const int32_t *ids)
     BE(be::h2d(r.id, idv.data(), sizeof(int32_t) * P));
     BE(be::dzero(r.acc, P));
     BE(be::sync());
-    // init_particle (utilities.jl:13-22): weight through evaluate_fitness!
-    BE(be::launch_eval(h->dcfg, h->dmodel, r.theta, (int64_t)P, nullptr, nullptr, r.w, h->ll_part));
+    // init_particle (utilities.jl:13-22): weight through evaluate_fitness!.  A tempered handle keeps the untempered
+    // log-likelihood in the row and forms the tempered weight from it and the prior (prop_prior is free scratch here)
+    if (r.ll) {
+        BE(be::launch_eval(h->dcfg, h->dmodel, r.theta, (int64_t)P, r.ll, h->prop_prior, nullptr, h->ll_part));
+        BE(be::launch_temper_weights(h->dcfg, h->prop_prior, r.ll, (int64_t)P, r.w));
+    } else
+        BE(be::launch_eval(h->dcfg, h->dmodel, r.theta, (int64_t)P, nullptr, nullptr, r.w, h->ll_part));
     BE(be::sync());
     h->has_state = true;
     return 0;
@@ -1012,6 +1070,9 @@ static int load_tape(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter, 
     if (cfg.kappa != 1.0 && !tape->keep) return fail(DEMCMC_EINVAL, "kappa != 1 needs tape.keep");
     if (Gt > 1 && (!tape->mig_n || !tape->mig_groups || !tape->mig_pick_u)) return fail(DEMCMC_EINVAL, "tape misses the migration arrays");
     if (cfg.donors && !tape->idx_row) return fail(DEMCMC_EINVAL, "sample = resample needs tape.idx_row");
+    if (!h->temper.empty() && Gt > 1)
+        for (int64_t it = 0; it < n_iter; ++it)
+            if (tape->mig_n[it] > 0) return fail(DEMCMC_EINVAL, "tape iteration %lld migrates: a tempered handle has no migration (it would move particles between temperatures)", (long long)it);
     auto slice = [&](const auto *src, size_t per) {           // [S][Pt][per] -> [S][P][per]
         std::vector<std::remove_const_t<std::remove_reference_t<decltype(*src)>>> v((size_t)S * P * per);
         for (int64_t s = 0; s < S; ++s) std::copy_n(src + ((size_t)s * Pt + pbeg) * per, (size_t)P * per, v.data() + (size_t)s * P * per);
@@ -1148,6 +1209,7 @@ static void fill_sweep_contexts(demcmc_handle *h, const RunCall &call, Chunk &ck
         // resample: donors are (row, id) cells of the rows stored before this iteration (crossover.jl:115)
         ctx.hist_theta = ghist ? h->ghist_theta : h->hist_theta; ctx.hist_pos = ghist ? h->ghist_pos : h->hist_pos; ctx.donor_rows = stored_rows(h, itg);
         ctx.next_pos = (stored && h->hist_pos && !ghist) ? h->hist_pos + (size_t)hist_row * P : nullptr;
+        ctx.cur_ll = cur.ll; ctx.next_ll = next.ll;
         if (h->tr_sweeps) {
             ctx.tr_theta = h->tr_theta + (size_t)s_local * P * d; ctx.tr_w = h->tr_w + (size_t)s_local * P;
             ctx.tr_adj = h->tr_adj + (size_t)s_local * P; ctx.tr_acc = h->tr_acc + (size_t)s_local * P;
@@ -1469,10 +1531,10 @@ int demcmc_replay(demcmc_handle *h, const demcmc_tape *tape, int64_t n_iter)
     return (h && h->multi) ? multi_run(h, tape, n_iter) : run_impl(h, tape, n_iter);
 }
 
-static int history_out(demcmc_handle *h, double *samples, double *lp, uint8_t *accept, int64_t n_rows)
+static int history_out(demcmc_handle *h, double *samples, double *lp, uint8_t *accept, int64_t n_rows, bool ll_col = false)
 {
     if (!h) return fail(DEMCMC_EINVAL, "null handle");
-    if (h->multi) return multi_history_out(h, samples, lp, accept, n_rows);
+    if (h->multi) return multi_history_out(h, samples, lp, accept, n_rows, ll_col);
     if (n_rows != stored_rows(h)) return fail(DEMCMC_EINVAL, "n_rows %lld != the %lld stored rows (iterations run / store_every + n_initial)", (long long)n_rows, (long long)stored_rows(h));
     if (h->n_ranks > 1) return fail(DEMCMC_EUNSUPPORTED, "by-id history of a sharded job: gather demcmc_get_history_by_slot on the host");
     BE(be::set_device(h->cfg.device));
@@ -1490,7 +1552,7 @@ static int history_out(demcmc_handle *h, double *samples, double *lp, uint8_t *a
         if (dl && be::dzero(dl, sizeof(double) * n_rows * P)) rc = DEMCMC_ECUDA;
         if (da && be::dzero(da, n_rows * P)) rc = DEMCMC_ECUDA;
         if (!rc && stored_rows(h) > 0 && (n0 == 0 || h->has_history) &&
-            be::launch_history_by_id(h->hist_theta, h->hist_w, h->hist_acc, h->hist_id, stored_rows(h), 0, n_rows, (int32_t)P, (int32_t)d,
+            be::launch_history_by_id(h->hist_theta, ll_col ? h->hist_ll : h->hist_w, h->hist_acc, h->hist_id, stored_rows(h), 0, n_rows, (int32_t)P, (int32_t)d,
                                      h->cfg.group_begin * h->cfg.Np, ds, lp_written ? dl : nullptr, da)) rc = DEMCMC_ECUDA;
         if (!rc && ds && be::d2h(samples, ds, sizeof(double) * n_rows * P * d)) rc = DEMCMC_ECUDA;
         if (!rc && dl && be::d2h(lp, dl, sizeof(double) * n_rows * P)) rc = DEMCMC_ECUDA;
@@ -1504,6 +1566,16 @@ static int history_out(demcmc_handle *h, double *samples, double *lp, uint8_t *a
 int demcmc_get_samples(demcmc_handle *h, double *out, int64_t n_rows) { return out ? history_out(h, out, nullptr, nullptr, n_rows) : fail(DEMCMC_EINVAL, "null out"); }
 int demcmc_get_accept(demcmc_handle *h, uint8_t *out, int64_t n_rows) { return out ? history_out(h, nullptr, nullptr, out, n_rows) : fail(DEMCMC_EINVAL, "null out"); }
 int demcmc_get_lp(demcmc_handle *h, double *out, int64_t n_rows) { return out ? history_out(h, nullptr, out, nullptr, n_rows) : fail(DEMCMC_EINVAL, "null out"); }
+int demcmc_get_loglike(demcmc_handle *h, double *out, int64_t n_rows)
+{
+    if (!h || !out) return fail(DEMCMC_EINVAL, "null argument");
+    if (h->temper.empty()) return fail(DEMCMC_ESTATE, "no stored log-likelihoods: the handle was not tempered (demcmc_set_temperatures)");
+    if (int rc = history_out(h, nullptr, out, nullptr, n_rows, true)) return rc;
+    const int64_t n0 = std::min<int64_t>(h->n0, n_rows);
+    for (size_t p = 0; p < (size_t)h->P; ++p)                  // the prior rows carry none (row fastest, as demcmc_get_lp)
+        for (int64_t r = 0; r < n0; ++r) out[p * n_rows + r] = NAN;
+    return 0;
+}
 
 int demcmc_get_moments(demcmc_handle *h, int64_t row0, int64_t n_rows, int64_t *count, double *mean, double *m2)
 {
@@ -1557,25 +1629,24 @@ static bool diag_finish(const std::vector<std::array<double, 3>> &head, const st
     return done;
 }
 
-int demcmc_get_diagnostics(demcmc_handle *h, int64_t row0, int64_t n_rows, double *rhat, double *ess)
+// split-R-hat and ESS over rows [row0, row0 + n_rows) with the ids [id_base, id_base + P_ids) as chains, of the d parameters
+// (ll: of the stored untempered log-likelihood, d = 1).  The range has been checked.
+static int diag_ids(demcmc_handle *h, bool ll, int64_t row0, int64_t n_rows, int32_t id_base, int32_t P_ids, int d, double *rhat, double *ess)
 {
-    if (!h || (!rhat && !ess)) return fail(DEMCMC_EINVAL, "null argument");
     demcmc_handle *h0 = h->multi ? h->kids[0] : h;
-    if (row0 < 0 || n_rows < 4 || row0 + n_rows > stored_rows(h0)) return fail(DEMCMC_EINVAL, "row range [%lld, %lld) outside the %lld stored rows (at least 4 rows)", (long long)row0, (long long)(row0 + n_rows), (long long)stored_rows(h0));
     const int64_t nh = n_rows / 2;
     if (nh > be::diag_max_half()) return fail(DEMCMC_EUNSUPPORTED, "diagnostics over more than %d stored rows per call: thin the run or pass a sub-range", 2 * be::diag_max_half());
     // the autocovariances come in batches of lags (an even number: Geyer's sequence sums pairs); a batch is computed only
     // while some parameter's sequence is still positive at the last lag of the one before it
     // (DEMCMC_DIAG_LAGS: test switch, a smaller batch so that short chains walk through several of them)
     const char *lag_env = getenv("DEMCMC_DIAG_LAGS");
-    const int d = h->d, lag_step = std::max(2, std::min(be::diag_max_lags(), lag_env ? atoi(lag_env) : be::diag_max_lags()) & ~1), n_lag = (int)std::min<int64_t>(nh, lag_step);
+    const int lag_step = std::max(2, std::min(be::diag_max_lags(), lag_env ? atoi(lag_env) : be::diag_max_lags()) & ~1), n_lag = (int)std::min<int64_t>(nh, lag_step);
     const size_t na = (size_t)d * (3 + n_lag);
     std::vector<demcmc_handle *> leaves = h->multi ? h->kids : std::vector<demcmc_handle *>{ h };
-    const int32_t Pt = (int32_t)h->P, id_base = h->multi ? 0 : h->cfg.group_begin * h->cfg.Np;
     // ids migrate between the shards of a job: every shard marks, in ONE map on the first device, where the ids it holds
     // sit at every row; the first device then gathers every chain through the map (peer access) and reduces
     BE(be::set_device(h0->cfg.device));
-    int32_t *pos = (int32_t *)be::dmalloc_shared(sizeof(int32_t) * (size_t)n_rows * Pt);
+    int32_t *pos = (int32_t *)be::dmalloc_shared(sizeof(int32_t) * (size_t)n_rows * P_ids);
     double *agg = (double *)be::dmalloc(sizeof(double) * na);
     std::vector<double> total(na);
     int rc = (!pos || !agg) ? fail(DEMCMC_ENOMEM, "diagnostics staging") : 0;
@@ -1584,27 +1655,133 @@ int demcmc_get_diagnostics(demcmc_handle *h, int64_t row0, int64_t n_rows, doubl
     sh.n = (int32_t)leaves.size(); sh.P_local = (int32_t)h0->P;
     for (size_t i = 0; i < leaves.size() && !rc; ++i) {
         demcmc_handle *k = leaves[i];
-        sh.theta[i] = k->hist_theta;
+        sh.theta[i] = ll ? k->hist_ll : k->hist_theta;
         if (be::set_device(k->cfg.device) ||
-            be::launch_diag_pos(k->hist_id, row0, n_rows, (int32_t)k->P, id_base, Pt, h->multi ? k->cfg.group_begin * k->cfg.Np : 0, pos) || be::sync())
+            be::launch_diag_pos(k->hist_id, row0, n_rows, (int32_t)k->P, id_base, P_ids, h->multi ? k->cfg.group_begin * k->cfg.Np : 0, pos) || be::sync())
             rc = fail(DEMCMC_ECUDA, "diagnostics: %s", be::last_error());
     }
     std::vector<std::array<double, 3>> head(d);
     std::vector<std::vector<double>> acov(d);
     for (int64_t lag0 = 0; lag0 < nh && !rc; lag0 += lag_step) {
         const int nl = (int)std::min<int64_t>(lag_step, nh - lag0);
-        if (be::set_device(h0->cfg.device) || be::launch_diag_aggregates(sh, pos, row0, n_rows, Pt, d, (int32_t)lag0, nl, agg) ||
+        if (be::set_device(h0->cfg.device) || be::launch_diag_aggregates(sh, pos, row0, n_rows, P_ids, d, (int32_t)lag0, nl, agg) ||
             be::d2h(total.data(), agg, sizeof(double) * (size_t)d * (3 + nl))) { rc = fail(DEMCMC_ECUDA, "diagnostics: %s", be::last_error()); break; }
         for (int k = 0; k < d; ++k) {
             const double *a = total.data() + (size_t)k * (3 + nl);
             if (lag0 == 0) head[k] = { a[0], a[1], a[2] };
             acov[k].insert(acov[k].end(), a + 3, a + 3 + nl);
         }
-        if (diag_finish(head, acov, nh, 2 * (int64_t)Pt, rhat, ess) || !ess) break;
+        if (diag_finish(head, acov, nh, 2 * (int64_t)P_ids, rhat, ess) || !ess) break;
     }
     be::set_device(h0->cfg.device);
     be::dfree_shared(pos); be::dfree(agg);
     return rc;
+}
+
+int demcmc_get_diagnostics(demcmc_handle *h, int64_t row0, int64_t n_rows, double *rhat, double *ess)
+{
+    if (!h || (!rhat && !ess)) return fail(DEMCMC_EINVAL, "null argument");
+    demcmc_handle *h0 = h->multi ? h->kids[0] : h;
+    if (row0 < 0 || n_rows < 4 || row0 + n_rows > stored_rows(h0)) return fail(DEMCMC_EINVAL, "row range [%lld, %lld) outside the %lld stored rows (at least 4 rows)", (long long)row0, (long long)(row0 + n_rows), (long long)stored_rows(h0));
+    return diag_ids(h, false, row0, n_rows, h->multi ? 0 : h->cfg.group_begin * h->cfg.Np, (int32_t)h->P, h->d, rhat, ess);
+}
+
+// ---- power posteriors: thermodynamic integration and stepping-stone sampling over the rungs of a tempered handle ----
+int demcmc_power_posterior(demcmc_handle *h, int64_t row0, int64_t n_rows, int32_t cap, demcmc_evidence *out, double *t, double *mean_ll,
+                           double *var_ll, double *ess_ll, double *rhat_ll, double *log_ratio)
+{
+    if (!h || !out) return fail(DEMCMC_EINVAL, "null argument");
+    if (h->temper.empty()) return fail(DEMCMC_ESTATE, "no temperatures: call demcmc_set_temperatures before demcmc_set_state");
+    if (!h->multi && h->G_local != h->cfg.n_groups) return fail(DEMCMC_EUNSUPPORTED, "power posterior of a sharded job: gather demcmc_get_history_by_slot on the host");
+    demcmc_handle *h0 = h->multi ? h->kids[0] : h;
+    if (!h0->has_state) return fail(DEMCMC_ESTATE, "no state");
+    const int Gt = h->cfg.n_groups, Np = h->cfg.Np;
+    // the rungs: maximal runs of groups at one temperature, increasing from 0 to 1
+    std::vector<int> first;                                  // first group of each rung, then Gt
+    for (int g = 0; g < Gt; ++g) if (g == 0 || h->temper[g] != h->temper[g - 1]) first.push_back(g);
+    const int K = (int)first.size();
+    first.push_back(Gt);
+    std::vector<double> T(K);
+    for (int k = 0; k < K; ++k) T[k] = h->temper[first[k]];
+    bool ladder = K >= 2 && T[0] == 0.0 && T[K - 1] == 1.0;
+    for (int k = 1; k < K; ++k) ladder = ladder && T[k] > T[k - 1];
+    if (!ladder) return fail(DEMCMC_EINVAL, "the rung temperatures must increase in group order from 0 to 1 (%d rungs, first %g, last %g)", K, T[0], T[K - 1]);
+    if (cap < K) return fail(DEMCMC_EINVAL, "cap %d < the %d rungs", cap, K);
+    if (row0 < h0->n0) return fail(DEMCMC_EINVAL, "row0 %lld < n_initial %lld: the prior rows carry no log-likelihood", (long long)row0, (long long)h0->n0);
+    if (n_rows < 4 || row0 + n_rows > stored_rows(h0)) return fail(DEMCMC_EINVAL, "row range [%lld, %lld) outside the %lld stored rows (at least 4 rows)", (long long)row0, (long long)(row0 + n_rows), (long long)stored_rows(h0));
+    for (int k = 0; k < h->d; ++k)
+        if (h->prior_kind[k] == DEMCMC_PRIOR_FLAT && (std::isinf(h0->lo[k]) || std::isinf(h0->hi[k])))
+            return fail(DEMCMC_EINVAL, "parameter %d has a flat prior on an unbounded range: the t = 0 rung would sample an improper prior", k);
+    std::vector<int> rung_of(Gt);
+    for (int k = 0; k < K; ++k) for (int g = first[k]; g < first[k + 1]; ++g) rung_of[g] = k;
+    // per-slice partials of every group, each shard on its own rows
+    const int64_t n_sl = (n_rows + PP_ROWS - 1) / PP_ROWS;
+    std::vector<double> part((size_t)Gt * n_sl * PP_OUT);
+    std::vector<demcmc_handle *> leaves = h->multi ? h->kids : std::vector<demcmc_handle *>{ h };
+    for (demcmc_handle *k : leaves) {
+        PPDelta dl;
+        memset(&dl, 0, sizeof dl);
+        for (int gl = 0; gl < k->G_local; ++gl) { const int r = rung_of[k->cfg.group_begin + gl]; dl.v[gl] = r + 1 < K ? T[r + 1] - T[r] : 0.0; }
+        BE(be::set_device(k->cfg.device));
+        const size_t nb = (size_t)k->G_local * n_sl * PP_OUT;
+        double *dpart = (double *)be::dmalloc(sizeof(double) * nb);
+        if (!dpart) return fail(DEMCMC_ENOMEM, "power-posterior staging");
+        const int rc = be::launch_power_posterior(k->hist_ll, row0, n_rows, (int32_t)k->P, Np, k->G_local, dl, dpart) ||
+                       be::d2h(part.data() + (size_t)k->cfg.group_begin * n_sl * PP_OUT, dpart, sizeof(double) * nb);
+        be::dfree(dpart);
+        if (rc) return fail(DEMCMC_ECUDA, "power posterior: %s", be::last_error());
+    }
+    // merge in rung, group and slice order: (count, mean, m2) by Chan's update, the exponential sums rescaled to the rung max
+    std::vector<double> mean(K), var(K), lr(K, NAN), ve(K, NAN), me(K, NAN), ess(K), rhat(K);
+    for (int k = 0; k < K; ++k) {
+        double c = 0.0, mu = 0.0, m2 = 0.0, mx = -INFINITY;
+        for (int g = first[k]; g < first[k + 1]; ++g)
+            for (int64_t sl = 0; sl < n_sl; ++sl) {
+                const double *o = part.data() + ((size_t)g * n_sl + sl) * PP_OUT;
+                const double cb = o[0], cn = c + cb, dl = o[1] - mu;
+                mu += dl * (cb / cn);
+                m2 += o[2] + dl * dl * (c * cb / cn);
+                c = cn;
+                mx = std::max(mx, o[3]);
+            }
+        mean[k] = mu; var[k] = m2 / (c - 1.0);
+        if (k + 1 < K) {
+            const double dl = T[k + 1] - T[k];
+            double s1 = 0.0, s2 = 0.0;
+            for (int g = first[k]; g < first[k + 1]; ++g)
+                for (int64_t sl = 0; sl < n_sl; ++sl) {
+                    const double *o = part.data() + ((size_t)g * n_sl + sl) * PP_OUT;
+                    const double f = exp(dl * (o[3] - mx));
+                    s1 += o[4] * f; s2 += o[5] * (f * f);
+                }
+            me[k] = s1 / c;
+            ve[k] = std::max(0.0, (s2 - s1 * me[k]) / (c - 1.0));
+            lr[k] = log(me[k]) + dl * mx;
+        }
+        if (int rc = diag_ids(h, true, row0, n_rows, first[k] * Np, (first[k + 1] - first[k]) * Np, 1, &rhat[k], &ess[k])) return rc;
+    }
+    double ti = 0.0, ti2 = 0.0, ss = 0.0, vti = 0.0, vss = 0.0;
+    for (int k = 0; k + 1 < K; ++k) {
+        const double dl = T[k + 1] - T[k];
+        ti += dl * (mean[k] + mean[k + 1]) / 2.0;
+        ti2 += dl * dl * (var[k + 1] - var[k]) / 12.0;
+        ss += lr[k];
+        vss += ve[k] / (ess[k] * me[k] * me[k]);
+    }
+    for (int k = 0; k < K; ++k) {                          // trapezoid weights
+        const double w = ((k > 0 ? T[k] - T[k - 1] : 0.0) + (k + 1 < K ? T[k + 1] - T[k] : 0.0)) / 2.0;
+        vti += w * w * var[k] / ess[k];
+    }
+    out->n_rungs = K; out->log_z_ti = ti; out->log_z_ti2 = ti - ti2; out->log_z_ss = ss; out->se_ti = sqrt(vti); out->se_ss = sqrt(vss);
+    for (int k = 0; k < K; ++k) {
+        if (t) t[k] = T[k];
+        if (mean_ll) mean_ll[k] = mean[k];
+        if (var_ll) var_ll[k] = var[k];
+        if (ess_ll) ess_ll[k] = ess[k];
+        if (rhat_ll) rhat_ll[k] = rhat[k];
+        if (log_ratio) log_ratio[k] = lr[k];
+    }
+    return 0;
 }
 
 int demcmc_get_chains(demcmc_handle *h, int64_t row0, int64_t n_rows, double *out)
@@ -1753,6 +1930,7 @@ int demcmc_set_weights(demcmc_handle *h, const double *w)
 {
     if (!h || !w) return fail(DEMCMC_EINVAL, "null argument");
     if (!h->has_state) return fail(DEMCMC_ESTATE, "set_state must come before set_weights");
+    if (!h->temper.empty()) return fail(DEMCMC_EINVAL, "a tempered handle keeps each particle's untempered log-likelihood, which saved weights do not carry: re-evaluate with demcmc_set_state");
     if (h->multi) return for_kids(h, [&](demcmc_handle *k, int) { return demcmc_set_weights(k, w + (size_t)k->cfg.group_begin * k->cfg.Np); }, false);
     BE(be::set_device(h->cfg.device));
     BE(be::h2d(cur_row(h).w, w, sizeof(double) * (size_t)h->P));

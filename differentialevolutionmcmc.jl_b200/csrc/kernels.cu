@@ -495,6 +495,8 @@ __global__ void __launch_bounds__(PA_THREADS) k_propose(ConfigDev cfg, ModelDev 
     if ((threadIdx.x & 31) == 0) { tl_max(tl, TL_P1); if (tl && wi == 0) tl[TL_N] = (unsigned long long)lv.n; }
 }
 
+// TEMPER: the power-posterior terms (a tempered handle); untempered handles launch k_accept<false>, which keeps its registers
+template <bool TEMPER>
 __global__ void __launch_bounds__(PA_THREADS) k_accept(ConfigDev cfg, ModelDev m, Level lv, unsigned long long *tl)
 {
     pdl_launch_dependents();
@@ -503,7 +505,7 @@ __global__ void __launch_bounds__(PA_THREADS) k_accept(ConfigDev cfg, ModelDev m
     if (wi >= lv.n) { pdl_wait(); return; }
     const uint32_t e = (uint32_t)lv.order[wi];
     const SweepCtx ctx = lv.ctxs[e >> LV_SLOT_SHIFT];
-    accept_particle(WarpLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
+    accept_particle<WarpLanes, TEMPER>(WarpLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
     if ((threadIdx.x & 31) == 0) tl_max(tl, TL_A1);
 }
 
@@ -584,7 +586,7 @@ __global__ void __launch_bounds__(PAW_THREADS, MINB) k_propose_wide(ConfigDev cf
     if (threadIdx.x == 0) { tl_max(tl, TL_P1); if (tl && wi == 0) tl[TL_N] = (unsigned long long)lv.n; }
 }
 
-template <int PAW_THREADS, int MINB>
+template <int PAW_THREADS, int MINB, bool TEMPER>
 __global__ void __launch_bounds__(PAW_THREADS, MINB) k_accept_wide(ConfigDev cfg, ModelDev m, Level lv, unsigned long long *tl)
 {
     __shared__ double red[PAW_THREADS / 32];
@@ -594,7 +596,7 @@ __global__ void __launch_bounds__(PAW_THREADS, MINB) k_accept_wide(ConfigDev cfg
     const uint32_t e = (uint32_t)lv.order[blockIdx.x];
     const SweepCtx ctx = lv.ctxs[e >> LV_SLOT_SHIFT];
     const BlockLanes<PAW_THREADS> co = { red, ired, tl, TL_AW };
-    accept_particle(co, cfg, m, ctx, (int)(e & LV_POS_MASK));
+    accept_particle<BlockLanes<PAW_THREADS>, TEMPER>(co, cfg, m, ctx, (int)(e & LV_POS_MASK));
     if (threadIdx.x == 0) tl_max(tl, TL_A1);
 }
 
@@ -911,14 +913,17 @@ int launch_accept(const ConfigDev &cfg, const ModelDev &m, const Level &lv)
     const int blocks = (lv.n * 32 + PA_THREADS - 1) / PA_THREADS;
     if (wide_enabled(cfg) && lv.ctxs) {
         switch (wide_shape() / 10) {
-        case 0: CU(launch_chained(k_accept_wide<256, 4>, dim3(lv.n), dim3(256), 0, cfg, m, lv, tl_slot())); break;
-        default: CU(launch_chained(k_accept_wide<128, 12>, dim3(lv.n), dim3(128), 0, cfg, m, lv, tl_slot())); break;
+        case 0: CU(cfg.temp ? launch_chained(k_accept_wide<256, 4, true>, dim3(lv.n), dim3(256), 0, cfg, m, lv, tl_slot())
+                            : launch_chained(k_accept_wide<256, 4, false>, dim3(lv.n), dim3(256), 0, cfg, m, lv, tl_slot())); break;
+        default: CU(cfg.temp ? launch_chained(k_accept_wide<128, 12, true>, dim3(lv.n), dim3(128), 0, cfg, m, lv, tl_slot())
+                             : launch_chained(k_accept_wide<128, 12, false>, dim3(lv.n), dim3(128), 0, cfg, m, lv, tl_slot())); break;
         }
         LAUNCHED("k_accept_wide");
         if (g_tl_cap > 0) ++g_tl_level;
         return 0;
     }
-    CU(launch_chained(k_accept, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv, tl_slot()));
+    if (cfg.temp) CU(launch_chained(k_accept<true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv, tl_slot()));
+    else CU(launch_chained(k_accept<false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv, tl_slot()));
     LAUNCHED("k_accept");
     if (g_tl_cap > 0) ++g_tl_level;
     return 0;
@@ -1005,7 +1010,7 @@ __device__ __forceinline__ void pointwise_par(const ModelDev &m, const double *t
 struct NoWaitLanes : WarpLanes { __device__ __forceinline__ void dependency_wait() const {} };
 // the whole update of one particle by one warp (small pointwise problems, n_split == 1): C = WarpLanes inside a PDL chain,
 // NoWaitLanes where the caller has done the waiting
-template <int KIND, class C>
+template <int KIND, bool TEMPER, class C>
 __device__ __forceinline__ void fused_update(const C &co, const ConfigDev &cfg, const ModelDev &m, const SweepCtx &ctx, int p)
 {
     const int lane = threadIdx.x & 31;
@@ -1027,10 +1032,11 @@ __device__ __forceinline__ void fused_update(const C &co, const ConfigDev &cfg, 
         if (lane == 0) ctx.ll_part[(size_t)p] = a;               // n_split == 1 on this path
         __syncwarp();
     }
-    accept_particle(NoWaitLanes(), cfg, m, ctx, p);
+    accept_particle<NoWaitLanes, TEMPER>(NoWaitLanes(), cfg, m, ctx, p);
 }
 
-template <int KIND>
+// TEMPER (here, in k_chunk_small and k_accept_wide): as k_accept's
+template <int KIND, bool TEMPER>
 __global__ void __launch_bounds__(PA_THREADS) k_level_fused(ConfigDev cfg, ModelDev m, Level lv)
 {
     pdl_launch_dependents();
@@ -1038,7 +1044,7 @@ __global__ void __launch_bounds__(PA_THREADS) k_level_fused(ConfigDev cfg, Model
     if (wi >= lv.n) { pdl_wait(); return; }
     const uint32_t e = (uint32_t)lv.order[wi];
     const SweepCtx ctx = lv.ctxs[e >> LV_SLOT_SHIFT];
-    fused_update<KIND>(WarpLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
+    fused_update<KIND, TEMPER>(WarpLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
 }
 
 // The reference's own examples (Gaussian_Example.jl: 4 groups x 6 particles, 50 observations) are a handful of warps: a
@@ -1048,7 +1054,7 @@ __global__ void __launch_bounds__(PA_THREADS) k_level_fused(ConfigDev cfg, Model
 constexpr int SC_MAX_LEVELS = 640, SC_MAX_WARPS = 12;       // 12 warps x 168 registers fit one SM
 constexpr int SC_MAX_P = 96;                                // beyond, a level is several rounds of the 12 warps and the level-by-level path (all SMs) wins
 struct SmallChunk { int32_t n_levels; int32_t off[SC_MAX_LEVELS + 1]; };
-template <int KIND>
+template <int KIND, bool TEMPER>
 __global__ void __launch_bounds__(SC_MAX_WARPS * 32, 1) k_chunk_small(const __grid_constant__ ConfigDev cfg, const __grid_constant__ ModelDev m,
                                                                        const int32_t *order, const SweepCtx *ctxs, const __grid_constant__ SmallChunk sc)
 {
@@ -1057,7 +1063,7 @@ __global__ void __launch_bounds__(SC_MAX_WARPS * 32, 1) k_chunk_small(const __gr
         for (int wi = sc.off[L] + warp; wi < sc.off[L + 1]; wi += nw) {
             const uint32_t e = (uint32_t)order[wi];
             const SweepCtx ctx = ctxs[e >> LV_SLOT_SHIFT];
-            fused_update<KIND>(NoWaitLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
+            fused_update<KIND, TEMPER>(NoWaitLanes(), cfg, m, ctx, (int)(e & LV_POS_MASK));
         }
         __syncthreads();
     }
@@ -1080,11 +1086,16 @@ int launch_level_fused(const ConfigDev &cfg, const ModelDev &m, const Level &lv)
     if (!lv.ctxs || !fused_eligible(cfg, m)) return 1;
     const int blocks = (lv.n * 32 + PA_THREADS - 1) / PA_THREADS;
     switch (m.kind) {
-    case M_GAUSSIAN: CU(launch_chained(k_level_fused<M_GAUSSIAN>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
-    case M_LNR: CU(launch_chained(k_level_fused<M_LNR>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
-    case M_LBA: CU(launch_chained(k_level_fused<M_LBA>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
-    case M_BINOMIAL: CU(launch_chained(k_level_fused<M_BINOMIAL>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
-    case M_RASTRIGIN: CU(launch_chained(k_level_fused<M_RASTRIGIN>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
+    case M_GAUSSIAN: CU(cfg.temp ? launch_chained(k_level_fused<M_GAUSSIAN, true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)
+                                : launch_chained(k_level_fused<M_GAUSSIAN, false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
+    case M_LNR: CU(cfg.temp ? launch_chained(k_level_fused<M_LNR, true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)
+                                : launch_chained(k_level_fused<M_LNR, false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
+    case M_LBA: CU(cfg.temp ? launch_chained(k_level_fused<M_LBA, true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)
+                                : launch_chained(k_level_fused<M_LBA, false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
+    case M_BINOMIAL: CU(cfg.temp ? launch_chained(k_level_fused<M_BINOMIAL, true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)
+                                : launch_chained(k_level_fused<M_BINOMIAL, false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
+    case M_RASTRIGIN: CU(cfg.temp ? launch_chained(k_level_fused<M_RASTRIGIN, true>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)
+                                : launch_chained(k_level_fused<M_RASTRIGIN, false>, dim3(blocks), dim3(PA_THREADS), 0, cfg, m, lv)); break;
     default: return 1;
     }
     LAUNCHED("k_level_fused");
@@ -1104,12 +1115,16 @@ int launch_chunk_small(const ConfigDev &cfg, const ModelDev &m, const int32_t *d
     for (int l = 0; l <= n_levels; ++l) sc.off[l] = level_off[l];
     for (int l = 0; l < n_levels; ++l) widest = std::max(widest, level_off[l + 1] - level_off[l]);
     const int threads = 32 * std::min(widest, SC_MAX_WARPS);
+    auto go = [&](auto kernel_untempered, auto kernel_tempered) {
+        if (cfg.temp) kernel_tempered<<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc);
+        else kernel_untempered<<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc);
+    };
     switch (m.kind) {
-    case M_GAUSSIAN: k_chunk_small<M_GAUSSIAN><<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc); break;
-    case M_LNR: k_chunk_small<M_LNR><<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc); break;
-    case M_LBA: k_chunk_small<M_LBA><<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc); break;
-    case M_BINOMIAL: k_chunk_small<M_BINOMIAL><<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc); break;
-    default: k_chunk_small<M_RASTRIGIN><<<1, threads, 0, stream()>>>(cfg, m, d_order, d_ctx, sc); break;
+    case M_GAUSSIAN: go(k_chunk_small<M_GAUSSIAN, false>, k_chunk_small<M_GAUSSIAN, true>); break;
+    case M_LNR: go(k_chunk_small<M_LNR, false>, k_chunk_small<M_LNR, true>); break;
+    case M_LBA: go(k_chunk_small<M_LBA, false>, k_chunk_small<M_LBA, true>); break;
+    case M_BINOMIAL: go(k_chunk_small<M_BINOMIAL, false>, k_chunk_small<M_BINOMIAL, true>); break;
+    default: go(k_chunk_small<M_RASTRIGIN, false>, k_chunk_small<M_RASTRIGIN, true>); break;
     }
     LAUNCHED("k_chunk_small");
     if (g_tl_cap > 0) g_tl_level += n_levels;
@@ -1748,7 +1763,8 @@ static size_t pk_smem_bytes(int nj)
     return sizeof(double) * ((size_t)8 * PK_STAGES * nj * 64 + 2 * pk_bbuf_doubles(nj)) + sizeof(uint64_t) * (8 * PK_STAGES + 6);
 }
 
-template <bool TL>
+// TEMPER: as k_accept's (the untempered instantiations keep the registers, and the spills, they had before tempering)
+template <bool TL, bool TEMPER>
 __global__ void __launch_bounds__(PK_THREADS, 1) k_chunk_persist(const __grid_constant__ ConfigDev cfg, const __grid_constant__ ModelDev m,
                                                                  const __grid_constant__ PChunk ck)
 {
@@ -1896,7 +1912,7 @@ __global__ void __launch_bounds__(PK_THREADS, 1) k_chunk_persist(const __grid_co
             FlagLanes co;
             unsigned long long *tl = (TL && ck.tl) ? ck.tl + (size_t)L * PT_WORDS : nullptr;
             co.w = { ck.xdot_done + pl.tile_base + tile, xd_tile_ctas(pl.g, tile) * 4 * m.n_ksplit, nullptr, 0, tl, PT_AW0, -1, 0ull };
-            accept_particle(co, cfg, m, ctx, (int)(e & LV_POS_MASK));
+            accept_particle<FlagLanes, TEMPER>(co, cfg, m, ctx, (int)(e & LV_POS_MASK));
             const unsigned long long ta1 = (TL && tl) ? gtime() : 0ull;
             arrive(ck.acc_done + L);
             if (TL && tl && lane == 0) {
@@ -2071,8 +2087,10 @@ int launch_chunk_persist(const ConfigDev &cfg, const ModelDev &m, const int32_t 
     static bool attr_set[64] = { false };
     const size_t smem = pk_smem_bytes(m.ssd_nj);
     if (!attr_set[g_dev]) {
-        CU(cudaFuncSetAttribute(k_chunk_persist<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
-        CU(cudaFuncSetAttribute(k_chunk_persist<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
+        CU(cudaFuncSetAttribute(k_chunk_persist<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
+        CU(cudaFuncSetAttribute(k_chunk_persist<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
+        CU(cudaFuncSetAttribute(k_chunk_persist<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
+        CU(cudaFuncSetAttribute(k_chunk_persist<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pk_smem_bytes(SSD_NJ)));
         attr_set[g_dev] = true;
     }
     // a cooperative launch: CUDA itself guarantees (or refuses) that all CTAs are resident at once,
@@ -2083,7 +2101,8 @@ int launch_chunk_persist(const ConfigDev &cfg, const ModelDev &m, const int32_t 
     at[0].id = cudaLaunchAttributeCooperative;
     at[0].val.cooperative = 1;
     lc.attrs = at; lc.numAttrs = 1;
-    const cudaError_t le = ck.tl ? cudaLaunchKernelEx(&lc, k_chunk_persist<true>, cfg, m, ck) : cudaLaunchKernelEx(&lc, k_chunk_persist<false>, cfg, m, ck);
+    const cudaError_t le = cfg.temp ? (ck.tl ? cudaLaunchKernelEx(&lc, k_chunk_persist<true, true>, cfg, m, ck) : cudaLaunchKernelEx(&lc, k_chunk_persist<false, true>, cfg, m, ck))
+                                    : (ck.tl ? cudaLaunchKernelEx(&lc, k_chunk_persist<true, false>, cfg, m, ck) : cudaLaunchKernelEx(&lc, k_chunk_persist<false, false>, cfg, m, ck));
     if (le == cudaErrorCooperativeLaunchTooLarge) { (void)cudaGetLastError(); return 1; }   // not all resident here: level by level
     if (le != cudaSuccess) return cu_fail(le, "k_chunk_persist");
     LAUNCHED("k_chunk_persist");
@@ -3676,6 +3695,75 @@ int launch_diag_aggregates(const DiagShards &sh, const int32_t *pos, int64_t row
     k_diag_merge<<<(unsigned)(((int64_t)d * (3 + n_lag) + 255) / 256), 256, 0, stream()>>>(part, d, n_lag, agg);
     LAUNCHED("k_diag_merge");
     dfree(part);
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// power posteriors (demcmc_power_posterior): the per-slice partials of the stored untempered log-likelihoods
+// ------------------------------------------------------------------------------------------------
+constexpr int PP_THREADS = 256;
+// sum and max over the block in a fixed order (lanes by the xor tree, then the warps in order), the same value to every thread
+__device__ __forceinline__ void pp_block_reduce(double &s, double &mx, double *red)
+{
+    for (int o = 16; o > 0; o >>= 1) { s += __shfl_xor_sync(0xffffffffu, s, o); mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o)); }
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) { red[2 * (threadIdx.x >> 5)] = s; red[2 * (threadIdx.x >> 5) + 1] = mx; }
+    __syncthreads();
+    s = 0.0; mx = -inf();
+    for (int w = 0; w < PP_THREADS / 32; ++w) { s += red[2 * w]; mx = fmax(mx, red[2 * w + 1]); }
+}
+// one block per (slice, local group): rows [row0 + slice * PP_ROWS, ...) of the group's Np positions.  Two passes over the
+// slice: count, sum and max; then the squared deviations from the slice mean and the exponentials shifted by the slice max.
+// (Without migration a particle never leaves its group, so the positions of a group hold the group's ids at every row.)
+__global__ void __launch_bounds__(PP_THREADS) k_power_posterior(const double *ll, int64_t row0, int64_t n_rows, int P, int Np,
+                                                                const PPDelta delta, double *part /* [G_local][n_slices][PP_OUT] */)
+{
+    __shared__ double red[2 * (PP_THREADS / 32)];
+    const int s = blockIdx.x, g = blockIdx.y, n_slices = gridDim.x;
+    const int64_t r0 = row0 + (int64_t)s * PP_ROWS, nr = min((int64_t)PP_ROWS, row0 + n_rows - r0), n = nr * Np;
+    const double dl = delta.v[g];
+    auto at = [&](int64_t e) { const int64_t r = e / Np; return ll[(r0 + r) * P + (size_t)g * Np + (e - r * Np)]; };
+    double sum = 0.0, mx = -inf();
+    for (int64_t e = threadIdx.x; e < n; e += PP_THREADS) { const double v = at(e); sum += v; mx = fmax(mx, v); }
+    pp_block_reduce(sum, mx, red);
+    const double mean = sum / (double)n;
+    double m2 = 0.0, e1 = 0.0, e2 = 0.0;
+    for (int64_t e = threadIdx.x; e < n; e += PP_THREADS) {
+        const double v = at(e), dv = v - mean, x = exp(dl * (v - mx));
+        m2 += dv * dv; e1 += x; e2 += x * x;
+    }
+    double unused = -inf();
+    pp_block_reduce(m2, unused, red);
+    unused = -inf();
+    pp_block_reduce(e1, unused, red);
+    unused = -inf();
+    pp_block_reduce(e2, unused, red);
+    if (threadIdx.x == 0) {
+        double *o = part + ((size_t)g * n_slices + s) * PP_OUT;
+        o[0] = (double)n; o[1] = mean; o[2] = m2; o[3] = mx; o[4] = e1; o[5] = e2;
+    }
+}
+__global__ void __launch_bounds__(256) k_temper_weights(ConfigDev cfg, const double *prior, const double *ll, int64_t n, double *w)
+{
+    const int64_t p = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (p >= n) return;
+    const double pr = prior[p];
+    w[p] = pr == -inf() ? -inf() : add(pr, tempered_ll(cfg, cfg.group_begin + (int)(p / cfg.Np), ll[p]));
+}
+int launch_temper_weights(const ConfigDev &cfg, const double *prior, const double *ll, int64_t n, double *w)
+{
+    if (n <= 0) return 0;
+    k_temper_weights<<<(unsigned)((n + 255) / 256), 256, 0, stream()>>>(cfg, prior, ll, n, w);
+    LAUNCHED("k_temper_weights");
+    return 0;
+}
+int launch_power_posterior(const double *ll_rows, int64_t row0, int64_t n_rows, int32_t P_local, int32_t Np, int32_t G_local,
+                           const PPDelta &delta, double *part)
+{
+    const int64_t n_slices = (n_rows + PP_ROWS - 1) / PP_ROWS;
+    if (n_rows < 1 || G_local < 1 || G_local > MAX_MIG || n_slices > INT32_MAX) { g_be_err = "power posterior: bad row range or group count"; return -1; }
+    k_power_posterior<<<dim3((unsigned)n_slices, (unsigned)G_local), PP_THREADS, 0, stream()>>>(ll_rows, row0, n_rows, P_local, Np, delta, part);
+    LAUNCHED("k_power_posterior");
     return 0;
 }
 

@@ -363,6 +363,36 @@ class Handle:
         check(_ffi.lib().demcmc_loo(self._h, ptr(th, _dp), th.shape[0], *(ptr(a, _dp) for a in out)))
         return tuple(out)
 
+    # ---- power posteriors ----------------------------------------------------------------------
+    def set_temperatures(self, t):
+        """Temper every group of the job: t[n_groups] in [0, 1]; a group's weights become prior + t * loglike
+        (demcmc_set_temperatures).  After set_model, before set_state."""
+        a = f8(t).reshape(-1)
+        self._temperatures = a
+        check(_ffi.lib().demcmc_set_temperatures(self._h, ptr(a, _dp), a.size))
+
+    def loglike(self):
+        """The stored untempered log-likelihoods of a tempered handle, in the layout of lp(): shape (P, n_rows); the
+        n_initial prior rows are NaN (demcmc_get_loglike)."""
+        out = np.zeros((self.P, self.n_rows))
+        check(_ffi.lib().demcmc_get_loglike(self._h, ptr(out, _dp), self.n_rows))
+        return out
+
+    def power_posterior(self, row0=None, n_rows=None):
+        """Thermodynamic-integration and stepping-stone estimates of log p(y) over the stored rows [row0, row0 + n_rows)
+        (by default every row after the n_initial prior rows) of the rungs of a tempered handle (demcmc_power_posterior):
+        a dict of the totals and the per-rung arrays t, mean_ll, var_ll, ess_ll, rhat_ll, log_ratio."""
+        row0 = self.n_initial if row0 is None else int(row0)
+        n = self.n_rows - row0 if n_rows is None else int(n_rows)
+        cap = self.n_groups
+        ev = _ffi.Evidence()
+        arr = {k: np.zeros(cap) for k in ("t", "mean_ll", "var_ll", "ess_ll", "rhat_ll", "log_ratio")}
+        check(_ffi.lib().demcmc_power_posterior(self._h, row0, n, cap, C.byref(ev), *(ptr(arr[k], _dp) for k in
+                                                ("t", "mean_ll", "var_ll", "ess_ll", "rhat_ll", "log_ratio"))))
+        out = {k: getattr(ev, k) for k, _ in _ffi.Evidence._fields_}
+        out.update({k: v[: ev.n_rungs] for k, v in arr.items()})
+        return out
+
     def comm_init(self, uid: bytes, rank: int, n_ranks: int):
         buf = np.frombuffer(uid, dtype=np.uint8).copy()
         check(_ffi.lib().demcmc_comm_init(self._h, ptr(buf, _bp), rank, n_ranks))

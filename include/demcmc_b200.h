@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define DEMCMC_ABI_VERSION 7
+#define DEMCMC_ABI_VERSION 8
 
 enum { DEMCMC_OK = 0, DEMCMC_EINVAL = -1, DEMCMC_ENODEVICE = -2, DEMCMC_ECUDA = -3, DEMCMC_ENOMEM = -4,
        DEMCMC_ESTATE = -5, DEMCMC_EUNSUPPORTED = -6, DEMCMC_ECOMM = -7 };
@@ -411,6 +411,56 @@ int demcmc_eval_pointwise(demcmc_handle *h, const double *theta, int64_t n, int6
 int demcmc_loo(demcmc_handle *h, const double *theta, int64_t n, double *elpd_loo, double *pareto_k,
                double *lppd, double *p_waic);
 #define DEMCMC_LOO_MAX_DRAWS 16384
+
+/* Model comparison: the marginal likelihood log p(y | M) by power posteriors (Friel & Pettitt 2008; Xie, Lewis, Fan, Kuo &
+ * Chen 2011; Annis, Evans, Miller & Palmeri 2019).
+ *
+ * A tempered handle gives each group g of the job a temperature t_g in [0, 1].  A particle's weight is then
+ * prior(theta) + t_g loglike(theta) (the prior alone at t_g = 0), or -Inf out of bounds: this is what the Metropolis accept,
+ * select_base, demcmc_get_state and the lp column see.  Each particle also carries loglike(theta) untempered; accept keeps
+ * it with theta and every stored row stores it.  A rung is a maximal run of consecutive groups at one temperature.  A
+ * tempered handle has no migration, so a particle never leaves its rung.  With every t_g = 1 the chains, lp and accept are
+ * bit for bit those of an untempered handle.
+ *
+ * Refused on a tempered handle: alpha > 0 with more than one group (migration would move particles between temperatures);
+ * sample = resample; update maximize! / minimize! and fitness = FUN; demcmc_set_weights (the saved particles' untempered
+ * log-likelihoods are unknown); a replay tape with a migration.  A DEMCMC_SIMULATED model takes only t = 1: a power of a
+ * noisy likelihood estimate breaks the pseudo-marginal target.
+ *
+ * demcmc_power_posterior, over the stored rows [row0, row0 + n) of every particle of rung k (temperature t_k, n_k = n times
+ * the rung's particles, ll_s the stored untempered log-likelihoods), for k < K rungs:
+ *   1. mean_ll[k] and var_ll[k] (ddof 1) of the ll_s;
+ *   2. ess_ll[k] and rhat_ll[k]: the split-R-hat and ESS of demcmc_get_diagnostics applied to the ll series, with every
+ *      particle id of the rung as one chain;
+ *   3. for k < K - 1, delta_k = t_(k+1) - t_k and m_k = max_s ll_s: log_ratio[k] = log((1 / n_k) sum_s e_s) + delta_k m_k with
+ *      e_s = exp(delta_k (ll_s - m_k)), the stepping-stone ratio log E_(t_k)[L^delta_k]; log_ratio[K - 1] = NaN.
+ * The totals need the rung temperatures to increase strictly in group order, from t_0 = 0 to t_(K-1) = 1:
+ *   log_z_ti  = sum_(k < K-1) delta_k (mean_ll[k] + mean_ll[k+1]) / 2                 (the trapezoid rule);
+ *   log_z_ti2 = log_z_ti - sum_(k < K-1) delta_k^2 (var_ll[k+1] - var_ll[k]) / 12     (Friel, Hurn & Wyse 2014);
+ *   log_z_ss  = sum_(k < K-1) log_ratio[k];
+ *   se_ti     = sqrt(sum_k w_k^2 var_ll[k] / ess_ll[k]), w_k the trapezoid weights (delta_(k-1) + delta_k) / 2;
+ *   se_ss     = sqrt(sum_(k < K-1) var(e) / (ess_ll[k] mean(e)^2)), the delta method for log of a mean of the e_s, with the
+ *               ESS of ll standing in for the ESS of e.
+ * The standard errors carry the Monte Carlo error only, not the bias of the temperature ladder.  The rows are cut into
+ * slices of one group and 256 rows; each slice's count, mean, sum of squared deviations, max and the two exponential sums
+ * are formed on the device (k_power_posterior) in a fixed order, and the host merges them in rung, group and slice order,
+ * so every output is the same bits from run to run and on any number of devices. */
+typedef struct {
+    int32_t n_rungs;
+    double log_z_ti, log_z_ti2, log_z_ss, se_ti, se_ss;
+} demcmc_evidence;
+/* t[n_groups of the whole job], each in [0, 1]: after demcmc_set_model, before demcmc_set_state (the initial weights are
+ * tempered; DEMCMC_ESTATE otherwise).  Works on multi-device handles and on the ranks of a sharded job. */
+int demcmc_set_temperatures(demcmc_handle *h, const double *t, int32_t n);
+/* the stored untempered log-likelihoods of a tempered handle, in the layout of demcmc_get_lp; the prior rows (< n_initial)
+ * are NaN */
+int demcmc_get_loglike(demcmc_handle *h, double *out, int64_t n_rows);
+/* the evidence above over the stored rows [row0, row0 + n_rows); the per-rung arrays [cap] may each be NULL.  DEMCMC_ESTATE
+ * without temperatures; DEMCMC_EINVAL when cap < the rungs, the rung temperatures are not 0 < ... < 1 increasing, row0 <
+ * n_initial, n_rows < 4, or a parameter has a FLAT prior with an infinite bound (the t = 0 rung would sample an improper
+ * prior); DEMCMC_EUNSUPPORTED above 49152 rows (as demcmc_get_diagnostics) and on a rank of a sharded job */
+int demcmc_power_posterior(demcmc_handle *h, int64_t row0, int64_t n_rows, int32_t cap, demcmc_evidence *out, double *t,
+                           double *mean_ll, double *var_ll, double *ess_ll, double *rhat_ll, double *log_ratio);
 
 /* Particle algebra on the device, for the reference's known-answer tests (test/utility_tests.jl):
  * project (utilities.jl:239-246), reset! (crossover.jl:336-352), random_gamma body

@@ -23,7 +23,7 @@
 # GPU path with a closure throws an ArgumentError -- there is no silent CPU fallback.
 
 const LIBDEMCMC = get(ENV, "LIBDEMCMC_B200", "libdemcmc_b200.so")
-const DEMCMC_ABI_VERSION = Int32(7)
+const DEMCMC_ABI_VERSION = Int32(8)
 
 const GPU_KINDS = (gaussian = 0, mvnormal = 1, binomial = 2, lnr = 3, lba = 4, hier_normal = 5, rastrigin = 6, mvnormal_full = 7, custom = 8, simulated = 9)
 const GPU_PRIORS = (flat = 0, normal = 1, halfcauchy = 2, uniform = 3, beta = 4, normal_ref = 5)
@@ -286,7 +286,8 @@ function model_geometry(ll::GPULoglike, d)
     return n_dim, n_per, n_obs, n_cols
 end
 
-function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_every = 1, return_particles = false)
+function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_every = 1, return_particles = false, temperatures = nothing,
+                     evidence = nothing)
     store_every == 1 || return_particles === false || throw(ArgumentError("optimize keeps every row"))
     store_every == 1 || return _sample_gpu_thinned(model, de, n_iter; device, devices, store_every, seed)
     devs = Vector{Int32}(devices)
@@ -349,10 +350,17 @@ function _sample_gpu(model, de, n_iter; device, seed, devices = Int32[], store_e
             if de.n_initial > 0
                 demcmc_check(ccall((:demcmc_set_history, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}), h[], init_rows))
             end
+            if temperatures !== nothing                        # power_posterior: one temperature per group, before the weights
+                set_temperatures!(h[], temperatures)
+            end
             # init_particle (src/utilities.jl:13-22) already started every particle from samples[1, :, id]
             # when n_initial > 0, so theta0 is right in both cases
             demcmc_check(ccall((:demcmc_set_state, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Int32}), h[], theta0, C_NULL))
             demcmc_check(ccall((:demcmc_run, LIBDEMCMC), Cint, (Ptr{Cvoid}, Int64), h[], n_iter))
+            if evidence !== nothing                            # every row after burn-in, as bundle_samples drops it
+                row0 = max(de.discard_burnin ? de.burnin : 0, de.n_initial)
+                evidence[] = handle_power_posterior(h[], row0, n_rows - row0, de.n_groups)
+            end
             demcmc_check(ccall((:demcmc_get_samples, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Int64), h[], samples, n_rows))
             demcmc_check(ccall((:demcmc_get_accept, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Int64), h[], accept, n_rows))
             demcmc_check(ccall((:demcmc_get_lp, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Int64), h[], lp, n_rows))
@@ -546,4 +554,52 @@ function loo(model::DEModel{<:GPULoglike}, chains; device = 0)
     return (elpd_loo = sum(elpd_i), se_elpd_loo = se(elpd_i), p_loo = sum(lppd_i) - sum(elpd_i), elpd_waic = sum(waic_i),
             se_elpd_waic = se(waic_i), p_waic = sum(pw_i), n_bad_k = count(>(0.7), k), elpd_loo_i = elpd_i, pareto_k = k,
             lppd_i = lppd_i, p_waic_i = pw_i)
+end
+
+# ---- power posteriors: the marginal likelihood log p(y | M) (include/demcmc_b200.h: demcmc_power_posterior) ----------------
+struct CEvidence
+    n_rungs::Int32
+    log_z_ti::Float64
+    log_z_ti2::Float64
+    log_z_ss::Float64
+    se_ti::Float64
+    se_ss::Float64
+end
+
+# t[g] in [0, 1] for every group of the job: after demcmc_set_model, before demcmc_set_state
+set_temperatures!(h::Ptr{Cvoid}, t::AbstractVector{<:Real}) = (tt = Vector{Float64}(t);
+    GC.@preserve tt demcmc_check(ccall((:demcmc_set_temperatures, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Int32), h, tt, length(tt))))
+
+# the stored untempered log-likelihoods, n_rows × P like Particle.lp (the n_initial prior rows are NaN)
+function get_loglike(h::Ptr{Cvoid}, n_rows, P)
+    out = zeros(Float64, n_rows, P)
+    GC.@preserve out demcmc_check(ccall((:demcmc_get_loglike, LIBDEMCMC), Cint, (Ptr{Cvoid}, Ptr{Float64}, Int64), h, out, n_rows))
+    return out
+end
+
+function handle_power_posterior(h::Ptr{Cvoid}, row0, n_rows, cap)
+    ev = Ref{CEvidence}()
+    a = ntuple(_ -> zeros(Float64, cap), 6)
+    GC.@preserve a demcmc_check(ccall((:demcmc_power_posterior, LIBDEMCMC), Cint,
+        (Ptr{Cvoid}, Int64, Int64, Int32, Ref{CEvidence}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}),
+        h, row0, n_rows, cap, ev, a[1], a[2], a[3], a[4], a[5], a[6]))
+    K = Int(ev[].n_rungs)
+    return (log_z_ti = ev[].log_z_ti, log_z_ti2 = ev[].log_z_ti2, log_z_ss = ev[].log_z_ss, se_ti = ev[].se_ti, se_ss = ev[].se_ss,
+            t = a[1][1:K], mean_ll = a[2][1:K], var_ll = a[3][1:K], ess_ll = a[4][1:K], rhat_ll = a[5][1:K], log_ratio = a[6][1:K])
+end
+
+# Thermodynamic integration and stepping stones in ONE run: rung k is de.n_groups groups at t_k = (k / (K - 1))^power, all
+# K rungs in one handle of K * de.n_groups groups (de.α must be 0: migration would move particles between temperatures).
+# Returns the estimates and the t = 1 rung's chains.
+function power_posterior(model::DEModel{<:GPULoglike}, de::DE, n_iter::Int; temperatures = nothing, n_temperatures = 32,
+                         power = 5.0, device = 0, seed = rand(UInt64))
+    t = temperatures === nothing ? [(k / (n_temperatures - 1))^power for k = 0:(n_temperatures - 1)] : Vector{Float64}(temperatures)
+    de.α > 0 && throw(ArgumentError("power_posterior runs every rung as groups of one handle: pass DE(α = 0)"))
+    G = de.n_groups
+    job = deepcopy(de)
+    job.n_groups = length(t) * G
+    ev = Ref{Any}(nothing)
+    chains = _sample_gpu(model, job, n_iter; device, seed, temperatures = repeat(t, inner = G), evidence = ev)
+    top = (size(chains, 3) - G * de.Np + 1):size(chains, 3)
+    return merge(ev[], (chains = chains[:, :, top],))
 end
